@@ -255,6 +255,28 @@ def _sharded_equals_single(engine, layout, FCNetwork, args, dev, comm, rank):
     return res
 
 
+def dump_outputs(eng, out_dir):
+    """Write what the engine's last generation hands its caller to ``out_dir/<name>.npy``, so that two
+    builds run with the same arguments can be compared output for output: per role the members' rewards
+    (fp64, this rank's members), the fitness the update used (fp64, all members), the updated base row and
+    the update applied to it (fp32, the row's parameters without the pitch padding), and the three rewards
+    of the evaluation games (fp64).  About 3.4 MB at the bench workload."""
+    import numpy as np
+    from coevonet_b200 import layout
+    arrays = {"eval_rewards": np.array(eng.last_eval(), dtype=np.float64)}
+    for r in ROLES:
+        d = layout.fc_dim(layout.OBS_DIM[r])
+        arrays[f"rewards_{r}"] = eng.rewards[r].cpu().numpy()
+        arrays[f"fitness_{r}"] = eng.fitness[r].cpu().numpy()
+        arrays[f"theta_{r}"] = eng.theta[r][:d].cpu().numpy()
+        arrays[f"delta_{r}"] = eng.last_delta[r][:d].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError(f"{name}: {a.dtype} is neither float32 nor float64")
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_gpu_arm(ns):
     import numpy as np
     import torch
@@ -310,6 +332,9 @@ def run_gpu_arm(ns):
     clocks = sampler.stop() if rank == 0 else None
     launches = ops.launch_count - launches0
     ms_total = e0.elapsed_time(e1)
+    # the passes below keep stepping the engine: its outputs are those of the last timed step only here
+    if ns.dump_outputs and rank == 0:
+        dump_outputs(eng, ns.dump_outputs)
 
     # ---- per-kernel durations for the roofline: the same generation with the three roles back to back
     # on one stream (in the timed region above they overlap on three streams, which is faster but makes
@@ -523,7 +548,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", dest="no_cpu_baseline", action="store_true")
     ap.add_argument("--no-secondary", dest="no_secondary", action="store_true",
                     help="skip the secondary configs / per-kernel rooflines (bench_secondary.py)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's outputs to DIR/<name>.npy (rank 0)")
     ns = ap.parse_args()
+    if ns.steps < 1 or ns.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if ns.impl == "reference" and ns.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of this build's GPU path (--impl b200)")
     if ns.impl == "reference":
         return run_reference_arm(ns)
     return run_gpu_arm(ns)

@@ -1,5 +1,5 @@
 import os, sys
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from coevonet_b200 import layout, ops
 pitch = layout.fc_pitch(10)

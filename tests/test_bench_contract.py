@@ -1,9 +1,13 @@
 """The committed bench lines (profiles/r0*_bench_n*.json, written by bench.py on a B200) carry every key
-the measurement contract names; bench.py's CLI parses the driver's flags.  No GPU needed."""
+the measurement contract names; bench.py's CLI parses the driver's flags and --dump-outputs writes the
+last step's arrays.  No GPU needed except for the test marked gpu."""
 import json
 import os
 import subprocess
 import sys
+import types
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -47,8 +51,77 @@ def test_eight_gpu_line_is_the_whole_job_aggregate():
 def test_bench_cli_accepts_the_driver_flags():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--help"], capture_output=True, text=True)
     assert out.returncode == 0
-    for flag in ("--gpus", "--steps", "--warmup", "--impl"):
+    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--dump-outputs"):
         assert flag in out.stdout
+
+
+def test_dump_outputs_writes_the_last_steps_arrays(tmp_path):
+    import numpy as np
+    import torch
+
+    import bench
+    from coevonet_b200 import layout
+    pitch = {r: layout.fc_pitch(layout.OBS_DIM[r]) for r in bench.ROLES}
+    eng = types.SimpleNamespace(
+        last_eval=lambda: (1.5, -2.0, 0.25),
+        rewards={r: torch.arange(4, dtype=torch.float64) for r in bench.ROLES},
+        fitness={r: torch.arange(8, dtype=torch.float64) for r in bench.ROLES},
+        theta={r: torch.ones(pitch[r]) for r in bench.ROLES},
+        last_delta={r: torch.full((pitch[r],), 0.5) for r in bench.ROLES})
+    bench.dump_outputs(eng, str(tmp_path / "out"))
+    files = sorted(p.name for p in (tmp_path / "out").iterdir())
+    assert files == sorted(["eval_rewards.npy"] + [f"{k}_{r}.npy" for r in bench.ROLES
+                                                   for k in ("rewards", "fitness", "theta", "delta")])
+    assert np.load(tmp_path / "out" / "eval_rewards.npy").tolist() == [1.5, -2.0, 0.25]
+    for r in bench.ROLES:
+        theta = np.load(tmp_path / "out" / f"theta_{r}.npy")
+        assert theta.dtype == np.float32 and theta.shape == (layout.fc_dim(layout.OBS_DIM[r]),)
+        assert np.load(tmp_path / "out" / f"fitness_{r}.npy").dtype == np.float64
+    assert sum(p.stat().st_size for p in (tmp_path / "out").iterdir()) < 64 << 20
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_a_real_engine_are_consistent_and_repeat(tmp_path):
+    """bench.dump_outputs on the bench's own engine (small population): the arrays are what the last
+    generation produced, and a second run with the same arguments writes the same bits."""
+    import numpy as np
+    import torch
+
+    import bench
+    from coevonet_b200 import engine, layout
+    from coevonet_b200.MPE.fcnetwork import FCNetwork
+    P = 64
+
+    def run(out):
+        torch.manual_seed(0)
+        theta = {r: FCNetwork(layout.OBS_DIM[r], 5, "float32").flat_row() for r in bench.ROLES}
+        eng = engine.ESEngine(bench._args_bag(P), torch.device("cuda", 0), theta, comm=engine.Comm())
+        eng.step(sync=False)
+        before = {r: eng.theta[r].cpu().numpy() for r in bench.ROLES}
+        eng.step(sync=False)
+        eng.check_status()
+        bench.dump_outputs(eng, str(out))
+        assert np.load(out / "eval_rewards.npy").tolist() == list(eng.last_eval())
+        return before
+
+    before = run(tmp_path / "a")
+    run(tmp_path / "b")
+    for f in sorted((tmp_path / "a").iterdir()):
+        assert np.array_equal(np.load(f), np.load(tmp_path / "b" / f.name)), f.name
+    for r in bench.ROLES:
+        d = layout.fc_dim(layout.OBS_DIM[r])
+        load = lambda k: np.load(tmp_path / "a" / f"{k}_{r}.npy")
+        rewards, fitness, theta, delta = load("rewards"), load("fitness"), load("theta"), load("delta")
+        assert rewards.shape == fitness.shape == (P,) and theta.shape == delta.shape == (d,)
+        assert np.array_equal(fitness, rewards.astype(np.float32).astype(np.float64))   # no fitness sharing
+        assert np.array_equal(theta, before[r][:d] + delta)                              # theta += delta
+        assert np.abs(delta).max() > 0
+
+
+def test_bench_rejects_a_step_count_below_one():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"],
+                         capture_output=True, text=True)
+    assert out.returncode != 0 and "--steps" in out.stderr
 
 
 def test_round2_line_carries_parity_secondary_and_floors():
