@@ -18,7 +18,8 @@ LIB_PATH = os.environ.get("COEVONET_LIB") or os.path.join(_HERE, "csrc", "libcoe
 CEV_OK = 0
 STATUS_NONFINITE = 1
 SEAT = {"adversary_0": 0, "agent_0": 1, "agent_1": 2}
-KIND_ES, KIND_GA, KIND_ENV, KIND_FRAMES, KIND_INIT, KIND_XOVER = 0, 1, 2, 3, 4, 5
+KIND_ES, KIND_GA, KIND_ENV, KIND_FRAMES, KIND_INIT, KIND_XOVER, KIND_ES_MIRROR = 0, 1, 2, 3, 4, 5, 6
+ES_SGD, ES_ADAM = 0, 1
 INIT_STATE_DIM = 11
 ROLLOUT_OUT_DIM = 4
 ORDER_STABLE_DESC, ORDER_REFERENCE = 0, 1
@@ -91,6 +92,13 @@ _SIGNATURES = {
     "cev_generation_end_f64": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_double,
                                        c_double, c_int, c_double, c_int, c_void_p]),
     "cev_axpy_f32": (c_int, [c_void_p, c_float, c_void_p, c_void_p, c_int64, c_void_p]),
+    "cev_es_perturb_mirrored_f32": (c_int, [c_void_p, c_void_p, c_int, c_float, c_void_p, c_uint64, c_int, c_uint32,
+                                            c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),
+    "cev_es_update_mirrored_f32": (c_int, [c_void_p, c_void_p, c_int, c_float, c_void_p, c_float, c_int64,
+                                           c_uint64, c_int, c_uint32, c_int64, c_int64, c_void_p, c_void_p]),
+    "cev_centered_ranks_f64": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p]),
+    "cev_es_apply_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, POINTER(c_int), c_int,
+                                 c_double, c_float, c_int, c_void_p]),
     "cev_diversity_dist_f32": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_int,
                                        c_void_p, c_void_p]),
     "cev_deepqn_forward": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_void_p, c_int, c_int,

@@ -86,6 +86,43 @@ __global__ void __launch_bounds__(PT) ga_repopulate_kernel(
 // Every segment boundary of the row is a multiple of 4 parameters except the end of the row, so a float4 is
 // perturbable or not as a whole (the LayerNorm float4s skip the Philox / Box-Muller work altogether).
 constexpr int K5T = 128;
+
+// One float4 (parameters j .. j+3) of K5.  `counter` is the Philox member word: the member id, or the pair id
+// q = c >> 1 under mirrored sampling, where the normals of one draw give the row theta + sigma z (`plus`, the
+// even member 2q) and the row theta - sigma z (`minus`, the odd member 2q+1) with the same rounded product.
+// A null row pointer skips that row (a pair cut by the shard boundary); noise rows receive +z / -z.
+template <bool MIRROR>
+__device__ __forceinline__ void es_perturb_float4(
+    const float* __restrict__ theta, const FcOffsets& o, int j4, float sigma, const PhiloxKeys& keys, uint32_t tag,
+    uint32_t gen, uint32_t counter, float* __restrict__ plus, float* __restrict__ minus,
+    float* __restrict__ noise_plus, float* __restrict__ noise_minus) {
+    const int j = j4 * 4;
+    const float4 pv = __ldg(reinterpret_cast<const float4*>(theta + j));
+    float p[4] = {pv.x, pv.y, pv.z, pv.w};
+    float m[4] = {pv.x, pv.y, pv.z, pv.w};
+    float z[4] = {0.f, 0.f, 0.f, 0.f};
+    if (j < o.total && fc_is_perturbable(o, j)) {
+        normal4(keys, tag, gen, counter, (uint32_t)j4, z);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            if (j + i < o.total) {
+                const float d = __fmul_rn(sigma, z[i]);
+                p[i] = __fadd_rn(p[i], d);
+                if (MIRROR) m[i] = __fadd_rn(m[i], -d);
+            } else { z[i] = 0.f; p[i] = 0.f; m[i] = 0.f; }
+        }
+    } else if (j >= o.total) {
+        p[0] = p[1] = p[2] = p[3] = 0.f;
+        m[0] = m[1] = m[2] = m[3] = 0.f;
+    }
+    if (!MIRROR || plus) __stcs(reinterpret_cast<float4*>(plus + j), make_float4(p[0], p[1], p[2], p[3]));
+    if (MIRROR && minus) __stcs(reinterpret_cast<float4*>(minus + j), make_float4(m[0], m[1], m[2], m[3]));
+    if (noise_plus)
+        *reinterpret_cast<float4*>(noise_plus + j) = make_float4(z[0], z[1], z[2], z[3]);
+    if (MIRROR && noise_minus)
+        *reinterpret_cast<float4*>(noise_minus + j) = make_float4(-z[0], -z[1], -z[2], -z[3]);
+}
+
 __global__ void __launch_bounds__(K5T, 10) es_perturb_kernel(
     const float* __restrict__ theta, int in_dim, int64_t pitch, float sigma_arg,
     const double* __restrict__ sigma_dev,
@@ -96,24 +133,30 @@ __global__ void __launch_bounds__(K5T, 10) es_perturb_kernel(
     const int64_t r = blockIdx.x;
     const int64_t c = row0 + r;
     const int j4 = blockIdx.y * K5T + threadIdx.x;
-    const int j = j4 * 4;
-    if ((int64_t)j >= pitch) return;
-    const float4 pv = __ldg(reinterpret_cast<const float4*>(theta + j));
-    float p[4] = {pv.x, pv.y, pv.z, pv.w};
-    float z[4] = {0.f, 0.f, 0.f, 0.f};
-    if (j < o.total && fc_is_perturbable(o, j)) {
-        normal4(keys, tag, gen, (uint32_t)c, (uint32_t)j4, z);
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            if (j + i < o.total) p[i] = __fadd_rn(p[i], __fmul_rn(sigma, z[i]));
-            else { z[i] = 0.f; p[i] = 0.f; }
-        }
-    } else if (j >= o.total) {
-        p[0] = p[1] = p[2] = p[3] = 0.f;
-    }
-    __stcs(reinterpret_cast<float4*>(out + r * pitch + j), make_float4(p[0], p[1], p[2], p[3]));
-    if (noise_out)
-        *reinterpret_cast<float4*>(noise_out + r * pitch + j) = make_float4(z[0], z[1], z[2], z[3]);
+    if ((int64_t)j4 * 4 >= pitch) return;
+    es_perturb_float4<false>(theta, o, j4, sigma, keys, tag, gen, (uint32_t)c, out + r * pitch, nullptr,
+                             noise_out ? noise_out + r * pitch : nullptr, nullptr);
+}
+
+// K5 under mirrored sampling (Salimans et al. 2017): one CTA row per PAIR q of the local block, members 2q and
+// 2q+1 from one normal draw (half the Philox / Box-Muller work of es_perturb_kernel).  Local row r holds global
+// member row0 + r; the first / last pair writes only its local row when row0 / row0 + n_rows is odd.
+__global__ void __launch_bounds__(K5T, 10) es_perturb_mirrored_kernel(
+    const float* __restrict__ theta, int in_dim, int64_t pitch, float sigma_arg,
+    const double* __restrict__ sigma_dev,
+    const PhiloxKeys keys, uint32_t tag, uint32_t gen, int64_t row0, int64_t n_rows,
+    float* __restrict__ out, float* __restrict__ noise_out) {
+    const float sigma = pick_sigma(sigma_arg, sigma_dev);
+    const FcOffsets o = fc_offsets(in_dim);
+    const int64_t q = (row0 >> 1) + blockIdx.x;
+    const int64_t r_plus = 2 * q - row0, r_minus = r_plus + 1;        // local rows of members 2q, 2q+1
+    const bool has_plus = r_plus >= 0, has_minus = r_minus < n_rows;
+    const int j4 = blockIdx.y * K5T + threadIdx.x;
+    if ((int64_t)j4 * 4 >= pitch) return;
+    es_perturb_float4<true>(theta, o, j4, sigma, keys, tag, gen, (uint32_t)q,
+                            has_plus ? out + r_plus * pitch : nullptr, has_minus ? out + r_minus * pitch : nullptr,
+                            noise_out && has_plus ? noise_out + r_plus * pitch : nullptr,
+                            noise_out && has_minus ? noise_out + r_minus * pitch : nullptr);
 }
 
 // K5 for rows whose perturbable parameters are a PREFIX of the row: DeepQN rows hold the conv / Linear
@@ -148,18 +191,16 @@ __global__ void __launch_bounds__(PT) es_perturb_prefix_kernel(
 // Philox key.  Members are split over blockIdx.y; partial sums are reduced in a
 // fixed order by the second kernel (deterministic, no atomics).
 // ---------------------------------------------------------------------------
-__global__ void __launch_bounds__(PT) es_update_partial_kernel(
-    const double* __restrict__ fitness, int in_dim, int64_t pitch, float sigma_arg,
-    const double* __restrict__ sigma_dev,
-    const PhiloxKeys keys, uint32_t tag, uint32_t gen, int64_t row0, int64_t n_rows,
-    int n_split, float* __restrict__ partial) {
-    const float sigma = pick_sigma(sigma_arg, sigma_dev);
+// Partial sum over the local rows [r_lo, r_hi) of split `sp`, in row order.  MIRROR: member c = row0 + r carries
+// s_c * (sigma z_q) with q = c >> 1, s_c = +1 for even c, -1 for odd c; z_q is generated once per pair, so the
+// terms, and their order, are those of the per-member loop (the negation is exact).
+template <bool MIRROR>
+__device__ __forceinline__ void es_update_partial_body(
+    const double* __restrict__ fitness, int in_dim, int64_t pitch, float sigma, const PhiloxKeys& keys,
+    uint32_t tag, uint32_t gen, int64_t row0, int64_t r_lo, int64_t r_hi, int sp, float* __restrict__ partial) {
     const FcOffsets o = fc_offsets(in_dim);
     const int j4 = blockIdx.x * PT + threadIdx.x;
     if ((int64_t)j4 * 4 >= pitch) return;
-    const int sp = blockIdx.y;
-    const int64_t per = (n_rows + n_split - 1) / n_split;
-    const int64_t r_lo = sp * per, r_hi = min(n_rows, r_lo + per);
     float acc[4] = {0.f, 0.f, 0.f, 0.f};
     bool pert[4];
 #pragma unroll
@@ -168,12 +209,32 @@ __global__ void __launch_bounds__(PT) es_update_partial_kernel(
         pert[i] = j < o.total && fc_is_perturbable(o, j);
     }
     if (pert[0] || pert[1] || pert[2] || pert[3]) {
-        for (int64_t r = r_lo; r < r_hi; ++r) {
-            const float f = (float)fitness[r];
-            float z[4];
-            normal4(keys, tag, gen, (uint32_t)(row0 + r), (uint32_t)j4, z);
+        if (!MIRROR) {
+            for (int64_t r = r_lo; r < r_hi; ++r) {
+                const float f = (float)fitness[r];
+                float z[4];
+                normal4(keys, tag, gen, (uint32_t)(row0 + r), (uint32_t)j4, z);
 #pragma unroll
-            for (int i = 0; i < 4; ++i) acc[i] = fmaf(__fmul_rn(sigma, z[i]), f, acc[i]);
+                for (int i = 0; i < 4; ++i) acc[i] = fmaf(__fmul_rn(sigma, z[i]), f, acc[i]);
+            }
+        } else {
+            for (int64_t r = r_lo; r < r_hi;) {
+                const int64_t c = row0 + r;
+                float z[4];
+                normal4(keys, tag, gen, (uint32_t)(c >> 1), (uint32_t)j4, z);
+#pragma unroll
+                for (int i = 0; i < 4; ++i) z[i] = __fmul_rn(sigma, z[i]);
+                if (!(c & 1)) {
+                    const float f = (float)fitness[r];
+#pragma unroll
+                    for (int i = 0; i < 4; ++i) acc[i] = fmaf(z[i], f, acc[i]);
+                    if (++r == r_hi) break;
+                }
+                const float f = (float)fitness[r];
+#pragma unroll
+                for (int i = 0; i < 4; ++i) acc[i] = fmaf(-z[i], f, acc[i]);
+                ++r;
+            }
         }
     }
 #pragma unroll
@@ -181,6 +242,35 @@ __global__ void __launch_bounds__(PT) es_update_partial_kernel(
         if (!pert[i]) acc[i] = 0.f;
     *reinterpret_cast<float4*>(partial + (int64_t)sp * pitch + (int64_t)j4 * 4) =
         make_float4(acc[0], acc[1], acc[2], acc[3]);
+}
+
+__global__ void __launch_bounds__(PT) es_update_partial_kernel(
+    const double* __restrict__ fitness, int in_dim, int64_t pitch, float sigma_arg,
+    const double* __restrict__ sigma_dev,
+    const PhiloxKeys keys, uint32_t tag, uint32_t gen, int64_t row0, int64_t n_rows,
+    int n_split, float* __restrict__ partial) {
+    const int sp = blockIdx.y;
+    const int64_t per = (n_rows + n_split - 1) / n_split;
+    const int64_t r_lo = sp * per, r_hi = min(n_rows, r_lo + per);
+    es_update_partial_body<false>(fitness, in_dim, pitch, pick_sigma(sigma_arg, sigma_dev), keys, tag, gen, row0,
+                                  r_lo, r_hi, sp, partial);
+}
+
+// Mirrored sampling: the splits cover GLOBAL rows [base + sp*per, base + (sp+1)*per) of this rank's block, with
+// base = row0 rounded down to even and `per` even, so every split but the first starts on a pair.
+__global__ void __launch_bounds__(PT) es_update_mirrored_partial_kernel(
+    const double* __restrict__ fitness, int in_dim, int64_t pitch, float sigma_arg,
+    const double* __restrict__ sigma_dev,
+    const PhiloxKeys keys, uint32_t tag, uint32_t gen, int64_t row0, int64_t n_rows,
+    int n_split, float* __restrict__ partial) {
+    const int sp = blockIdx.y;
+    const int64_t base = row0 & ~(int64_t)1;
+    const int64_t span = row0 + n_rows - base;
+    const int64_t per = ((span + n_split - 1) / n_split + 1) & ~(int64_t)1;
+    const int64_t r_lo = max(base + sp * per, row0) - row0;
+    const int64_t r_hi = min(base + (sp + 1) * per, row0 + n_rows) - row0;
+    es_update_partial_body<true>(fitness, in_dim, pitch, pick_sigma(sigma_arg, sigma_dev), keys, tag, gen, row0,
+                                 r_lo, r_hi, sp, partial);
 }
 
 // The same partial sums from the MATERIALISED members: sigma z_i = member_i - theta up to one rounding
@@ -227,6 +317,92 @@ __global__ void __launch_bounds__(PT) axpy_kernel(float a, const float* __restri
                                                   float* __restrict__ y, int64_t n) {
     const int64_t j = (int64_t)blockIdx.x * PT + threadIdx.x;
     if (j < n) y[j] = __fadd_rn(y[j], __fmul_rn(a, x[j]));
+}
+
+// ---------------------------------------------------------------------------
+// Centered-rank fitness shaping (Salimans et al. 2017; extends evolutionary_strategy.py:120-148, whose
+// normalisation is commented out at :133-135).  u_i = r_i / (P-1) - 0.5 with the average rank
+// r_i = #{F_j < F_i} + (#{F_j == F_i} - 1) / 2 over the GLOBAL fitness; the thread of local row r ranks member
+// row0 + r against all P keys staged in shared-memory tiles (integer compares only: P * n_rows of them).
+// ---------------------------------------------------------------------------
+constexpr int RK_T = 256;
+constexpr int RK_TILE = 2048;          // keys per tile: 16 KB of shared memory
+
+// Order-preserving key of an fp64 value: -0.0 maps to +0.0's key, every NaN to 0 (below -inf, whose key is
+// 0x000FFFFFFFFFFFFF): all NaNs tie and rank below every number.
+__device__ __forceinline__ unsigned long long rank_key(double x) {
+    if (x != x) return 0ull;
+    unsigned long long b = (unsigned long long)__double_as_longlong(x);
+    if ((b << 1) == 0ull) b = 0ull;
+    return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
+}
+
+__global__ void __launch_bounds__(RK_T) centered_ranks_kernel(const double* __restrict__ fitness, int64_t P,
+                                                              int64_t row0, int64_t n_rows,
+                                                              double* __restrict__ out) {
+    __shared__ unsigned long long tile[RK_TILE];
+    const int64_t r = (int64_t)blockIdx.x * RK_T + threadIdx.x;
+    const unsigned long long k = r < n_rows ? rank_key(fitness[row0 + r]) : 0ull;
+    int64_t lt = 0, eq = 0;
+    for (int64_t t0 = 0; t0 < P; t0 += RK_TILE) {
+        const int n = (int)min((int64_t)RK_TILE, P - t0);
+        __syncthreads();
+        for (int i = threadIdx.x; i < n; i += RK_T) tile[i] = rank_key(fitness[t0 + i]);
+        __syncthreads();
+        int lt_t = 0, eq_t = 0;
+#pragma unroll 8
+        for (int i = 0; i < n; ++i) {
+            const unsigned long long kj = tile[i];
+            lt_t += kj < k;
+            eq_t += kj == k;
+        }
+        lt += lt_t;
+        eq += eq_t;
+    }
+    if (r >= n_rows) return;
+    const double rank = __dadd_rn((double)lt, __dmul_rn(0.5, (double)(eq - 1)));   // exact: a multiple of 1/2
+    out[r] = P > 1 ? __dsub_rn(__ddiv_rn(rank, (double)(P - 1)), 0.5) : 0.0;
+}
+
+// ---------------------------------------------------------------------------
+// Fused ES apply over the roles' concatenated rows (extends evolutionary_strategy.py:259-265; the reference
+// builds an Adam optimizer per agent and never uses it, MPE/mpe_agent.py:20).  g = ghat - l2 * theta, then
+//   sgd:  theta += lr * g
+//   adam: m = b1 m + (1-b1) g ; v = b2 v + (1-b2) g g ; theta += alpha_t m / (sqrt(v) + eps)
+// one IEEE-rounded fp32 operation at a time (no contraction), on the perturbable entries only: LayerNorm
+// entries and padding of theta, m and v keep their bits.
+// ---------------------------------------------------------------------------
+struct ApplySegments {
+    int n;
+    int in_dim[CEV_MAX_ROLES];
+    int64_t end[CEV_MAX_ROLES];        // exclusive end offset of each segment in the concatenated row
+};
+
+__global__ void __launch_bounds__(PT) es_apply_kernel(float* __restrict__ theta, const float* __restrict__ delta,
+                                                      float* __restrict__ m, float* __restrict__ v,
+                                                      const ApplySegments seg, int adam, float step, float l2) {
+    const int64_t i = (int64_t)blockIdx.x * PT + threadIdx.x;
+    int in_dim = seg.in_dim[0];
+    int64_t start = 0, end = seg.end[0];
+#pragma unroll
+    for (int s = 1; s < CEV_MAX_ROLES; ++s)          // constant indices: the segment table stays in registers
+        if (s < seg.n && i >= end) { in_dim = seg.in_dim[s]; start = end; end = seg.end[s]; }
+    if (i >= end) return;
+    const FcOffsets o = fc_offsets(in_dim);
+    const int j = (int)(i - start);
+    if (j >= o.total || !fc_is_perturbable(o, j)) return;
+    const float th = theta[i];
+    const float g = __fsub_rn(delta[i], __fmul_rn(l2, th));
+    if (!adam) {
+        theta[i] = __fadd_rn(th, __fmul_rn(step, g));
+        return;
+    }
+    const float b1 = CEV_ADAM_BETA1, b2 = CEV_ADAM_BETA2, eps = CEV_ADAM_EPS;
+    const float mi = __fadd_rn(__fmul_rn(b1, m[i]), __fmul_rn(__fsub_rn(1.f, b1), g));
+    const float vi = __fadd_rn(__fmul_rn(b2, v[i]), __fmul_rn(__fmul_rn(__fsub_rn(1.f, b2), g), g));
+    m[i] = mi;
+    v[i] = vi;
+    theta[i] = __fadd_rn(th, __fdiv_rn(__fmul_rn(step, mi), __fadd_rn(__fsqrt_rn(vi), eps)));
 }
 
 // ---------------------------------------------------------------------------
@@ -771,6 +947,93 @@ int cev_es_update_members_f32(cev_handle* h, const double* fitness, const float*
     es_update_finish_kernel<<<(unsigned)((pitch + PT - 1) / PT), PT, 0, (cudaStream_t)stream>>>(
         partial, n_split, pitch, (double)lr, (double)n_total, sigma, sigma_dev, delta);
     return check_cuda(cudaGetLastError(), "es_update_members kernels");
+}
+
+int cev_es_perturb_mirrored_f32(cev_handle* h, const float* theta, int in_dim, float sigma, const double* sigma_dev,
+                                uint64_t seed, int role, uint32_t gen, int64_t row0, int64_t n_rows, int64_t pitch,
+                                float* out, float* noise_out, cev_stream stream) {
+    CEV_REQUIRE(h != nullptr, "es_perturb_mirrored: null handle");
+    if (n_rows == 0) return CEV_OK;                   // an empty shard contributes nothing
+    CEV_REQUIRE(theta && out, "es_perturb_mirrored: null pointer");
+    CEV_REQUIRE(in_dim == IN_ADV || in_dim == IN_GOOD, "es_perturb_mirrored: in_dim must be 8 or 10");
+    CEV_REQUIRE(pitch >= fc_offsets(in_dim).total && pitch % 4 == 0, "es_perturb_mirrored: bad pitch");
+    CEV_REQUIRE(aligned16(theta) && aligned16(out) && aligned16(noise_out), "es_perturb_mirrored: 16B alignment");
+    CEV_REQUIRE(row0 >= 0 && n_rows >= 0 && row0 + n_rows <= 0xFFFFFFFFll, "es_perturb_mirrored: bad row range");
+    CEV_GUARD(h);
+    uint32_t k0, k1;
+    split_seed(seed, k0, k1);
+    const int64_t n_pairs = ((row0 + n_rows - 1) >> 1) - (row0 >> 1) + 1;
+    dim3 grid((unsigned)n_pairs, (unsigned)((pitch / 4 + K5T - 1) / K5T));
+    es_perturb_mirrored_kernel<<<grid, K5T, 0, (cudaStream_t)stream>>>(
+        theta, in_dim, pitch, sigma, sigma_dev, philox_keys(k0, k1), noise_tag(CEV_KIND_ES_MIRROR, role), gen, row0,
+        n_rows, out, noise_out);
+    return check_cuda(cudaGetLastError(), "es_perturb_mirrored_kernel");
+}
+
+int cev_es_update_mirrored_f32(cev_handle* h, const double* fitness, int in_dim, float sigma, const double* sigma_dev,
+                               float lr, int64_t n_total, uint64_t seed, int role, uint32_t gen, int64_t row0,
+                               int64_t n_rows, float* delta, cev_stream stream) {
+    // an empty shard (n_rows == 0, fitness may be null) still writes its all-zero partial delta
+    CEV_REQUIRE(h && (fitness || n_rows == 0) && delta, "es_update_mirrored: null pointer");
+    CEV_REQUIRE(in_dim == IN_ADV || in_dim == IN_GOOD, "es_update_mirrored: in_dim must be 8 or 10");
+    CEV_REQUIRE(n_total >= 1 && n_rows >= 0 && (sigma_dev || sigma > 0.f), "es_update_mirrored: bad n/sigma");
+    CEV_REQUIRE(row0 >= 0 && row0 + n_rows <= 0xFFFFFFFFll, "es_update_mirrored: bad row range");
+    CEV_REQUIRE(aligned16(delta), "es_update_mirrored: 16B alignment");
+    CEV_GUARD(h);
+    const int64_t pitch = fc_pitch(in_dim);
+    int n_split = (int)((n_rows + 63) / 64);
+    if (n_split > 16) n_split = 16;
+    if (n_split < 1) n_split = 1;
+    int rc = ensure_workspace(h, (size_t)n_split * pitch * sizeof(float));
+    if (rc) return rc;
+    uint32_t k0, k1;
+    split_seed(seed, k0, k1);
+    float* partial = static_cast<float*>(h->workspace);
+    dim3 grid((unsigned)((pitch / 4 + PT - 1) / PT), (unsigned)n_split);
+    es_update_mirrored_partial_kernel<<<grid, PT, 0, (cudaStream_t)stream>>>(
+        fitness, in_dim, pitch, sigma, sigma_dev, philox_keys(k0, k1), noise_tag(CEV_KIND_ES_MIRROR, role), gen, row0,
+        n_rows, n_split, partial);
+    CEV_CUDA(cudaGetLastError());
+    es_update_finish_kernel<<<(unsigned)((pitch + PT - 1) / PT), PT, 0, (cudaStream_t)stream>>>(
+        partial, n_split, pitch, (double)lr, (double)n_total, sigma, sigma_dev, delta);
+    return check_cuda(cudaGetLastError(), "es_update_mirrored kernels");
+}
+
+int cev_centered_ranks_f64(cev_handle* h, const double* fitness, int64_t P, int64_t row0, int64_t n_rows,
+                           double* out, cev_stream stream) {
+    CEV_REQUIRE(h != nullptr, "centered_ranks: null handle");
+    CEV_REQUIRE(P >= 1 && row0 >= 0 && n_rows >= 0 && row0 + n_rows <= P, "centered_ranks: need 0 <= row0, "
+                "row0 + n_rows <= P (row0 %lld, n_rows %lld, P %lld)", (long long)row0, (long long)n_rows, (long long)P);
+    if (n_rows == 0) return CEV_OK;
+    CEV_REQUIRE(fitness && out, "centered_ranks: null pointer");
+    CEV_GUARD(h);
+    centered_ranks_kernel<<<(unsigned)((n_rows + RK_T - 1) / RK_T), RK_T, 0, (cudaStream_t)stream>>>(
+        fitness, P, row0, n_rows, out);
+    return check_cuda(cudaGetLastError(), "centered_ranks_kernel");
+}
+
+int cev_es_apply_f32(cev_handle* h, float* theta, const float* delta, float* m, float* v, int n_segments,
+                     const int* in_dims, int optimizer, double lr, float l2_coeff, int t, cev_stream stream) {
+    CEV_REQUIRE(h && theta && delta && in_dims, "es_apply: null pointer");
+    CEV_REQUIRE(n_segments >= 1 && n_segments <= CEV_MAX_ROLES, "es_apply: need 1 <= n_segments <= %d", CEV_MAX_ROLES);
+    CEV_REQUIRE(optimizer == CEV_ES_SGD || optimizer == CEV_ES_ADAM, "es_apply: optimizer must be CEV_ES_SGD or CEV_ES_ADAM");
+    CEV_REQUIRE(optimizer == CEV_ES_SGD || (m && v && t >= 1), "es_apply: Adam needs m, v and t >= 1");
+    ApplySegments seg{};
+    seg.n = n_segments;
+    int64_t off = 0;
+    for (int s = 0; s < n_segments; ++s) {
+        CEV_REQUIRE(in_dims[s] == IN_ADV || in_dims[s] == IN_GOOD, "es_apply: in_dim must be 8 or 10");
+        seg.in_dim[s] = in_dims[s];
+        off += fc_pitch(in_dims[s]);
+        seg.end[s] = off;
+    }
+    // Adam's bias-corrected step size in fp64, rounded once to fp32
+    const double step = optimizer == CEV_ES_ADAM
+        ? lr * sqrt(1.0 - pow(CEV_ADAM_BETA2, (double)t)) / (1.0 - pow(CEV_ADAM_BETA1, (double)t)) : lr;
+    CEV_GUARD(h);
+    es_apply_kernel<<<(unsigned)((off + PT - 1) / PT), PT, 0, (cudaStream_t)stream>>>(
+        theta, delta, m, v, seg, optimizer == CEV_ES_ADAM, (float)step, l2_coeff);
+    return check_cuda(cudaGetLastError(), "es_apply_kernel");
 }
 
 int cev_axpy_f32(cev_handle* h, float a, const float* x, float* y, int64_t n, cev_stream stream) {

@@ -128,6 +128,31 @@ def sync_torch_rng(comm, device="cpu"):
     torch.set_rng_state(buf.cpu())
 
 
+#: the opt-in Co-ES update options (Salimans et al. 2017) and their defaults, which run the reference's update
+ES_OPTION_DEFAULTS = {"mirrored_sampling": False, "fitness_shaping": "none", "es_optimizer": "sgd", "l2_coeff": 0.0}
+
+
+def es_options(args, algorithm=None):
+    """The Co-ES update options of ``args`` (an absent attribute is its default), validated: ``ValueError`` for an
+    unknown value, for mirrored sampling with an odd population and for any non-default option with the GA
+    (``algorithm``, or ``args.algorithm`` when not given)."""
+    opts = {k: getattr(args, k, d) for k, d in ES_OPTION_DEFAULTS.items()}
+    opts["mirrored_sampling"] = bool(opts["mirrored_sampling"])
+    opts["l2_coeff"] = float(opts["l2_coeff"])
+    if opts["fitness_shaping"] not in ("none", "centered_rank"):
+        raise ValueError(f"fitness_shaping must be 'none' or 'centered_rank', not {opts['fitness_shaping']!r}")
+    if opts["es_optimizer"] not in ("sgd", "adam"):
+        raise ValueError(f"es_optimizer must be 'sgd' or 'adam', not {opts['es_optimizer']!r}")
+    if not np.isfinite(opts["l2_coeff"]) or opts["l2_coeff"] < 0:
+        raise ValueError(f"l2_coeff must be a finite number >= 0, not {opts['l2_coeff']}")
+    if opts != ES_OPTION_DEFAULTS and (algorithm or getattr(args, "algorithm", "ES")) == "GA":
+        changed = sorted(k for k in opts if opts[k] != ES_OPTION_DEFAULTS[k])
+        raise ValueError(f"{', '.join(changed)}: Co-ES options, not available with --algorithm GA")
+    if opts["mirrored_sampling"] and int(args.population) % 2:
+        raise ValueError(f"mirrored sampling needs an even population, not {args.population}")
+    return opts
+
+
 def default_kernels():
     from . import ops
     return ops
@@ -418,6 +443,7 @@ class GAEngine(_EngineBase):
     def __init__(self, args, device, pop_rows, hof_rows, founder_rows, env=None, kernels=None, comm=None):
         super().__init__(args, device, env, kernels, comm)
         self.P = int(args.population)
+        es_options(args, "GA")                           # refuses the Co-ES options
         self.shard = Shard(self.P, self.comm.rank, self.comm.world)
         self.pop = {r: pop_rows[r].to(self.device).contiguous() for r in ROLES}       # [n_local, pitch]
         self.hof = {r: hof_rows[r].to(self.device).contiguous() for r in ROLES}       # [hof, pitch]
@@ -600,13 +626,24 @@ class GAEngine(_EngineBase):
 class ESEngine(_EngineBase):
     """State: one replicated base row per role.  Members of a generation are
     ``theta + sigma * N(0,1)`` regenerated from the Philox key both when they are
-    materialised for the rollout (K5) and when the update is formed (K6)."""
+    materialised for the rollout (K5) and when the update is formed (K6).
+
+    Opt-in update options (``es_options``): mirrored sampling (members 2q and 2q+1 are
+    ``theta +- sigma * z_q``), centered-rank fitness shaping of the global fitness, and an Adam step
+    and / or L2 weight decay applied by one fused kernel after the delta all-reduce (K6 then yields
+    the ascent estimate itself, at lr = 1).  Adam's moments ``m`` / ``v`` are laid out like
+    ``theta_cat`` and replicated like it."""
 
     kind = "ES"
 
     def __init__(self, args, device, theta_rows, env=None, kernels=None, comm=None):
         super().__init__(args, device, env, kernels, comm)
         self.P = int(args.population)
+        self.options = es_options(args, "ES")
+        self.mirrored = self.options["mirrored_sampling"]
+        self.shaping = self.options["fitness_shaping"] == "centered_rank"
+        #: the fused apply kernel instead of K6 at lr + axpy (the default path)
+        self.fused_apply = self.options["es_optimizer"] == "adam" or self.options["l2_coeff"] != 0.0
         self.shard = Shard(self.P, self.comm.rank, self.comm.world)
         pitches = [layout.fc_pitch(layout.OBS_DIM[r]) for r in ROLES]
         # the three base rows / deltas live in one buffer each: one all-reduce, one apply
@@ -619,9 +656,15 @@ class ESEngine(_EngineBase):
             self.theta[r].copy_(theta_rows[r].reshape(-1)[:pitch])
             off += pitch
         self.comm.broadcast0(self.theta_cat)              # rank 0's base agents everywhere (ADVICE r1)
+        self.adam_m = self.adam_v = None
+        if self.options["es_optimizer"] == "adam":
+            self.adam_m = torch.zeros_like(self.theta_cat)
+            self.adam_v = torch.zeros_like(self.theta_cat)
         self.members = {r: torch.empty((self.shard.n_local, layout.fc_pitch(layout.OBS_DIM[r])),
                                        dtype=torch.float32, device=self.device) for r in ROLES}
         self.fitness = {r: None for r in ROLES}
+        #: this rank's rows of the centered-rank shaped fitness the update used (fitness shaping only)
+        self.shaped_fitness = {r: None for r in ROLES}
         self.rewards = {r: None for r in ROLES}
         self.diversity = {r: None for r in ROLES}
         self.weight_stats = {r: None for r in ROLES}      # fp32 [n_local, 4] when args.log_member_weight_stats
@@ -658,8 +701,9 @@ class ESEngine(_EngineBase):
 
         def prepare(role):
             in_dim = layout.OBS_DIM[role]
-            self.k.es_perturb(self.theta[role], in_dim, self.sigma_dev(role), self.seed, role, self.gen,
-                              self.shard.row0, self.shard.n_local, out=self.members[role])
+            perturb = self.k.es_perturb_mirrored if self.mirrored else self.k.es_perturb
+            perturb(self.theta[role], in_dim, self.sigma_dev(role), self.seed, role, self.gen,
+                    self.shard.row0, self.shard.n_local, out=self.members[role])
             if self.member_stats:
                 # per-member statistics of the perturbed weights (MPE/mpe_agent.py:30-50, agent.py:66)
                 self.weight_stats[role] = self.k.weight_stats(self.members[role], in_dim)
@@ -705,23 +749,38 @@ class ESEngine(_EngineBase):
                 else:
                     self.fitness[role] = allp[:, i].contiguous()
 
-        if a.fitness_sharing:
-            finish_fitness()              # the update needs the shared fitness
+        need_global = a.fitness_sharing or self.shaping
+        if need_global:
+            finish_fitness()              # the update needs the shared fitness / the ranks of the global fitness
+        # with the fused apply K6 yields the ascent estimate ghat (lr = 1); the step size is applied after it
+        lr = 1.0 if self.fused_apply else a.learning_rate
         for role in ROLES:
             in_dim = layout.OBS_DIM[role]
+            fit = fit_local[role].contiguous()
+            if self.shaping:
+                # ranks over the global fitness (after sharing: its division by one positive scalar keeps the order)
+                fit = self.k.centered_ranks(self.fitness[role], self.shard.row0, self.shard.n_local)
+                self.shaped_fitness[role] = fit
             if self.update_from_members and hasattr(self.k, "es_update_members"):
                 # sigma*z_i read back from the materialised members (HBM bound) instead of regenerated
-                self.k.es_update_members(fit_local[role].contiguous(), self.members[role], self.theta[role],
-                                         in_dim, self.sigma_dev(role), a.learning_rate, self.P,
+                self.k.es_update_members(fit, self.members[role], self.theta[role],
+                                         in_dim, self.sigma_dev(role), lr, self.P,
                                          out=self.last_delta[role])
             else:
-                self.k.es_update(fit_local[role].contiguous(), in_dim, self.sigma_dev(role), a.learning_rate,
-                                 self.P, self.seed, role, self.gen, self.shard.row0, out=self.last_delta[role])
-        if not a.fitness_sharing:
+                update = self.k.es_update_mirrored if self.mirrored else self.k.es_update
+                update(fit, in_dim, self.sigma_dev(role), lr,
+                       self.P, self.seed, role, self.gen, self.shard.row0, out=self.last_delta[role])
+        if not need_global:
             finish_fitness()              # the global fitness is a record only: gathered under the three K6 launches
         self.comm.all_reduce_sum(self.delta_cat)
         self._join_eval()                 # the previous generation's evaluation games read theta
-        self.k.axpy(1.0, self.delta_cat, self.theta_cat)
+        if self.fused_apply:
+            # replicated on every rank from the same all-reduced delta: the replicas stay identical
+            self.k.es_apply(self.theta_cat, self.delta_cat, [layout.OBS_DIM[r] for r in ROLES],
+                            optimizer=self.options["es_optimizer"], lr=a.learning_rate,
+                            l2_coeff=self.options["l2_coeff"], t=self.gen + 1, m=self.adam_m, v=self.adam_v)
+        else:
+            self.k.axpy(1.0, self.delta_cat, self.theta_cat)
 
     def step(self, init_by_role=None, sync=True):
         """One generation.  ``sync=True`` returns the evaluation triple (one host read);
@@ -742,19 +801,31 @@ class ESEngine(_EngineBase):
                 diversity={r: (float(self.diversity[r]) if self.diversity[r] is not None else None) for r in ROLES},
                 evals=self.last_eval(),
                 delta={r: self.last_delta[r].cpu().numpy().copy() for r in ROLES},
+                shaped_fitness={r: (self.comm.all_gather_rows(self.shaped_fitness[r], self.shard).cpu().numpy().copy()
+                                    if self.shaping else None) for r in ROLES},
                 sigma={r: float(hs["sigma_history"][r][self.gen]) for r in ROLES}))
         self.gen += 1
         return self.last_eval() if sync else None
 
     def state_dict(self):
+        """Base rows, the update options and, for Adam, its moments (its step count is the generation count)."""
         sd = self._base_state()
-        sd.update(theta={r: self.theta[r].cpu().clone() for r in ROLES})
+        sd.update(theta={r: self.theta[r].cpu().clone() for r in ROLES}, es_options=dict(self.options))
+        if self.adam_m is not None:
+            sd.update(adam_m=self.adam_m.cpu().clone(), adam_v=self.adam_v.cpu().clone())
         return sd
 
     def load_state_dict(self, sd):
+        """Refuses a checkpoint written with other update options (one without them was written with the defaults)."""
+        saved = sd.get("es_options", ES_OPTION_DEFAULTS)
+        if saved != self.options:
+            raise ValueError(f"checkpoint was written with ES options {saved}, this run uses {self.options}")
         self._load_base_state(sd)
         for r in ROLES:
             self.theta[r].copy_(sd["theta"][r])
+        if self.adam_m is not None:
+            self.adam_m.copy_(sd["adam_m"])
+            self.adam_v.copy_(sd["adam_v"])
 
 
 def adapt_sigma(args, hist0, hist1, histadv, gen):

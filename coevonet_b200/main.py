@@ -65,6 +65,20 @@ def parse_arguments(argv=None):
                    help="ES update: regenerate sigma*z from the Philox key (the reference's exact `noises` array) "
                         "instead of reading it back as members - theta (faster, differs by the rounding of the "
                         "perturbation's add)")
+    p.add_argument("--mirrored_sampling", action="store_true",
+                   help="ES: members come in antithetic pairs theta +- sigma*z_q sharing one normal draw (Salimans et "
+                        "al. 2017); halves the noise generation; needs an even --population")
+    p.add_argument("--fitness_shaping", choices=["none", "centered_rank"], default="none",
+                   help="ES: weight the update by centered ranks r_i/(P-1) - 0.5 of the global fitness (ties share "
+                        "their average rank) instead of the raw fitness.  With --fitness_sharing the ranks are taken "
+                        "after its division, which divides every member by the same positive scalar and so does not "
+                        "change them")
+    p.add_argument("--es_optimizer", choices=["sgd", "adam"], default="sgd",
+                   help="ES: step along the update estimate with plain SGD (the reference) or Adam (b1 0.9, b2 0.999, "
+                        "eps 1e-8); --learning_rate is then Adam's step size, and 0.1, the reference's SGD default, is "
+                        "large for Adam (try 0.01)")
+    p.add_argument("--l2_coeff", type=float, default=0.0,
+                   help="ES: L2 weight decay, the step follows g = ghat - l2_coeff * theta (with sgd or adam)")
     p.add_argument("--play_discarded_hof_games", action="store_true",
                    help="GA, reference_compat: also simulate the hof_size-1 games per member whose reward the "
                         "reference overwrites (they never reach the fitness; skipped by default)")
@@ -142,6 +156,12 @@ class Args:
         self.resume = a.resume
         self.crossover_rate = a.crossover_rate
         self.log_member_weight_stats = a.log_member_weight_stats
+        self.mirrored_sampling = a.mirrored_sampling
+        self.fitness_shaping = a.fitness_shaping
+        self.es_optimizer = a.es_optimizer
+        self.l2_coeff = a.l2_coeff
+        from .engine import es_options
+        es_options(self)                  # ValueError: odd population with mirrored sampling, an ES option with GA
 
     def print_attributes(self, args=None):
         for k, v in vars(self).items():

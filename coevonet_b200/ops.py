@@ -16,7 +16,8 @@ from ._lib import RolloutCfg, check, handle, load
 MAX_CYCLES = 25
 
 #: kernels launched per C-ABI call (bench.py reports the total as ``gpu_launches``)
-_KERNELS_PER_CALL = {"cev_es_update_f32": 2, "cev_es_update_members_f32": 2, "cev_fp32_peak": 4}
+_KERNELS_PER_CALL = {"cev_es_update_f32": 2, "cev_es_update_members_f32": 2, "cev_es_update_mirrored_f32": 2,
+                     "cev_fp32_peak": 4}
 launch_count = 0
 
 
@@ -318,6 +319,17 @@ def select_topk(fitness, k, order=_lib.ORDER_STABLE_DESC):
 
 def es_perturb(theta, in_dim, sigma, seed, role, gen, row0, n_rows, *, out=None, noise_out=None):
     """K5: perturbed member rows theta + sigma*N(0,1) (Linear parameters only)."""
+    return _es_perturb("cev_es_perturb_f32", theta, in_dim, sigma, seed, role, gen, row0, n_rows, out, noise_out)
+
+
+def es_perturb_mirrored(theta, in_dim, sigma, seed, role, gen, row0, n_rows, *, out=None, noise_out=None):
+    """K5 with mirrored sampling: global member c = theta + s*sigma*z_q, pair q = c >> 1, s = +1 for even c and
+    -1 for odd c (one normal draw per pair); ``noise_out`` receives s*z."""
+    return _es_perturb("cev_es_perturb_mirrored_f32", theta, in_dim, sigma, seed, role, gen, row0, n_rows, out,
+                       noise_out)
+
+
+def _es_perturb(name, theta, in_dim, sigma, seed, role, gen, row0, n_rows, out, noise_out):
     dev = _need_cuda(theta, out, noise_out)
     pitch = layout.fc_pitch(in_dim)
     if theta.numel() < pitch:
@@ -326,9 +338,9 @@ def es_perturb(theta, in_dim, sigma, seed, role, gen, row0, n_rows, *, out=None,
         out = torch.empty((n_rows, pitch), dtype=torch.float32, device=dev)
     role_id = layout.ROLE_ID[role] if isinstance(role, str) else int(role)
     sig, sig_dev = _sigma_args(sigma)
-    check(_call("cev_es_perturb_f32", 
+    check(_call(name,
         _h(dev), _ptr(theta), int(in_dim), sig, sig_dev, int(seed), role_id, int(gen),
-        int(row0), int(n_rows), pitch, _ptr(out), _ptr(noise_out), _stream(dev)), "cev_es_perturb_f32")
+        int(row0), int(n_rows), pitch, _ptr(out), _ptr(noise_out), _stream(dev)), name)
     return out
 
 
@@ -352,6 +364,16 @@ def es_perturb_dqn(theta, c_in, n_actions, sigma, seed, role, gen, row0, n_rows,
 def es_update(fitness, in_dim, sigma, lr, n_total, seed, role, gen, row0, *, out=None):
     """K6: delta fp32[pitch] = lr/(n_total*sigma) * sum_i (sigma z_i) fitness_i over the
     local members [row0, row0+len(fitness))."""
+    return _es_update("cev_es_update_f32", fitness, in_dim, sigma, lr, n_total, seed, role, gen, row0, out)
+
+
+def es_update_mirrored(fitness, in_dim, sigma, lr, n_total, seed, role, gen, row0, *, out=None):
+    """K6 with mirrored sampling, noise regenerated: the delta of :func:`es_update` for the members
+    :func:`es_perturb_mirrored` writes (sigma z_i = s_i * sigma z_{i >> 1}, one draw per pair)."""
+    return _es_update("cev_es_update_mirrored_f32", fitness, in_dim, sigma, lr, n_total, seed, role, gen, row0, out)
+
+
+def _es_update(name, fitness, in_dim, sigma, lr, n_total, seed, role, gen, row0, out):
     dev = _need_cuda(fitness, out)
     if fitness.dtype != torch.float64:
         raise _lib.CevError("es_update: fitness must be float64")
@@ -360,10 +382,9 @@ def es_update(fitness, in_dim, sigma, lr, n_total, seed, role, gen, row0, *, out
         out = torch.empty(pitch, dtype=torch.float32, device=dev)
     role_id = layout.ROLE_ID[role] if isinstance(role, str) else int(role)
     sig, sig_dev = _sigma_args(sigma)
-    check(_call("cev_es_update_f32", 
+    check(_call(name,
         _h(dev), _ptr(fitness), int(in_dim), sig, sig_dev, float(lr), int(n_total),
-        int(seed), role_id, int(gen), int(row0), fitness.shape[0], _ptr(out), _stream(dev)),
-        "cev_es_update_f32")
+        int(seed), role_id, int(gen), int(row0), fitness.shape[0], _ptr(out), _stream(dev)), name)
     return out
 
 
@@ -428,6 +449,36 @@ def generation_end(eval_out, gstate, hist_capacity, *, agent_step_limit=None, re
                 int(bool(early_stopping)), float(min_delta), int(patience), _stream(dev)),
           "cev_generation_end_f64")
     return gstate
+
+
+def centered_ranks(fitness, row0=0, n_rows=None, *, out=None):
+    """Centered-rank fitness shaping: fp64[n_rows] = rank_i / (P-1) - 0.5 for the rows [row0, row0 + n_rows) of
+    the GLOBAL fitness fp64[P] (average ranks for ties, -0.0 == +0.0, NaNs tie below every number)."""
+    dev = _need_cuda(fitness, out)
+    if fitness.dtype != torch.float64 or fitness.dim() != 1:
+        raise _lib.CevError("centered_ranks: fitness must be float64 [P]")
+    P = fitness.shape[0]
+    n_rows = P - int(row0) if n_rows is None else int(n_rows)
+    if out is None:
+        out = torch.empty(n_rows, dtype=torch.float64, device=dev)
+    check(_call("cev_centered_ranks_f64", _h(dev), _ptr(fitness), P, int(row0), n_rows, _ptr(out), _stream(dev)),
+          "cev_centered_ranks_f64")
+    return out
+
+
+def es_apply(theta, delta, in_dims, *, optimizer="sgd", lr, l2_coeff=0.0, t=1, m=None, v=None):
+    """Fused ES apply over the FCNetwork rows of ``in_dims`` concatenated in ``theta`` / ``delta`` (and the Adam
+    moments ``m`` / ``v``, same layout): g = delta - l2_coeff * theta, then ``sgd``: theta += lr * g, or ``adam``
+    at step ``t`` (updates applied including this one).  Only the Linear entries change."""
+    dev = _need_cuda(theta, delta, m, v)
+    n = sum(layout.fc_pitch(d) for d in in_dims)
+    if any(x is not None and (x.dtype != torch.float32 or x.numel() != n) for x in (theta, delta, m, v)):
+        raise _lib.CevError(f"es_apply: theta / delta / m / v must be float32 [{n}]")
+    opt = {"sgd": _lib.ES_SGD, "adam": _lib.ES_ADAM}[optimizer]
+    dims = (ctypes.c_int * len(in_dims))(*[int(d) for d in in_dims])
+    check(_call("cev_es_apply_f32", _h(dev), _ptr(theta), _ptr(delta), _ptr(m), _ptr(v), len(in_dims), dims, opt,
+                float(lr), float(l2_coeff), int(t), _stream(dev)), "cev_es_apply_f32")
+    return theta
 
 
 def axpy(a, x, y):

@@ -54,6 +54,7 @@ typedef void* cev_stream;               /* cudaStream_t */
 #define CEV_KIND_FRAMES 3
 #define CEV_KIND_INIT 4
 #define CEV_KIND_XOVER 5
+#define CEV_KIND_ES_MIRROR 6            /* ES pair noise under mirrored sampling: member = pair id */
 
 int cev_version(void);
 const char* cev_last_error(void);
@@ -287,6 +288,65 @@ int cev_es_update_members_f32(cev_handle* h, const double* fitness, const float*
 
 /* theta[j] += delta[j] (evolutionary_strategy.py:259-265) */
 int cev_axpy_f32(cev_handle* h, float a, const float* x, float* y, int64_t n, cev_stream stream);
+
+/*
+ * Opt-in Co-ES update options (Salimans et al. 2017, "Evolution Strategies as a Scalable Alternative to
+ * RL"), extending compute_weight_update (evolutionary_strategy.py:120-148) and Agent.mutate_ES
+ * (agent.py:31-70).  None of them is used unless the caller asks for it.
+ *
+ * K5 with mirrored sampling: members come in pairs; global member c = theta + s*sigma*z_q on the Linear
+ * parameters, pair q = c >> 1, s = +1 for even c, -1 for odd c, z_q = Philox(seed, ES_MIRROR, role, gen,
+ * member=q).  The odd row is theta + (-(sigma*z)) with the even row's rounded product.  A pair cut by
+ * the shard boundary (row0 or row0 + n_rows odd) writes only its local row.  noise_out (optional)
+ * receives s*z.  Same arguments as cev_es_perturb_f32.
+ */
+int cev_es_perturb_mirrored_f32(cev_handle* h, const float* theta, int in_dim,
+                                float sigma, const double* sigma_dev, uint64_t seed, int role, uint32_t gen,
+                                int64_t row0, int64_t n_rows, int64_t pitch,
+                                float* out, float* noise_out, cev_stream stream);
+
+/*
+ * K6 with mirrored sampling, noise regenerated: the delta of cev_es_update_f32 for members
+ * s_c * sigma*z_{c>>1} (the rows cev_es_perturb_mirrored_f32 writes); z_q is generated once per pair.
+ * The terms are accumulated (fmaf) in row order within splits that start on even global rows, so the
+ * result is bit-identical to a per-member loop over the same splits.
+ */
+int cev_es_update_mirrored_f32(cev_handle* h, const double* fitness, int in_dim,
+                               float sigma, const double* sigma_dev, float lr, int64_t n_total,
+                               uint64_t seed, int role, uint32_t gen,
+                               int64_t row0, int64_t n_rows,
+                               float* delta, cev_stream stream);
+
+/*
+ * Centered-rank fitness shaping of rows [row0, row0 + n_rows) of the GLOBAL fitness[P] (fp64):
+ * out[r] = rank_i / (P-1) - 0.5 (0 when P = 1) for i = row0 + r, with the average rank
+ * rank_i = #{j : F_j < F_i} + (#{j : F_j == F_i} - 1) / 2 (ties share their average rank, -0.0 == +0.0,
+ * every NaN ties with every other NaN and ranks below every number).  Exact in fp64.
+ */
+int cev_centered_ranks_f64(cev_handle* h, const double* fitness, int64_t P, int64_t row0, int64_t n_rows,
+                           double* out, cev_stream stream);
+
+/*
+ * Fused ES apply over n_segments (<= 3) FCNetwork rows concatenated in one buffer, segment s of
+ * cev_fc_pitch(in_dims[s]) floats (in_dims: HOST array).  delta holds the ascent estimate
+ * ghat = 1/(n sigma) sum_i (sigma z_i) F_i (K6 with lr = 1, all-reduced).  g = ghat - l2_coeff * theta, then
+ *   CEV_ES_SGD:  theta += lr * g                                        (m, v unused, may be NULL)
+ *   CEV_ES_ADAM: m = b1 m + (1-b1) g,  v = b2 v + (1-b2) g g,
+ *                theta += alpha_t m / (sqrt(v) + eps),
+ *                alpha_t = lr sqrt(1 - b2^t) / (1 - b1^t) in fp64, rounded to fp32; t = updates applied
+ *                including this one (>= 1).  (The reference builds an Adam optimizer per agent and never
+ *                uses it, MPE/mpe_agent.py:20.)
+ * fp32, one IEEE-rounded operation at a time (no FMA contraction; 1-b1 and 1-b2 are rounded fp32
+ * differences).  Only the Linear (perturbable) entries change: LayerNorm entries and padding of theta, m
+ * and v keep their bits.
+ */
+#define CEV_ES_SGD 0
+#define CEV_ES_ADAM 1
+#define CEV_ADAM_BETA1 0.9
+#define CEV_ADAM_BETA2 0.999
+#define CEV_ADAM_EPS 1e-8
+int cev_es_apply_f32(cev_handle* h, float* theta, const float* delta, float* m, float* v, int n_segments,
+                     const int* in_dims, int optimizer, double lr, float l2_coeff, int t, cev_stream stream);
 
 /*
  * K7 -- fitness-sharing distances.  Replaces the distance loop of
