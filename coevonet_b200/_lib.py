@@ -99,6 +99,12 @@ _SIGNATURES = {
     "cev_centered_ranks_f64": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p]),
     "cev_es_apply_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, POINTER(c_int), c_int,
                                  c_double, c_float, c_int, c_void_p]),
+    "cev_es_perturb_diag_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_uint64, c_int, c_uint32,
+                                        c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),
+    "cev_es_update_diag_f32": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int64, c_uint64, c_int, c_uint32, c_int64,
+                                       c_int64, c_void_p, c_void_p, c_void_p]),
+    "cev_es_apply_diag_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, POINTER(c_int),
+                                      c_float, POINTER(c_double), c_float, c_float, c_void_p]),
     "cev_diversity_dist_f32": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_int,
                                        c_void_p, c_void_p]),
     "cev_deepqn_forward": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_void_p, c_int, c_int,

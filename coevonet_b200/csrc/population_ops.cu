@@ -87,14 +87,25 @@ __global__ void __launch_bounds__(PT) ga_repopulate_kernel(
 // perturbable or not as a whole (the LayerNorm float4s skip the Philox / Box-Muller work altogether).
 constexpr int K5T = 128;
 
+// Mutation power of K5: one scalar for the whole row (the isotropic search distribution), or a row of
+// per-parameter sigmas laid out like theta (separable NES), read as the float4 of parameters j .. j+3.
+struct ScalarSigma {
+    float s;
+    __device__ __forceinline__ float4 at(int) const { return make_float4(s, s, s, s); }
+};
+struct RowSigma {
+    const float* __restrict__ row;
+    __device__ __forceinline__ float4 at(int j) const { return __ldg(reinterpret_cast<const float4*>(row + j)); }
+};
+
 // One float4 (parameters j .. j+3) of K5.  `counter` is the Philox member word: the member id, or the pair id
 // q = c >> 1 under mirrored sampling, where the normals of one draw give the row theta + sigma z (`plus`, the
 // even member 2q) and the row theta - sigma z (`minus`, the odd member 2q+1) with the same rounded product.
 // A null row pointer skips that row (a pair cut by the shard boundary); noise rows receive +z / -z.
-template <bool MIRROR>
+template <bool MIRROR, class Sigma>
 __device__ __forceinline__ void es_perturb_float4(
-    const float* __restrict__ theta, const FcOffsets& o, int j4, float sigma, const PhiloxKeys& keys, uint32_t tag,
-    uint32_t gen, uint32_t counter, float* __restrict__ plus, float* __restrict__ minus,
+    const float* __restrict__ theta, const FcOffsets& o, int j4, const Sigma& sigma, const PhiloxKeys& keys,
+    uint32_t tag, uint32_t gen, uint32_t counter, float* __restrict__ plus, float* __restrict__ minus,
     float* __restrict__ noise_plus, float* __restrict__ noise_minus) {
     const int j = j4 * 4;
     const float4 pv = __ldg(reinterpret_cast<const float4*>(theta + j));
@@ -103,10 +114,12 @@ __device__ __forceinline__ void es_perturb_float4(
     float z[4] = {0.f, 0.f, 0.f, 0.f};
     if (j < o.total && fc_is_perturbable(o, j)) {
         normal4(keys, tag, gen, counter, (uint32_t)j4, z);
+        const float4 sv = sigma.at(j);
+        const float s[4] = {sv.x, sv.y, sv.z, sv.w};
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
             if (j + i < o.total) {
-                const float d = __fmul_rn(sigma, z[i]);
+                const float d = __fmul_rn(s[i], z[i]);
                 p[i] = __fadd_rn(p[i], d);
                 if (MIRROR) m[i] = __fadd_rn(m[i], -d);
             } else { z[i] = 0.f; p[i] = 0.f; m[i] = 0.f; }
@@ -134,7 +147,7 @@ __global__ void __launch_bounds__(K5T, 10) es_perturb_kernel(
     const int64_t c = row0 + r;
     const int j4 = blockIdx.y * K5T + threadIdx.x;
     if ((int64_t)j4 * 4 >= pitch) return;
-    es_perturb_float4<false>(theta, o, j4, sigma, keys, tag, gen, (uint32_t)c, out + r * pitch, nullptr,
+    es_perturb_float4<false>(theta, o, j4, ScalarSigma{sigma}, keys, tag, gen, (uint32_t)c, out + r * pitch, nullptr,
                              noise_out ? noise_out + r * pitch : nullptr, nullptr);
 }
 
@@ -153,10 +166,37 @@ __global__ void __launch_bounds__(K5T, 10) es_perturb_mirrored_kernel(
     const bool has_plus = r_plus >= 0, has_minus = r_minus < n_rows;
     const int j4 = blockIdx.y * K5T + threadIdx.x;
     if ((int64_t)j4 * 4 >= pitch) return;
-    es_perturb_float4<true>(theta, o, j4, sigma, keys, tag, gen, (uint32_t)q,
+    es_perturb_float4<true>(theta, o, j4, ScalarSigma{sigma}, keys, tag, gen, (uint32_t)q,
                             has_plus ? out + r_plus * pitch : nullptr, has_minus ? out + r_minus * pitch : nullptr,
                             noise_out && has_plus ? noise_out + r_plus * pitch : nullptr,
                             noise_out && has_minus ? noise_out + r_minus * pitch : nullptr);
+}
+
+// K5 of separable NES: member = theta + fl(sigma[j] z_j) with the per-parameter sigma row, on the CTA grid and
+// Philox streams of es_perturb_kernel (MIRROR = false) / es_perturb_mirrored_kernel (MIRROR = true), so a row of
+// sigma0 gives their members bit for bit.
+template <bool MIRROR>
+__global__ void __launch_bounds__(K5T, 10) es_perturb_diag_kernel(
+    const float* __restrict__ theta, const float* __restrict__ sigma, int in_dim, int64_t pitch,
+    const PhiloxKeys keys, uint32_t tag, uint32_t gen, int64_t row0, int64_t n_rows,
+    float* __restrict__ out, float* __restrict__ noise_out) {
+    const FcOffsets o = fc_offsets(in_dim);
+    const int j4 = blockIdx.y * K5T + threadIdx.x;
+    if ((int64_t)j4 * 4 >= pitch) return;
+    const RowSigma sig{sigma};
+    if (!MIRROR) {
+        const int64_t r = blockIdx.x;
+        es_perturb_float4<false>(theta, o, j4, sig, keys, tag, gen, (uint32_t)(row0 + r), out + r * pitch, nullptr,
+                                 noise_out ? noise_out + r * pitch : nullptr, nullptr);
+    } else {
+        const int64_t q = (row0 >> 1) + blockIdx.x;
+        const int64_t r_plus = 2 * q - row0, r_minus = r_plus + 1;
+        const bool has_plus = r_plus >= 0, has_minus = r_minus < n_rows;
+        es_perturb_float4<true>(theta, o, j4, sig, keys, tag, gen, (uint32_t)q,
+                                has_plus ? out + r_plus * pitch : nullptr, has_minus ? out + r_minus * pitch : nullptr,
+                                noise_out && has_plus ? noise_out + r_plus * pitch : nullptr,
+                                noise_out && has_minus ? noise_out + r_minus * pitch : nullptr);
+    }
 }
 
 // K5 for rows whose perturbable parameters are a PREFIX of the row: DeepQN rows hold the conv / Linear
@@ -194,14 +234,20 @@ __global__ void __launch_bounds__(PT) es_perturb_prefix_kernel(
 // Partial sum over the local rows [r_lo, r_hi) of split `sp`, in row order.  MIRROR: member c = row0 + r carries
 // s_c * (sigma z_q) with q = c >> 1, s_c = +1 for even c, -1 for odd c; z_q is generated once per pair, so the
 // terms, and their order, are those of the per-member loop (the negation is exact).
-template <bool MIRROR>
+//
+// DIAG (separable NES): no sigma; two sums of the raw normals, sum_i F_i z_i into `partial` and
+// sum_i F_i (z_i^2 - 1) into `partial_sigma` (the z^2 - 1 factor is fl(fl(z z) - 1); under mirroring (s z)^2 = z^2
+// exactly, so both members of a pair add the same factor).
+template <bool MIRROR, bool DIAG = false>
 __device__ __forceinline__ void es_update_partial_body(
     const double* __restrict__ fitness, int in_dim, int64_t pitch, float sigma, const PhiloxKeys& keys,
-    uint32_t tag, uint32_t gen, int64_t row0, int64_t r_lo, int64_t r_hi, int sp, float* __restrict__ partial) {
+    uint32_t tag, uint32_t gen, int64_t row0, int64_t r_lo, int64_t r_hi, int sp, float* __restrict__ partial,
+    float* __restrict__ partial_sigma = nullptr) {
     const FcOffsets o = fc_offsets(in_dim);
     const int j4 = blockIdx.x * PT + threadIdx.x;
     if ((int64_t)j4 * 4 >= pitch) return;
     float acc[4] = {0.f, 0.f, 0.f, 0.f};
+    float acc2[4] = {0.f, 0.f, 0.f, 0.f};
     bool pert[4];
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
@@ -215,33 +261,71 @@ __device__ __forceinline__ void es_update_partial_body(
                 float z[4];
                 normal4(keys, tag, gen, (uint32_t)(row0 + r), (uint32_t)j4, z);
 #pragma unroll
-                for (int i = 0; i < 4; ++i) acc[i] = fmaf(__fmul_rn(sigma, z[i]), f, acc[i]);
+                for (int i = 0; i < 4; ++i) {
+                    if (DIAG) {
+                        acc[i] = fmaf(z[i], f, acc[i]);
+                        acc2[i] = fmaf(__fsub_rn(__fmul_rn(z[i], z[i]), 1.f), f, acc2[i]);
+                    } else {
+                        acc[i] = fmaf(__fmul_rn(sigma, z[i]), f, acc[i]);
+                    }
+                }
             }
         } else {
             for (int64_t r = r_lo; r < r_hi;) {
                 const int64_t c = row0 + r;
-                float z[4];
+                float z[4], zz[4];
                 normal4(keys, tag, gen, (uint32_t)(c >> 1), (uint32_t)j4, z);
 #pragma unroll
-                for (int i = 0; i < 4; ++i) z[i] = __fmul_rn(sigma, z[i]);
+                for (int i = 0; i < 4; ++i) {
+                    if (DIAG) zz[i] = __fsub_rn(__fmul_rn(z[i], z[i]), 1.f);
+                    else z[i] = __fmul_rn(sigma, z[i]);
+                }
                 if (!(c & 1)) {
                     const float f = (float)fitness[r];
 #pragma unroll
-                    for (int i = 0; i < 4; ++i) acc[i] = fmaf(z[i], f, acc[i]);
+                    for (int i = 0; i < 4; ++i) {
+                        acc[i] = fmaf(z[i], f, acc[i]);
+                        if (DIAG) acc2[i] = fmaf(zz[i], f, acc2[i]);
+                    }
                     if (++r == r_hi) break;
                 }
                 const float f = (float)fitness[r];
 #pragma unroll
-                for (int i = 0; i < 4; ++i) acc[i] = fmaf(-z[i], f, acc[i]);
+                for (int i = 0; i < 4; ++i) {
+                    acc[i] = fmaf(-z[i], f, acc[i]);
+                    if (DIAG) acc2[i] = fmaf(zz[i], f, acc2[i]);
+                }
                 ++r;
             }
         }
     }
 #pragma unroll
     for (int i = 0; i < 4; ++i)
-        if (!pert[i]) acc[i] = 0.f;
+        if (!pert[i]) acc[i] = acc2[i] = 0.f;
     *reinterpret_cast<float4*>(partial + (int64_t)sp * pitch + (int64_t)j4 * 4) =
         make_float4(acc[0], acc[1], acc[2], acc[3]);
+    if (DIAG)
+        *reinterpret_cast<float4*>(partial_sigma + (int64_t)sp * pitch + (int64_t)j4 * 4) =
+            make_float4(acc2[0], acc2[1], acc2[2], acc2[3]);
+}
+
+// Local rows [r_lo, r_hi) of split sp.  Plain: n_split equal blocks of the local rows.  Mirrored sampling: the
+// splits cover GLOBAL rows [base + sp*per, base + (sp+1)*per) of this rank's block, with base = row0 rounded down
+// to even and `per` even, so every split but the first starts on a pair.
+template <bool MIRROR>
+__device__ __forceinline__ void es_update_split(int64_t row0, int64_t n_rows, int n_split, int sp, int64_t& r_lo,
+                                                int64_t& r_hi) {
+    if (!MIRROR) {
+        const int64_t per = (n_rows + n_split - 1) / n_split;
+        r_lo = sp * per;
+        r_hi = min(n_rows, r_lo + per);
+    } else {
+        const int64_t base = row0 & ~(int64_t)1;
+        const int64_t span = row0 + n_rows - base;
+        const int64_t per = ((span + n_split - 1) / n_split + 1) & ~(int64_t)1;
+        r_lo = max(base + sp * per, row0) - row0;
+        r_hi = min(base + (sp + 1) * per, row0 + n_rows) - row0;
+    }
 }
 
 __global__ void __launch_bounds__(PT) es_update_partial_kernel(
@@ -250,27 +334,52 @@ __global__ void __launch_bounds__(PT) es_update_partial_kernel(
     const PhiloxKeys keys, uint32_t tag, uint32_t gen, int64_t row0, int64_t n_rows,
     int n_split, float* __restrict__ partial) {
     const int sp = blockIdx.y;
-    const int64_t per = (n_rows + n_split - 1) / n_split;
-    const int64_t r_lo = sp * per, r_hi = min(n_rows, r_lo + per);
+    int64_t r_lo, r_hi;
+    es_update_split<false>(row0, n_rows, n_split, sp, r_lo, r_hi);
     es_update_partial_body<false>(fitness, in_dim, pitch, pick_sigma(sigma_arg, sigma_dev), keys, tag, gen, row0,
                                   r_lo, r_hi, sp, partial);
 }
 
-// Mirrored sampling: the splits cover GLOBAL rows [base + sp*per, base + (sp+1)*per) of this rank's block, with
-// base = row0 rounded down to even and `per` even, so every split but the first starts on a pair.
 __global__ void __launch_bounds__(PT) es_update_mirrored_partial_kernel(
     const double* __restrict__ fitness, int in_dim, int64_t pitch, float sigma_arg,
     const double* __restrict__ sigma_dev,
     const PhiloxKeys keys, uint32_t tag, uint32_t gen, int64_t row0, int64_t n_rows,
     int n_split, float* __restrict__ partial) {
     const int sp = blockIdx.y;
-    const int64_t base = row0 & ~(int64_t)1;
-    const int64_t span = row0 + n_rows - base;
-    const int64_t per = ((span + n_split - 1) / n_split + 1) & ~(int64_t)1;
-    const int64_t r_lo = max(base + sp * per, row0) - row0;
-    const int64_t r_hi = min(base + (sp + 1) * per, row0 + n_rows) - row0;
+    int64_t r_lo, r_hi;
+    es_update_split<true>(row0, n_rows, n_split, sp, r_lo, r_hi);
     es_update_partial_body<true>(fitness, in_dim, pitch, pick_sigma(sigma_arg, sigma_dev), keys, tag, gen, row0,
                                  r_lo, r_hi, sp, partial);
+}
+
+// K6 of separable NES, noise regenerated: partial sums of F_i z_i and F_i (z_i^2 - 1) over the splits of the plain /
+// mirrored K6.  partial_sigma = partial + n_split * pitch.
+template <bool MIRROR>
+__global__ void __launch_bounds__(PT) es_update_diag_partial_kernel(
+    const double* __restrict__ fitness, int in_dim, int64_t pitch, const PhiloxKeys keys, uint32_t tag, uint32_t gen,
+    int64_t row0, int64_t n_rows, int n_split, float* __restrict__ partial) {
+    const int sp = blockIdx.y;
+    int64_t r_lo, r_hi;
+    es_update_split<MIRROR>(row0, n_rows, n_split, sp, r_lo, r_hi);
+    es_update_partial_body<MIRROR, true>(fitness, in_dim, pitch, 0.f, keys, tag, gen, row0, r_lo, r_hi, sp, partial,
+                                         partial + (int64_t)n_split * pitch);
+}
+
+// g_mu = fl32(1/n_total) * (sum of the splits in order), g_sigma likewise from the second half of the workspace
+__global__ void __launch_bounds__(PT) es_update_diag_finish_kernel(
+    const float* __restrict__ partial, int n_split, int64_t pitch, double n_total, float* __restrict__ g_mu,
+    float* __restrict__ g_sigma) {
+    const int64_t j = (int64_t)blockIdx.x * PT + threadIdx.x;
+    if (j >= pitch) return;
+    const float inv_n = (float)(1.0 / n_total);
+    const float* partial_sigma = partial + (int64_t)n_split * pitch;
+    float s = 0.f, t = 0.f;
+    for (int sp = 0; sp < n_split; ++sp) {
+        s += partial[(int64_t)sp * pitch + j];
+        t += partial_sigma[(int64_t)sp * pitch + j];
+    }
+    g_mu[j] = __fmul_rn(inv_n, s);
+    g_sigma[j] = __fmul_rn(inv_n, t);
 }
 
 // The same partial sums from the MATERIALISED members: sigma z_i = member_i - theta up to one rounding
@@ -403,6 +512,36 @@ __global__ void __launch_bounds__(PT) es_apply_kernel(float* __restrict__ theta,
     m[i] = mi;
     v[i] = vi;
     theta[i] = __fadd_rn(th, __fdiv_rn(__fmul_rn(step, mi), __fadd_rn(__fsqrt_rn(vi), eps)));
+}
+
+// Separable NES apply (Wierstra et al. 2014, SNES) over the same concatenated rows, perturbable entries only:
+//   theta += fl(lr * fl(sigma * g_mu))                          (the old sigma)
+//   sigma  = clamp(fl(sigma * fl32(exp(half_eta[s] * g_sigma))), sigma_min, sigma_max)     (exp in fp64)
+// half_eta[s] = eta_sigma / 2 of segment s.  fminf / fmaxf: a NaN product clamps to sigma_min.
+struct DiagEta {
+    double half[CEV_MAX_ROLES];
+};
+
+__global__ void __launch_bounds__(PT) es_apply_diag_kernel(float* __restrict__ theta, float* __restrict__ sigma,
+                                                           const float* __restrict__ g_mu,
+                                                           const float* __restrict__ g_sigma, const ApplySegments seg,
+                                                           const DiagEta eta, float lr, float sigma_min,
+                                                           float sigma_max) {
+    const int64_t i = (int64_t)blockIdx.x * PT + threadIdx.x;
+    int in_dim = seg.in_dim[0];
+    double half_eta = eta.half[0];
+    int64_t start = 0, end = seg.end[0];
+#pragma unroll
+    for (int s = 1; s < CEV_MAX_ROLES; ++s)          // constant indices: the tables stay in registers
+        if (s < seg.n && i >= end) { in_dim = seg.in_dim[s]; half_eta = eta.half[s]; start = end; end = seg.end[s]; }
+    if (i >= end) return;
+    const FcOffsets o = fc_offsets(in_dim);
+    const int j = (int)(i - start);
+    if (j >= o.total || !fc_is_perturbable(o, j)) return;
+    const float s = sigma[i];
+    theta[i] = __fadd_rn(theta[i], __fmul_rn(lr, __fmul_rn(s, g_mu[i])));
+    const float factor = (float)exp(__dmul_rn(half_eta, (double)g_sigma[i]));
+    sigma[i] = fminf(fmaxf(__fmul_rn(s, factor), sigma_min), sigma_max);
 }
 
 // ---------------------------------------------------------------------------
@@ -1034,6 +1173,93 @@ int cev_es_apply_f32(cev_handle* h, float* theta, const float* delta, float* m, 
     es_apply_kernel<<<(unsigned)((off + PT - 1) / PT), PT, 0, (cudaStream_t)stream>>>(
         theta, delta, m, v, seg, optimizer == CEV_ES_ADAM, (float)step, l2_coeff);
     return check_cuda(cudaGetLastError(), "es_apply_kernel");
+}
+
+int cev_es_perturb_diag_f32(cev_handle* h, const float* theta, const float* sigma, int in_dim, int mirrored,
+                            uint64_t seed, int role, uint32_t gen, int64_t row0, int64_t n_rows, int64_t pitch,
+                            float* out, float* noise_out, cev_stream stream) {
+    CEV_REQUIRE(h != nullptr, "es_perturb_diag: null handle");
+    if (n_rows == 0) return CEV_OK;                   // an empty shard contributes nothing
+    CEV_REQUIRE(theta && sigma && out, "es_perturb_diag: null pointer");
+    CEV_REQUIRE(in_dim == IN_ADV || in_dim == IN_GOOD, "es_perturb_diag: in_dim must be 8 or 10");
+    CEV_REQUIRE(pitch >= fc_offsets(in_dim).total && pitch % 4 == 0, "es_perturb_diag: bad pitch");
+    CEV_REQUIRE(aligned16(theta) && aligned16(sigma) && aligned16(out) && aligned16(noise_out),
+                "es_perturb_diag: 16B alignment");
+    CEV_REQUIRE(row0 >= 0 && n_rows >= 0 && row0 + n_rows <= 0xFFFFFFFFll, "es_perturb_diag: bad row range");
+    CEV_GUARD(h);
+    uint32_t k0, k1;
+    split_seed(seed, k0, k1);
+    const unsigned ny = (unsigned)((pitch / 4 + K5T - 1) / K5T);
+    if (mirrored) {
+        const int64_t n_pairs = ((row0 + n_rows - 1) >> 1) - (row0 >> 1) + 1;
+        es_perturb_diag_kernel<true><<<dim3((unsigned)n_pairs, ny), K5T, 0, (cudaStream_t)stream>>>(
+            theta, sigma, in_dim, pitch, philox_keys(k0, k1), noise_tag(CEV_KIND_ES_MIRROR, role), gen, row0, n_rows,
+            out, noise_out);
+    } else {
+        es_perturb_diag_kernel<false><<<dim3((unsigned)n_rows, ny), K5T, 0, (cudaStream_t)stream>>>(
+            theta, sigma, in_dim, pitch, philox_keys(k0, k1), noise_tag(CEV_KIND_ES, role), gen, row0, n_rows, out,
+            noise_out);
+    }
+    return check_cuda(cudaGetLastError(), "es_perturb_diag_kernel");
+}
+
+int cev_es_update_diag_f32(cev_handle* h, const double* fitness, int in_dim, int mirrored, int64_t n_total,
+                           uint64_t seed, int role, uint32_t gen, int64_t row0, int64_t n_rows, float* g_mu,
+                           float* g_sigma, cev_stream stream) {
+    // an empty shard (n_rows == 0, fitness may be null) still writes its all-zero partial sums
+    CEV_REQUIRE(h && (fitness || n_rows == 0) && g_mu && g_sigma, "es_update_diag: null pointer");
+    CEV_REQUIRE(in_dim == IN_ADV || in_dim == IN_GOOD, "es_update_diag: in_dim must be 8 or 10");
+    CEV_REQUIRE(n_total >= 1 && n_rows >= 0, "es_update_diag: bad n");
+    CEV_REQUIRE(row0 >= 0 && row0 + n_rows <= 0xFFFFFFFFll, "es_update_diag: bad row range");
+    CEV_REQUIRE(aligned16(g_mu) && aligned16(g_sigma), "es_update_diag: 16B alignment");
+    CEV_GUARD(h);
+    const int64_t pitch = fc_pitch(in_dim);
+    int n_split = (int)((n_rows + 63) / 64);         // the splits of cev_es_update_f32 / cev_es_update_mirrored_f32
+    if (n_split > 16) n_split = 16;
+    if (n_split < 1) n_split = 1;
+    int rc = ensure_workspace(h, (size_t)2 * n_split * pitch * sizeof(float));
+    if (rc) return rc;
+    uint32_t k0, k1;
+    split_seed(seed, k0, k1);
+    float* partial = static_cast<float*>(h->workspace);
+    dim3 grid((unsigned)((pitch / 4 + PT - 1) / PT), (unsigned)n_split);
+    if (mirrored)
+        es_update_diag_partial_kernel<true><<<grid, PT, 0, (cudaStream_t)stream>>>(
+            fitness, in_dim, pitch, philox_keys(k0, k1), noise_tag(CEV_KIND_ES_MIRROR, role), gen, row0, n_rows,
+            n_split, partial);
+    else
+        es_update_diag_partial_kernel<false><<<grid, PT, 0, (cudaStream_t)stream>>>(
+            fitness, in_dim, pitch, philox_keys(k0, k1), noise_tag(CEV_KIND_ES, role), gen, row0, n_rows, n_split,
+            partial);
+    CEV_CUDA(cudaGetLastError());
+    es_update_diag_finish_kernel<<<(unsigned)((pitch + PT - 1) / PT), PT, 0, (cudaStream_t)stream>>>(
+        partial, n_split, pitch, (double)n_total, g_mu, g_sigma);
+    return check_cuda(cudaGetLastError(), "es_update_diag kernels");
+}
+
+int cev_es_apply_diag_f32(cev_handle* h, float* theta, float* sigma, const float* g_mu, const float* g_sigma,
+                          int n_segments, const int* in_dims, float lr, const double* sigma_lr, float sigma_min,
+                          float sigma_max, cev_stream stream) {
+    CEV_REQUIRE(h && theta && sigma && g_mu && g_sigma && in_dims && sigma_lr, "es_apply_diag: null pointer");
+    CEV_REQUIRE(n_segments >= 1 && n_segments <= CEV_MAX_ROLES, "es_apply_diag: need 1 <= n_segments <= %d",
+                CEV_MAX_ROLES);
+    CEV_REQUIRE(sigma_min > 0.f && sigma_min <= sigma_max, "es_apply_diag: need 0 < sigma_min <= sigma_max");
+    ApplySegments seg{};
+    DiagEta eta{};
+    seg.n = n_segments;
+    int64_t off = 0;
+    for (int s = 0; s < n_segments; ++s) {
+        CEV_REQUIRE(in_dims[s] == IN_ADV || in_dims[s] == IN_GOOD, "es_apply_diag: in_dim must be 8 or 10");
+        CEV_REQUIRE(sigma_lr[s] > 0.0 && std::isfinite(sigma_lr[s]), "es_apply_diag: sigma_lr must be finite and > 0");
+        seg.in_dim[s] = in_dims[s];
+        eta.half[s] = 0.5 * sigma_lr[s];
+        off += fc_pitch(in_dims[s]);
+        seg.end[s] = off;
+    }
+    CEV_GUARD(h);
+    es_apply_diag_kernel<<<(unsigned)((off + PT - 1) / PT), PT, 0, (cudaStream_t)stream>>>(
+        theta, sigma, g_mu, g_sigma, seg, eta, lr, sigma_min, sigma_max);
+    return check_cuda(cudaGetLastError(), "es_apply_diag_kernel");
 }
 
 int cev_axpy_f32(cev_handle* h, float a, const float* x, float* y, int64_t n, cev_stream stream) {

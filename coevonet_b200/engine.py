@@ -153,6 +153,43 @@ def es_options(args, algorithm=None):
     return opts
 
 
+#: the Co-ES search distribution and its default: one isotropic Gaussian per role (the reference), or separable NES
+#: (a per-parameter mutation strength, Schaul et al. 2011); sigma_learning_rate None = default_sigma_learning_rate
+ES_DISTRIBUTION_DEFAULTS = {"es_distribution": "isotropic", "sigma_learning_rate": None}
+
+
+def es_distribution(args, algorithm=None):
+    """The Co-ES search distribution settings of ``args`` (an absent attribute is its default), validated:
+    ``ValueError`` for an unknown distribution, for any non-default setting with the GA, for ``separable`` with
+    Adam, L2 weight decay or ``--adaptive`` (they would fight the per-parameter step) and for a
+    ``sigma_learning_rate`` that is not a finite number > 0 or is given without ``separable``."""
+    opts = {k: getattr(args, k, d) for k, d in ES_DISTRIBUTION_DEFAULTS.items()}
+    if opts["es_distribution"] not in ("isotropic", "separable"):
+        raise ValueError(f"es_distribution must be 'isotropic' or 'separable', not {opts['es_distribution']!r}")
+    if opts != ES_DISTRIBUTION_DEFAULTS and (algorithm or getattr(args, "algorithm", "ES")) == "GA":
+        changed = sorted(k for k in opts if opts[k] != ES_DISTRIBUTION_DEFAULTS[k])
+        raise ValueError(f"{', '.join(changed)}: Co-ES options, not available with --algorithm GA")
+    separable = opts["es_distribution"] == "separable"
+    if opts["sigma_learning_rate"] is not None:
+        opts["sigma_learning_rate"] = float(opts["sigma_learning_rate"])
+        if not separable:
+            raise ValueError("sigma_learning_rate needs es_distribution 'separable'")
+        if not np.isfinite(opts["sigma_learning_rate"]) or opts["sigma_learning_rate"] <= 0:
+            raise ValueError(f"sigma_learning_rate must be a finite number > 0, not {opts['sigma_learning_rate']}")
+    if separable:
+        if getattr(args, "es_optimizer", "sgd") != "sgd" or float(getattr(args, "l2_coeff", 0.0)) != 0.0:
+            raise ValueError("es_distribution 'separable' takes its own step: not available with es_optimizer "
+                             "'adam' or a nonzero l2_coeff")
+        if getattr(args, "adaptive", False):
+            raise ValueError("es_distribution 'separable' adapts every sigma itself: not available with --adaptive")
+    return opts
+
+
+def default_sigma_learning_rate(d):
+    """SNES's sigma learning rate for d parameters, (3 + ln d) / (5 sqrt d) (Schaul et al. 2011), in fp64."""
+    return (3.0 + np.log(float(d))) / (5.0 * np.sqrt(float(d)))
+
+
 def default_kernels():
     from . import ops
     return ops
@@ -444,6 +481,7 @@ class GAEngine(_EngineBase):
         super().__init__(args, device, env, kernels, comm)
         self.P = int(args.population)
         es_options(args, "GA")                           # refuses the Co-ES options
+        es_distribution(args, "GA")
         self.shard = Shard(self.P, self.comm.rank, self.comm.world)
         self.pop = {r: pop_rows[r].to(self.device).contiguous() for r in ROLES}       # [n_local, pitch]
         self.hof = {r: hof_rows[r].to(self.device).contiguous() for r in ROLES}       # [hof, pitch]
@@ -632,7 +670,11 @@ class ESEngine(_EngineBase):
     ``theta +- sigma * z_q``), centered-rank fitness shaping of the global fitness, and an Adam step
     and / or L2 weight decay applied by one fused kernel after the delta all-reduce (K6 then yields
     the ascent estimate itself, at lr = 1).  Adam's moments ``m`` / ``v`` are laid out like
-    ``theta_cat`` and replicated like it."""
+    ``theta_cat`` and replicated like it.
+
+    Opt-in search distribution (``es_distribution``): separable NES keeps a per-parameter sigma
+    (``sigma_cat``, laid out like ``theta_cat`` and replicated like it) that the population's rewards adapt
+    through the natural gradient of log sigma; K5 / K6 / the apply become their diag forms."""
 
     kind = "ES"
 
@@ -656,6 +698,31 @@ class ESEngine(_EngineBase):
             self.theta[r].copy_(theta_rows[r].reshape(-1)[:pitch])
             off += pitch
         self.comm.broadcast0(self.theta_cat)              # rank 0's base agents everywhere (ADVICE r1)
+        self.distribution = es_distribution(args, "ES")
+        self.separable = self.distribution["es_distribution"] == "separable"
+        self.sigma_cat = self.grad_cat = None
+        self.sigma_rows, self.sigma_grad, self.sigma_lr = {}, {}, {}
+        if self.separable:
+            # per-parameter sigma laid out like theta_cat (sigma0 on the Linear entries, 0 elsewhere), replicated like
+            # it; grad_cat = [g_mu of the roles | g_sigma of the roles]: still one all-reduce per generation
+            n = self.theta_cat.numel()
+            self.sigma_cat = torch.zeros(n, dtype=torch.float32, device=self.device)
+            self.grad_cat = torch.zeros(2 * n, dtype=torch.float32, device=self.device)
+            self.delta_cat = self.grad_cat[:n]
+            sigma0 = {"agent_0": args.mutation_power_agent_0, "agent_1": args.mutation_power_agent_1,
+                      "adversary_0": args.mutation_power_adversary}
+            off = 0
+            for r, pitch in zip(ROLES, pitches):
+                pidx = torch.from_numpy(layout.fc_perturbable_index(layout.OBS_DIM[r]))
+                row = torch.zeros(pitch, dtype=torch.float32)
+                row[pidx] = float(np.float32(sigma0[r]))
+                self.sigma_rows[r] = self.sigma_cat[off:off + pitch]
+                self.sigma_rows[r].copy_(row)
+                self.last_delta[r] = self.grad_cat[off:off + pitch]
+                self.sigma_grad[r] = self.grad_cat[n + off:n + off + pitch]
+                lr = self.distribution["sigma_learning_rate"]
+                self.sigma_lr[r] = float(lr) if lr is not None else default_sigma_learning_rate(len(pidx))
+                off += pitch
         self.adam_m = self.adam_v = None
         if self.options["es_optimizer"] == "adam":
             self.adam_m = torch.zeros_like(self.theta_cat)
@@ -701,9 +768,14 @@ class ESEngine(_EngineBase):
 
         def prepare(role):
             in_dim = layout.OBS_DIM[role]
-            perturb = self.k.es_perturb_mirrored if self.mirrored else self.k.es_perturb
-            perturb(self.theta[role], in_dim, self.sigma_dev(role), self.seed, role, self.gen,
-                    self.shard.row0, self.shard.n_local, out=self.members[role])
+            if self.separable:
+                self.k.es_perturb_diag(self.theta[role], self.sigma_rows[role], in_dim, self.seed, role, self.gen,
+                                       self.shard.row0, self.shard.n_local, mirrored=self.mirrored,
+                                       out=self.members[role])
+            else:
+                perturb = self.k.es_perturb_mirrored if self.mirrored else self.k.es_perturb
+                perturb(self.theta[role], in_dim, self.sigma_dev(role), self.seed, role, self.gen,
+                        self.shard.row0, self.shard.n_local, out=self.members[role])
             if self.member_stats:
                 # per-member statistics of the perturbed weights (MPE/mpe_agent.py:30-50, agent.py:66)
                 self.weight_stats[role] = self.k.weight_stats(self.members[role], in_dim)
@@ -761,7 +833,11 @@ class ESEngine(_EngineBase):
                 # ranks over the global fitness (after sharing: its division by one positive scalar keeps the order)
                 fit = self.k.centered_ranks(self.fitness[role], self.shard.row0, self.shard.n_local)
                 self.shaped_fitness[role] = fit
-            if self.update_from_members and hasattr(self.k, "es_update_members"):
+            if self.separable:
+                # always from regenerated noise: z = (member - theta) / sigma would not be exact
+                self.k.es_update_diag(fit, in_dim, self.P, self.seed, role, self.gen, self.shard.row0,
+                                      mirrored=self.mirrored, g_mu=self.last_delta[role], g_sigma=self.sigma_grad[role])
+            elif self.update_from_members and hasattr(self.k, "es_update_members"):
                 # sigma*z_i read back from the materialised members (HBM bound) instead of regenerated
                 self.k.es_update_members(fit, self.members[role], self.theta[role],
                                          in_dim, self.sigma_dev(role), lr, self.P,
@@ -772,9 +848,16 @@ class ESEngine(_EngineBase):
                        self.P, self.seed, role, self.gen, self.shard.row0, out=self.last_delta[role])
         if not need_global:
             finish_fitness()              # the global fitness is a record only: gathered under the three K6 launches
-        self.comm.all_reduce_sum(self.delta_cat)
+        self.comm.all_reduce_sum(self.grad_cat if self.separable else self.delta_cat)
         self._join_eval()                 # the previous generation's evaluation games read theta
-        if self.fused_apply:
+        if self.separable:
+            # replicated on every rank from the same all-reduced gradients: the replicas stay identical
+            n = self.theta_cat.numel()
+            self.k.es_apply_diag(self.theta_cat, self.sigma_cat, self.grad_cat[:n], self.grad_cat[n:],
+                                 [layout.OBS_DIM[r] for r in ROLES], lr=a.learning_rate,
+                                 sigma_lr=[self.sigma_lr[r] for r in ROLES], sigma_min=a.min_mutation_power,
+                                 sigma_max=a.max_mutation_power)
+        elif self.fused_apply:
             # replicated on every rank from the same all-reduced delta: the replicas stay identical
             self.k.es_apply(self.theta_cat, self.delta_cat, [layout.OBS_DIM[r] for r in ROLES],
                             optimizer=self.options["es_optimizer"], lr=a.learning_rate,
@@ -803,26 +886,46 @@ class ESEngine(_EngineBase):
                 delta={r: self.last_delta[r].cpu().numpy().copy() for r in ROLES},
                 shaped_fitness={r: (self.comm.all_gather_rows(self.shaped_fitness[r], self.shard).cpu().numpy().copy()
                                     if self.shaping else None) for r in ROLES},
-                sigma={r: float(hs["sigma_history"][r][self.gen]) for r in ROLES}))
+                sigma={r: float(hs["sigma_history"][r][self.gen]) for r in ROLES},
+                sigma_stats={r: self._sigma_stats(r) for r in ROLES}))
         self.gen += 1
         return self.last_eval() if sync else None
 
+    def _sigma_stats(self, role):
+        """(mean, min, max, std) of the role's per-parameter sigma after this generation's update over its Linear
+        entries (separable NES), None for the isotropic distribution."""
+        if not self.separable:
+            return None
+        st = self.k.weight_stats(self.sigma_rows[role].reshape(1, -1), layout.OBS_DIM[role])
+        return tuple(float(x) for x in st[0].cpu().tolist())
+
     def state_dict(self):
-        """Base rows, the update options and, for Adam, its moments (its step count is the generation count)."""
+        """Base rows, the update options and search distribution settings, for Adam its moments (its step count is
+        the generation count) and for separable NES the per-parameter sigmas."""
         sd = self._base_state()
-        sd.update(theta={r: self.theta[r].cpu().clone() for r in ROLES}, es_options=dict(self.options))
+        sd.update(theta={r: self.theta[r].cpu().clone() for r in ROLES}, es_options=dict(self.options),
+                  es_distribution=dict(self.distribution))
         if self.adam_m is not None:
             sd.update(adam_m=self.adam_m.cpu().clone(), adam_v=self.adam_v.cpu().clone())
+        if self.separable:
+            sd.update(sigma=self.sigma_cat.cpu().clone())
         return sd
 
     def load_state_dict(self, sd):
-        """Refuses a checkpoint written with other update options (one without them was written with the defaults)."""
+        """Refuses a checkpoint written with other update options or search distribution settings (one without
+        them was written with the defaults)."""
         saved = sd.get("es_options", ES_OPTION_DEFAULTS)
         if saved != self.options:
             raise ValueError(f"checkpoint was written with ES options {saved}, this run uses {self.options}")
+        saved = sd.get("es_distribution", ES_DISTRIBUTION_DEFAULTS)
+        if saved != self.distribution:
+            raise ValueError(f"checkpoint was written with the ES distribution {saved}, this run uses "
+                             f"{self.distribution}")
         self._load_base_state(sd)
         for r in ROLES:
             self.theta[r].copy_(sd["theta"][r])
+        if self.separable:
+            self.sigma_cat.copy_(sd["sigma"])
         if self.adam_m is not None:
             self.adam_m.copy_(sd["adam_m"])
             self.adam_v.copy_(sd["adam_v"])

@@ -79,6 +79,16 @@ def parse_arguments(argv=None):
                         "large for Adam (try 0.01)")
     p.add_argument("--l2_coeff", type=float, default=0.0,
                    help="ES: L2 weight decay, the step follows g = ghat - l2_coeff * theta (with sgd or adam)")
+    p.add_argument("--es_distribution", choices=["isotropic", "separable"], default="isotropic",
+                   help="ES: search with one mutation power per role (isotropic, the reference) or with one per "
+                        "parameter adapted by separable NES (Schaul et al. 2011): sigma starts at "
+                        "--initial_mutation_power_*, moves by exp(sigma_learning_rate/2 * g_sigma) every generation and "
+                        "stays in [--min_mutation_power, --max_mutation_power]; --learning_rate is then SNES's "
+                        "eta_mu (1.0 is the textbook value; the default stays the reference's 0.1).  Not with "
+                        "--es_optimizer adam, --l2_coeff or --adaptive")
+    p.add_argument("--sigma_learning_rate", type=float, default=None,
+                   help="ES, separable: learning rate of log sigma for all roles (default: (3 + ln d) / (5 sqrt d) "
+                        "per role, d = its number of Linear parameters)")
     p.add_argument("--play_discarded_hof_games", action="store_true",
                    help="GA, reference_compat: also simulate the hof_size-1 games per member whose reward the "
                         "reference overwrites (they never reach the fitness; skipped by default)")
@@ -160,8 +170,11 @@ class Args:
         self.fitness_shaping = a.fitness_shaping
         self.es_optimizer = a.es_optimizer
         self.l2_coeff = a.l2_coeff
-        from .engine import es_options
+        self.es_distribution = a.es_distribution
+        self.sigma_learning_rate = a.sigma_learning_rate
+        from .engine import es_distribution, es_options
         es_options(self)                  # ValueError: odd population with mirrored sampling, an ES option with GA
+        es_distribution(self)
 
     def print_attributes(self, args=None):
         for k, v in vars(self).items():

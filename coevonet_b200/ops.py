@@ -17,7 +17,7 @@ MAX_CYCLES = 25
 
 #: kernels launched per C-ABI call (bench.py reports the total as ``gpu_launches``)
 _KERNELS_PER_CALL = {"cev_es_update_f32": 2, "cev_es_update_members_f32": 2, "cev_es_update_mirrored_f32": 2,
-                     "cev_fp32_peak": 4}
+                     "cev_es_update_diag_f32": 2, "cev_fp32_peak": 4}
 launch_count = 0
 
 
@@ -479,6 +479,70 @@ def es_apply(theta, delta, in_dims, *, optimizer="sgd", lr, l2_coeff=0.0, t=1, m
     check(_call("cev_es_apply_f32", _h(dev), _ptr(theta), _ptr(delta), _ptr(m), _ptr(v), len(in_dims), dims, opt,
                 float(lr), float(l2_coeff), int(t), _stream(dev)), "cev_es_apply_f32")
     return theta
+
+
+def _need_f32(name, x, n):
+    if x.dtype != torch.float32 or x.dim() != 1 or x.numel() != n:
+        raise _lib.CevError(f"{name}: need a float32 [{n}] vector, got {tuple(x.shape)} {x.dtype}")
+
+
+def es_perturb_diag(theta, sigma, in_dim, seed, role, gen, row0, n_rows, *, mirrored=False, out=None,
+                    noise_out=None):
+    """K5 of separable NES: member rows theta + fl(sigma * z) with the per-parameter sigma row fp32[pitch] (Linear
+    parameters only).  z is the normal stream of :func:`es_perturb` (``mirrored`` False) or of
+    :func:`es_perturb_mirrored` (True), so a sigma row of sigma0 gives their rows bit for bit; ``noise_out``
+    receives s*z."""
+    dev = _need_cuda(theta, sigma, out, noise_out)
+    pitch = layout.fc_pitch(in_dim)
+    _need_f32("es_perturb_diag: theta", theta, pitch)
+    _need_f32("es_perturb_diag: sigma", sigma, pitch)
+    for name, t in (("out", out), ("noise_out", noise_out)):
+        if t is not None and (t.dtype != torch.float32 or tuple(t.shape) != (int(n_rows), pitch)):
+            raise _lib.CevError(f"es_perturb_diag: {name} must be float32 [{n_rows}, {pitch}]")
+    if out is None:
+        out = torch.empty((n_rows, pitch), dtype=torch.float32, device=dev)
+    role_id = layout.ROLE_ID[role] if isinstance(role, str) else int(role)
+    check(_call("cev_es_perturb_diag_f32", _h(dev), _ptr(theta), _ptr(sigma), int(in_dim), int(bool(mirrored)),
+                int(seed), role_id, int(gen), int(row0), int(n_rows), pitch, _ptr(out), _ptr(noise_out),
+                _stream(dev)), "cev_es_perturb_diag_f32")
+    return out
+
+
+def es_update_diag(fitness, in_dim, n_total, seed, role, gen, row0, *, mirrored=False, g_mu=None, g_sigma=None):
+    """K6 of separable NES, noise regenerated: (g_mu, g_sigma) fp32[pitch] = 1/n_total * sum_i F_i z_i and
+    1/n_total * sum_i F_i (z_i^2 - 1) over the local members [row0, row0 + len(fitness)), z the stream of
+    :func:`es_perturb_diag` with the same ``mirrored``."""
+    dev = _need_cuda(fitness, g_mu, g_sigma)
+    if fitness.dtype != torch.float64 or fitness.dim() != 1:
+        raise _lib.CevError("es_update_diag: fitness must be float64 [n_rows]")
+    pitch = layout.fc_pitch(in_dim)
+    g_mu = torch.empty(pitch, dtype=torch.float32, device=dev) if g_mu is None else g_mu
+    g_sigma = torch.empty(pitch, dtype=torch.float32, device=dev) if g_sigma is None else g_sigma
+    _need_f32("es_update_diag: g_mu", g_mu, pitch)
+    _need_f32("es_update_diag: g_sigma", g_sigma, pitch)
+    role_id = layout.ROLE_ID[role] if isinstance(role, str) else int(role)
+    n = fitness.shape[0]
+    check(_call("cev_es_update_diag_f32", _h(dev), ctypes.c_void_p(0) if n == 0 else _ptr(fitness), int(in_dim),
+                int(bool(mirrored)), int(n_total), int(seed), role_id, int(gen), int(row0), n, _ptr(g_mu),
+                _ptr(g_sigma), _stream(dev)), "cev_es_update_diag_f32")
+    return g_mu, g_sigma
+
+
+def es_apply_diag(theta, sigma, g_mu, g_sigma, in_dims, *, lr, sigma_lr, sigma_min, sigma_max):
+    """Separable NES apply over the FCNetwork rows of ``in_dims`` concatenated in ``theta`` / ``sigma`` / ``g_mu`` /
+    ``g_sigma``: theta += lr * (sigma * g_mu), then sigma *= exp(sigma_lr[s] / 2 * g_sigma) clamped to
+    [sigma_min, sigma_max] (``sigma_lr``: one learning rate per row).  Only the Linear entries change."""
+    dev = _need_cuda(theta, sigma, g_mu, g_sigma)
+    n = sum(layout.fc_pitch(d) for d in in_dims)
+    for name, x in (("theta", theta), ("sigma", sigma), ("g_mu", g_mu), ("g_sigma", g_sigma)):
+        _need_f32(f"es_apply_diag: {name}", x, n)
+    if len(sigma_lr) != len(in_dims):
+        raise _lib.CevError("es_apply_diag: one sigma_lr per row")
+    dims = (ctypes.c_int * len(in_dims))(*[int(d) for d in in_dims])
+    etas = (ctypes.c_double * len(in_dims))(*[float(e) for e in sigma_lr])
+    check(_call("cev_es_apply_diag_f32", _h(dev), _ptr(theta), _ptr(sigma), _ptr(g_mu), _ptr(g_sigma), len(in_dims),
+                dims, float(lr), etas, float(sigma_min), float(sigma_max), _stream(dev)), "cev_es_apply_diag_f32")
+    return theta, sigma
 
 
 def axpy(a, x, y):

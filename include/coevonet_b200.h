@@ -349,6 +349,48 @@ int cev_es_apply_f32(cev_handle* h, float* theta, const float* delta, float* m, 
                      const int* in_dims, int optimizer, double lr, float l2_coeff, int t, cev_stream stream);
 
 /*
+ * Separable natural evolution strategies (SNES; Schaul, Glasmachers & Schmidhuber 2011; Wierstra et al.,
+ * JMLR 2014): the search distribution of a role is N(mu, diag(sigma^2)), mu = theta, sigma an fp32 row laid
+ * out like theta (cev_fc_pitch(in_dim) floats; sigma0 on the Linear entries, 0 on LayerNorm entries and
+ * padding).
+ *
+ * K5: member = theta + fl(sigma[j] * z_j) on the Linear entries (LayerNorm entries copied, padding 0).  z comes
+ * from the streams of cev_es_perturb_f32 (mirrored = 0: Philox(ES), member = c) or of
+ * cev_es_perturb_mirrored_f32 (mirrored = 1: Philox(ES_MIRROR), member = pair c >> 1, the odd member of a pair
+ * takes -z), with their shard and pair-cut rules: with sigma equal to sigma0 on every Linear entry the rows
+ * are theirs bit for bit.  noise_out (optional) receives s*z.
+ */
+int cev_es_perturb_diag_f32(cev_handle* h, const float* theta, const float* sigma, int in_dim, int mirrored,
+                            uint64_t seed, int role, uint32_t gen, int64_t row0, int64_t n_rows, int64_t pitch,
+                            float* out, float* noise_out, cev_stream stream);
+
+/*
+ * K6 of SNES, noise regenerated, over members [row0, row0 + n_rows) of n_total:
+ *   g_mu[j]    = fl32(1/n_total) * sum_i F_i z_ij
+ *   g_sigma[j] = fl32(1/n_total) * sum_i F_i (z_ij^2 - 1)      (z^2 - 1 = fl(fl(z z) - 1))
+ * fp32 fmaf in row order within the splits of cev_es_update_f32 (mirrored = 0) or cev_es_update_mirrored_f32
+ * (mirrored = 1: splits start on even global rows), the splits summed in order.  g_mu and g_sigma are
+ * fp32[cev_fc_pitch(in_dim)], zeros on LayerNorm entries and padding; partial sums over a rank's members are
+ * all-reduced by the caller.  Workspace: 2 * n_split * pitch floats.
+ */
+int cev_es_update_diag_f32(cev_handle* h, const double* fitness, int in_dim, int mirrored, int64_t n_total,
+                           uint64_t seed, int role, uint32_t gen, int64_t row0, int64_t n_rows, float* g_mu,
+                           float* g_sigma, cev_stream stream);
+
+/*
+ * SNES apply over n_segments (<= 3) FCNetwork rows concatenated like cev_es_apply_f32 (in_dims and
+ * sigma_lr: HOST arrays, sigma_lr[s] = eta_sigma of segment s, fp64, > 0).  On the Linear entries only,
+ * one IEEE-rounded fp32 operation at a time, the mu step with the OLD sigma:
+ *   theta[j] += fl(lr * fl(sigma[j] * g_mu[j]))
+ *   sigma[j]  = clamp(fl(sigma[j] * fl32(exp(0.5 * sigma_lr[s] * g_sigma[j]))), sigma_min, sigma_max)
+ * (the exp and its argument in fp64; the clamp is fminf(fmaxf(x, sigma_min), sigma_max)).  LayerNorm entries
+ * and padding of theta and sigma keep their bits.
+ */
+int cev_es_apply_diag_f32(cev_handle* h, float* theta, float* sigma, const float* g_mu, const float* g_sigma,
+                          int n_segments, const int* in_dims, float lr, const double* sigma_lr, float sigma_min,
+                          float sigma_max, cev_stream stream);
+
+/*
  * K7 -- fitness-sharing distances.  Replaces the distance loop of
  * diversity_penalty (utils/game_logic_functions.py:12-37):
  * d[i] = || pop[i] - ref ||_2 over the perturbable (Linear) parameters.
