@@ -902,6 +902,21 @@ __global__ void __launch_bounds__(PT) philox_words_kernel(uint32_t k0, uint32_t 
     out[i] = make_uint4(v.x, v.y, v.z, v.w);
 }
 
+// Co-ES Hall of Fame: slot of opponent set k (0 = the newest snapshot, k >= 1 uniform over the filled slots)
+__global__ void __launch_bounds__(PT) es_hof_opponents_kernel(uint32_t k0, uint32_t k1, uint32_t gen, int K,
+                                                              uint64_t filled, int64_t newest,
+                                                              int64_t* __restrict__ out) {
+    const int k = blockIdx.x * PT + threadIdx.x;
+    if (k >= K) return;
+    if (k == 0) {
+        out[0] = newest;
+        return;
+    }
+    const U4 v = philox4x32_10(U4{(uint32_t)((k - 1) >> 2), 0u, gen, noise_tag(CEV_KIND_HOF, 0)}, k0, k1);
+    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+    out[k] = (int64_t)(((uint64_t)w[(k - 1) & 3] * filled) >> 32);
+}
+
 // ---------------------------------------------------------------------------
 // FP32 FMA-pipe peak (roofline denominator for K1, SURVEY.md section 8d)
 // ---------------------------------------------------------------------------
@@ -1333,6 +1348,21 @@ int cev_philox_words(cev_handle* h, uint64_t seed, int kind, int role, uint32_t 
     philox_words_kernel<<<(unsigned)((n + PT - 1) / PT), PT, 0, (cudaStream_t)stream>>>(
         k0, k1, noise_tag(kind, role), gen, member0, n_members, n4, reinterpret_cast<uint4*>(out));
     return check_cuda(cudaGetLastError(), "philox_words_kernel");
+}
+
+int cev_es_hof_opponents_i64(cev_handle* h, uint64_t seed, uint32_t gen, int K, int64_t filled, int64_t newest,
+                             int64_t* out, cev_stream stream) {
+    CEV_REQUIRE(h && out, "es_hof_opponents: null pointer");
+    CEV_REQUIRE(K >= 1, "es_hof_opponents: need K >= 1, got %d", K);
+    CEV_REQUIRE(filled >= 1 && filled <= 0x100000000ll, "es_hof_opponents: need 1 <= filled <= 2^32, got %lld",
+                (long long)filled);
+    CEV_REQUIRE(newest >= 0 && newest < filled, "es_hof_opponents: need 0 <= newest < filled");
+    CEV_GUARD(h);
+    uint32_t k0, k1;
+    split_seed(seed, k0, k1);
+    es_hof_opponents_kernel<<<(unsigned)((K + PT - 1) / PT), PT, 0, (cudaStream_t)stream>>>(
+        k0, k1, gen, K, (uint64_t)filled, newest, out);
+    return check_cuda(cudaGetLastError(), "es_hof_opponents_kernel");
 }
 
 int cev_weight_stats_f32(cev_handle* h, const float* rows, int64_t n_rows, int64_t pitch, int in_dim, float* out,

@@ -185,6 +185,28 @@ def es_distribution(args, algorithm=None):
     return opts
 
 
+#: the Co-ES Hall of Fame and its defaults: 0 = off (every member plays the other roles' current base agents only)
+ES_HOF_DEFAULTS = {"es_hof_size": 0, "es_hof_opponents": 1}
+
+
+def es_hof(args, algorithm=None):
+    """The Co-ES Hall-of-Fame settings of ``args`` (an absent attribute is its default), validated: ``ValueError``
+    for a negative archive size H, for K opponent sets outside [1, H] when H > 0, for K other than 1 when H = 0 and
+    for any non-default setting with the GA (which keeps its own Hall of Fame, ``--hof_size``)."""
+    opts = {k: int(getattr(args, k, d)) for k, d in ES_HOF_DEFAULTS.items()}
+    H, K = opts["es_hof_size"], opts["es_hof_opponents"]
+    if opts != ES_HOF_DEFAULTS and (algorithm or getattr(args, "algorithm", "ES")) == "GA":
+        raise ValueError("es_hof_size, es_hof_opponents: Co-ES options, not available with --algorithm GA "
+                         "(the GA keeps its own Hall of Fame, --hof_size)")
+    if H < 0:
+        raise ValueError(f"es_hof_size must be >= 0, not {H}")
+    if H == 0 and K != 1:
+        raise ValueError(f"es_hof_opponents {K} needs an archive: es_hof_size must be >= {max(K, 1)}")
+    if H > 0 and not 1 <= K <= H:
+        raise ValueError(f"es_hof_opponents must be in [1, es_hof_size = {H}], not {K}")
+    return opts
+
+
 def default_sigma_learning_rate(d):
     """SNES's sigma learning rate for d parameters, (3 + ln d) / (5 sqrt d) (Schaul et al. 2011), in fp64."""
     return (3.0 + np.log(float(d))) / (5.0 * np.sqrt(float(d)))
@@ -482,6 +504,7 @@ class GAEngine(_EngineBase):
         self.P = int(args.population)
         es_options(args, "GA")                           # refuses the Co-ES options
         es_distribution(args, "GA")
+        es_hof(args, "GA")
         self.shard = Shard(self.P, self.comm.rank, self.comm.world)
         self.pop = {r: pop_rows[r].to(self.device).contiguous() for r in ROLES}       # [n_local, pitch]
         self.hof = {r: hof_rows[r].to(self.device).contiguous() for r in ROLES}       # [hof, pitch]
@@ -674,9 +697,16 @@ class ESEngine(_EngineBase):
 
     Opt-in search distribution (``es_distribution``): separable NES keeps a per-parameter sigma
     (``sigma_cat``, laid out like ``theta_cat`` and replicated like it) that the population's rewards adapt
-    through the natural gradient of log sigma; K5 / K6 / the apply become their diag forms."""
+    through the natural gradient of log sigma; K5 / K6 / the apply become their diag forms.
+
+    Opt-in Hall of Fame (``es_hof``): an archive ring ``hof_ring`` fp32 [H, len(theta_cat)] of ``theta_cat``
+    snapshots (the founders, then one after every apply), replicated like theta.  Every member then plays K
+    opponent sets of E games each: set 0 is the current base agents, sets 1..K-1 are snapshots drawn on the device
+    (``cev_es_hof_opponents_i64``, keyed by (seed, generation)), and its reward is the mean over the K x E games."""
 
     kind = "ES"
+    #: Philox stream of the initial states of ``hof_matrix``
+    _hof_matrix_tag = 0x50000000
 
     def __init__(self, args, device, theta_rows, env=None, kernels=None, comm=None):
         super().__init__(args, device, env, kernels, comm)
@@ -698,6 +728,25 @@ class ESEngine(_EngineBase):
             self.theta[r].copy_(theta_rows[r].reshape(-1)[:pitch])
             off += pitch
         self.comm.broadcast0(self.theta_cat)              # rank 0's base agents everywhere (ADVICE r1)
+        #: (offset, pitch) of each role's row in theta_cat (every offset is a multiple of 32 floats)
+        self.cols = {r: (o, p) for r, o, p in zip(ROLES, np.cumsum([0] + pitches[:-1]).tolist(), pitches)}
+        self.hof_opts = es_hof(args, "ES")
+        self.hof_size = self.hof_opts["es_hof_size"]
+        #: opponent sets per member: K with the Hall of Fame, else the current base agents only
+        self.K = self.hof_opts["es_hof_opponents"] if self.hof_size else 1
+        self.hof_ring = self.hof_opp = self.hof_ids = None
+        if self.hof_size:
+            n = self.theta_cat.numel()
+            self.hof_ring = torch.zeros((self.hof_size, n), dtype=torch.float32, device=self.device)
+            self.hof_ring[0].copy_(self.theta_cat)
+            #: ring bookkeeping on the host (no sync needed): next slot to write, filled slots [0, filled), and
+            #: the generation whose base agents each slot holds (-1: empty)
+            self.hof_head, self.hof_filled = 1 % self.hof_size, 1
+            self.hof_slot_gen = [0] + [-1] * (self.hof_size - 1)
+            #: this generation's K snapshots, gathered once: the roles' opponents are column views of it
+            self.hof_opp = torch.empty((self.K, n), dtype=torch.float32, device=self.device)
+            self.hof_ids = torch.empty(self.K, dtype=torch.int64, device=self.device)
+            self._hof_eval_slot_gen = None
         self.distribution = es_distribution(args, "ES")
         self.separable = self.distribution["es_distribution"] == "separable"
         self.sigma_cat = self.grad_cat = None
@@ -736,33 +785,56 @@ class ESEngine(_EngineBase):
         self.diversity = {r: None for r in ROLES}
         self.weight_stats = {r: None for r in ROLES}      # fp32 [n_local, 4] when args.log_member_weight_stats
         self.member_stats = bool(getattr(args, "log_member_weight_stats", False))
-        self.variant = self.rollout_variant(self.P, 1)
+        self.variant = self.rollout_variant(self.P, self.K)
 
     def _base_opponents(self, role):
-        t = self.theta
+        """Rows of the two other seats (ascending seat order): the base rows [1, pitch], or with the Hall of Fame the
+        roles' columns of this generation's K gathered snapshots [K, pitch] (row pitch len(theta_cat))."""
+        if self.hof_size:
+            t = {r: self.hof_opp[:, o:o + p] for r, (o, p) in self.cols.items()}
+        else:
+            t = {r: self.theta[r].reshape(1, -1) for r in ROLES}
         if role == "agent_0":
-            return t["adversary_0"].reshape(1, -1), t["agent_1"].reshape(1, -1)
+            return t["adversary_0"], t["agent_1"]
         if role == "agent_1":
-            return t["adversary_0"].reshape(1, -1), t["agent_0"].reshape(1, -1)
-        return t["agent_0"].reshape(1, -1), t["agent_1"].reshape(1, -1)
+            return t["adversary_0"], t["agent_0"]
+        return t["agent_0"], t["agent_1"]
 
     def _reference_initial_states(self):
         """The reference interleaves the three roles per member
-        (evolutionary_strategy.py:236-251): game 3*i + role_index."""
-        E = self.E
-        block = self.env.draw_initial_states(self.P * 3 * E).reshape(self.P, 3, E, mpe_spec.INIT_STATE_DIM)
+        (evolutionary_strategy.py:236-251): game 3*i + role_index; with K opponent sets the
+        records of a member and role are laid out [K, E]."""
+        K, E = self.K, self.E
+        block = self.env.draw_initial_states(self.P * 3 * K * E).reshape(self.P, 3, K, E, mpe_spec.INIT_STATE_DIM)
         sl = slice(self.shard.row0, self.shard.row0 + self.shard.n_local)
-        return {r: torch.from_numpy(np.ascontiguousarray(block[sl, i][:, None])).to(self.device)
+        return {r: torch.from_numpy(np.ascontiguousarray(block[sl, i])).to(self.device)
                 for i, r in enumerate(ROLES)}
+
+    def _gather_hof_opponents(self):
+        """The K opponent snapshots of this generation: slots drawn on the device, rows gathered from the ring."""
+        newest = (self.hof_head - 1) % self.hof_size
+        self.k.es_hof_opponents(self.seed, self.gen, self.K, self.hof_filled, newest, self.device, out=self.hof_ids)
+        self.k.gather_rows(self.hof_ring, self.hof_ids, out=self.hof_opp)
+        self._hof_eval_slot_gen = list(self.hof_slot_gen)
+
+    def _hof_append(self):
+        """Archive the base agents just applied (a stream-ordered device copy; the bookkeeping stays on the host)."""
+        self.hof_ring[self.hof_head].copy_(self.theta_cat)
+        self.hof_slot_gen[self.hof_head] = self.gen + 1
+        self.hof_head = (self.hof_head + 1) % self.hof_size
+        self.hof_filled = min(self.hof_filled + 1, self.hof_size)
 
     def evaluate(self, init_by_role=None):
         """Perturb + one rollout per member and role against the other roles'
-        BASE policies (mutate_weights, evolutionary_strategy.py:63-116).
-        ``init_by_role`` (optional) supplies the initial states [n_local,1,E,11] per role."""
+        BASE policies (mutate_weights, evolutionary_strategy.py:63-116), or with the
+        Hall of Fame against K opponent sets.
+        ``init_by_role`` (optional) supplies the initial states [n_local,K,E,11] per role."""
         limit = self.args.max_timesteps_per_episode
         ref_init = init_by_role
         if ref_init is None and self.init_mode == "reference":
             ref_init = self._reference_initial_states()
+        if self.hof_size:
+            self._gather_hof_opponents()
 
         specs = {}
 
@@ -782,15 +854,15 @@ class ESEngine(_EngineBase):
             if ref_init is not None:
                 init = ref_init[role]
             else:
-                init = self._initial_states(self.P, 1, self.shard, ROLES.index(role) + 4 * self.gen)
+                init = self._initial_states(self.P, self.K, self.shard, ROLES.index(role) + 4 * self.gen)
             opp_a, opp_b = self._base_opponents(role)
             specs[role] = (role, self.members[role], opp_a, opp_b, init)
 
         self._run_roles(prepare)
         outs = self._rollouts([specs[r] for r in ROLES], limit)
         for role in ROLES:
-            slot = self._role_slot(outs[role], role, limit)           # [n_local, 1, E]
-            self.rewards[role] = slot.mean(dim=(1, 2)).contiguous()
+            slot = self._role_slot(outs[role], role, limit)           # [n_local, K, E]
+            self.rewards[role] = slot.mean(dim=(1, 2)).contiguous()   # the mean over all K x E games
 
     def update(self):
         """compute_weight_update + apply (evolutionary_strategy.py:120-148,255-265) for the three
@@ -864,6 +936,8 @@ class ESEngine(_EngineBase):
                             l2_coeff=self.options["l2_coeff"], t=self.gen + 1, m=self.adam_m, v=self.adam_v)
         else:
             self.k.axpy(1.0, self.delta_cat, self.theta_cat)
+        if self.hof_size:
+            self._hof_append()
 
     def step(self, init_by_role=None, sync=True):
         """One generation.  ``sync=True`` returns the evaluation triple (one host read);
@@ -887,9 +961,45 @@ class ESEngine(_EngineBase):
                 shaped_fitness={r: (self.comm.all_gather_rows(self.shaped_fitness[r], self.shard).cpu().numpy().copy()
                                     if self.shaping else None) for r in ROLES},
                 sigma={r: float(hs["sigma_history"][r][self.gen]) for r in ROLES},
-                sigma_stats={r: self._sigma_stats(r) for r in ROLES}))
+                sigma_stats={r: self._sigma_stats(r) for r in ROLES},
+                hof_ids=self._hof_ids_record()))
         self.gen += 1
         return self.last_eval() if sync else None
+
+    def _hof_ids_record(self):
+        """(archive slots, their generations) of this generation's K opponent sets; None without the Hall of Fame."""
+        if not self.hof_size:
+            return None
+        slots = self.hof_ids.cpu().numpy().copy()
+        return slots, np.array([self._hof_eval_slot_gen[s] for s in slots], dtype=np.int64)
+
+    def hof_generations(self):
+        """Generations of the filled archive entries, oldest first: the order of :meth:`hof_matrix`."""
+        return sorted(self.hof_slot_gen[:self.hof_filled])
+
+    def hof_matrix(self, E=None):
+        """Cross-generation matrix of the archive (current individual vs ancestral opponents): fp64
+        [filled, filled, 2], entries oldest first (:meth:`hof_generations`).  ``[i, j]`` holds the mean true
+        good-team and adversary rewards (rollout columns 0 and 2, the reference's attribution not applied) when the
+        good team of entry i plays the adversary of entry j, over E games (default ``envs_per_member``) up to
+        ``max_evaluation_steps``.  One structured rollout: the adversaries are the members, the good teams the K
+        opponent sets; the initial states come from a Philox stream of their own, so the training run is not
+        disturbed.  Replicated: every rank can compute it."""
+        if not self.hof_size:
+            raise ValueError("hof_matrix needs the Hall of Fame (es_hof_size > 0)")
+        E = self.E if E is None else int(E)
+        n = self.hof_filled
+        order = sorted(range(n), key=lambda s: self.hof_slot_gen[s])
+        idx = torch.tensor(order, dtype=torch.int64).to(self.device)
+        rows = self.k.gather_rows(self.hof_ring, idx)                        # [n, len(theta_cat)], oldest first
+        col = {r: rows[:, o:o + p] for r, (o, p) in self.cols.items()}
+        init = self.k.init_states(self.seed, self._hof_matrix_tag, n * n * E, self.device)
+        out = self.k.mpe_rollout("adversary_0", col["adversary_0"].contiguous(), col["agent_0"], col["agent_1"],
+                                 init.reshape(n, n, E, mpe_spec.INIT_STATE_DIM),
+                                 n_cycles=_limit_cycles(self.k, self.args.max_evaluation_steps),
+                                 pos_first=self.pos_first, status=self.status)      # [n adversaries, n teams, E, 4]
+        self.k.raise_on_status(self.status)
+        return out[..., [0, 2]].mean(dim=2).transpose(0, 1).contiguous().to(torch.float64)
 
     def _sigma_stats(self, role):
         """(mean, min, max, std) of the role's per-parameter sigma after this generation's update over its Linear
@@ -901,19 +1011,23 @@ class ESEngine(_EngineBase):
 
     def state_dict(self):
         """Base rows, the update options and search distribution settings, for Adam its moments (its step count is
-        the generation count) and for separable NES the per-parameter sigmas."""
+        the generation count), for separable NES the per-parameter sigmas and for the Hall of Fame its settings, the
+        archive ring and its bookkeeping."""
         sd = self._base_state()
         sd.update(theta={r: self.theta[r].cpu().clone() for r in ROLES}, es_options=dict(self.options),
-                  es_distribution=dict(self.distribution))
+                  es_distribution=dict(self.distribution), es_hof=dict(self.hof_opts))
         if self.adam_m is not None:
             sd.update(adam_m=self.adam_m.cpu().clone(), adam_v=self.adam_v.cpu().clone())
         if self.separable:
             sd.update(sigma=self.sigma_cat.cpu().clone())
+        if self.hof_size:
+            sd.update(hof_ring=self.hof_ring.cpu().clone(), hof_head=self.hof_head, hof_filled=self.hof_filled,
+                      hof_slot_gen=list(self.hof_slot_gen))
         return sd
 
     def load_state_dict(self, sd):
-        """Refuses a checkpoint written with other update options or search distribution settings (one without
-        them was written with the defaults)."""
+        """Refuses a checkpoint written with other update options, search distribution or Hall-of-Fame settings
+        (one without them was written with the defaults)."""
         saved = sd.get("es_options", ES_OPTION_DEFAULTS)
         if saved != self.options:
             raise ValueError(f"checkpoint was written with ES options {saved}, this run uses {self.options}")
@@ -921,11 +1035,18 @@ class ESEngine(_EngineBase):
         if saved != self.distribution:
             raise ValueError(f"checkpoint was written with the ES distribution {saved}, this run uses "
                              f"{self.distribution}")
+        saved = sd.get("es_hof", ES_HOF_DEFAULTS)
+        if saved != self.hof_opts:
+            raise ValueError(f"checkpoint was written with the ES Hall of Fame {saved}, this run uses {self.hof_opts}")
         self._load_base_state(sd)
         for r in ROLES:
             self.theta[r].copy_(sd["theta"][r])
         if self.separable:
             self.sigma_cat.copy_(sd["sigma"])
+        if self.hof_size:
+            self.hof_ring.copy_(sd["hof_ring"])
+            self.hof_head, self.hof_filled = int(sd["hof_head"]), int(sd["hof_filled"])
+            self.hof_slot_gen = [int(g) for g in sd["hof_slot_gen"]]
         if self.adam_m is not None:
             self.adam_m.copy_(sd["adam_m"])
             self.adam_v.copy_(sd["adam_v"])

@@ -89,6 +89,15 @@ def parse_arguments(argv=None):
     p.add_argument("--sigma_learning_rate", type=float, default=None,
                    help="ES, separable: learning rate of log sigma for all roles (default: (3 + ln d) / (5 sqrt d) "
                         "per role, d = its number of Linear parameters)")
+    p.add_argument("--es_hof_size", type=int, default=0,
+                   help="ES: keep a Hall of Fame of the last H base agents (the founders, then one snapshot per "
+                        "generation) and evaluate every member against --es_hof_opponents sets drawn from it; "
+                        "0 = off (every member plays the current base agents only, the reference)")
+    p.add_argument("--es_hof_opponents", type=int, default=1,
+                   help="ES, with --es_hof_size H: opponent sets K per member, 1 <= K <= H.  Set 0 is the current "
+                        "base agents, sets 1..K-1 are snapshots drawn uniformly with replacement (the same on every "
+                        "rank); each set plays --envs_per_member games, and the reward is the mean over the K x E "
+                        "games")
     p.add_argument("--play_discarded_hof_games", action="store_true",
                    help="GA, reference_compat: also simulate the hof_size-1 games per member whose reward the "
                         "reference overwrites (they never reach the fitness; skipped by default)")
@@ -172,9 +181,12 @@ class Args:
         self.l2_coeff = a.l2_coeff
         self.es_distribution = a.es_distribution
         self.sigma_learning_rate = a.sigma_learning_rate
-        from .engine import es_distribution, es_options
+        self.es_hof_size = a.es_hof_size
+        self.es_hof_opponents = a.es_hof_opponents
+        from .engine import es_distribution, es_hof, es_options
         es_options(self)                  # ValueError: odd population with mirrored sampling, an ES option with GA
         es_distribution(self)
+        es_hof(self)
 
     def print_attributes(self, args=None):
         for k, v in vars(self).items():

@@ -66,6 +66,16 @@ def _need_cuda(*tensors):
     return dev
 
 
+def _need_rows(dev, *rows):
+    """Weight rows handed to the kernels with their ``stride(0)`` as the row pitch: CUDA [n, pitch] tensors on
+    ``dev`` whose rows are contiguous (column views of a wider buffer qualify)."""
+    for t in rows:
+        if not t.is_cuda or t.device != dev:
+            raise _lib.CevError("weight rows must be CUDA tensors on the device of the other operands")
+        if t.dim() != 2 or t.stride(1) != 1:
+            raise _lib.CevError("weight rows must be a [n, pitch] tensor with contiguous rows")
+
+
 def cycles_for_limit(agent_step_limit):
     """World steps executed under ``play_MPE``'s agent-step limit
     (``utils/game_logic_functions.py:127,195-210``; truncation after 25 cycles)."""
@@ -125,10 +135,12 @@ def mpe_rollout(member_role, members, opp_a, opp_b, init, *, n_cycles=MAX_CYCLES
     """K1 structured rollout.
 
     members fp32[P, pitch]; opp_a / opp_b fp32[K, pitch] for the two other seats
-    in ascending seat order (adversary_0 < agent_0 < agent_1); init fp64
-    [P, K, E, 11] (or [K, E, 11] with ``init_shared``).  Returns fp64 [P, K, E, 4].
+    in ascending seat order (adversary_0 < agent_0 < agent_1), rows contiguous, the row
+    pitch taken from ``stride(0)``; init fp64 [P, K, E, 11] (or [K, E, 11] with
+    ``init_shared``).  Returns fp64 [P, K, E, 4].
     """
-    dev = _need_cuda(members, opp_a, opp_b, init, out, status)
+    dev = _need_cuda(members, init, out, status)
+    _need_rows(dev, opp_a, opp_b)
     seat = layout.SEAT_OF[member_role] if isinstance(member_role, str) else int(member_role)
     P, K = members.shape[0], opp_a.shape[0]
     if opp_b.shape[0] != K:
@@ -161,13 +173,14 @@ def mpe_rollout_roles(roles, *, n_cycles=MAX_CYCLES, pos_first=True, init_shared
     """K1 for the roles of one generation in one pass (``cev_mpe_rollout_roles_f32``).
 
     ``roles``: list of (member_role, members fp32[P, pitch], opp_a fp32[K, pitch], opp_b, init fp64[P, K, E, 11])
-    with the same P, K, E for every role.  Returns the list of fp64 [P, K, E, 4] results, identical to one
-    :func:`mpe_rollout` per role."""
+    with the same P, K, E for every role (opponent rows as in :func:`mpe_rollout`).  Returns the list of fp64
+    [P, K, E, 4] results, identical to one :func:`mpe_rollout` per role."""
     outs, recs, keep = [], (_lib.RolloutRole * len(roles))(), []
     P = K = E = None
     dev = None
     for i, (member_role, members, opp_a, opp_b, init) in enumerate(roles):
-        dev = _need_cuda(members, opp_a, opp_b, init, status)
+        dev = _need_cuda(members, init, status)
+        _need_rows(dev, opp_a, opp_b)
         seat = layout.SEAT_OF[member_role] if isinstance(member_role, str) else int(member_role)
         p_, k_ = members.shape[0], opp_a.shape[0]
         e_ = init.shape[1] if init_shared else init.shape[2]
@@ -543,6 +556,20 @@ def es_apply_diag(theta, sigma, g_mu, g_sigma, in_dims, *, lr, sigma_lr, sigma_m
     check(_call("cev_es_apply_diag_f32", _h(dev), _ptr(theta), _ptr(sigma), _ptr(g_mu), _ptr(g_sigma), len(in_dims),
                 dims, float(lr), etas, float(sigma_min), float(sigma_max), _stream(dev)), "cev_es_apply_diag_f32")
     return theta, sigma
+
+
+def es_hof_opponents(seed, gen, K, filled, newest, device, *, out=None):
+    """Co-ES Hall of Fame: int64[K] archive slots of generation ``gen``'s opponent sets on the device.  Set 0 is
+    ``newest`` (the current base agents); sets 1..K-1 are drawn uniformly with replacement from the ``filled``
+    slots [0, filled) by the Philox stream of kind ``KIND_HOF`` keyed by (seed, gen), the same on every rank."""
+    if out is None:
+        out = torch.empty(int(K), dtype=torch.int64, device=device)
+    dev = _need_cuda(out)
+    if out.dtype != torch.int64 or tuple(out.shape) != (int(K),):
+        raise _lib.CevError(f"es_hof_opponents: out must be int64 [{K}]")
+    check(_call("cev_es_hof_opponents_i64", _h(dev), int(seed), int(gen), int(K), int(filled), int(newest), _ptr(out),
+                _stream(dev)), "cev_es_hof_opponents_i64")
+    return out
 
 
 def axpy(a, x, y):

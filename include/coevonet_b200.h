@@ -55,6 +55,7 @@ typedef void* cev_stream;               /* cudaStream_t */
 #define CEV_KIND_INIT 4
 #define CEV_KIND_XOVER 5
 #define CEV_KIND_ES_MIRROR 6            /* ES pair noise under mirrored sampling: member = pair id */
+#define CEV_KIND_HOF 7                  /* Co-ES Hall-of-Fame opponent draws: member 0, role 0 */
 
 int cev_version(void);
 const char* cev_last_error(void);
@@ -389,6 +390,19 @@ int cev_es_update_diag_f32(cev_handle* h, const double* fitness, int in_dim, int
 int cev_es_apply_diag_f32(cev_handle* h, float* theta, float* sigma, const float* g_mu, const float* g_sigma,
                           int n_segments, const int* in_dims, float lr, const double* sigma_lr, float sigma_min,
                           float sigma_max, cev_stream stream);
+
+/*
+ * Co-ES Hall of Fame: the archive slots of the K opponent sets of generation `gen` (out: DEVICE int64[K]).
+ * The archive is a ring whose slots [0, filled) hold snapshots (1 <= filled <= 2^32); `newest` is the slot of
+ * the current base agents.  Set 0 is always `newest`; set k >= 1 is drawn uniformly with replacement from the
+ * filled slots:
+ *   w_k    = word (k - 1) & 3 of Philox(seed; ctr = ((k - 1) >> 2, 0, gen, CEV_KIND_HOF << 8))
+ *   out[k] = (uint64(w_k) * filled) >> 32
+ * (multiply-shift: slot s is drawn with probability floor or ceil of 2^32 / filled over 2^32, so the bias
+ * is at most filled / 2^32).  The key is (seed, gen) alone, so every rank draws the same slots.
+ */
+int cev_es_hof_opponents_i64(cev_handle* h, uint64_t seed, uint32_t gen, int K, int64_t filled, int64_t newest,
+                             int64_t* out, cev_stream stream);
 
 /*
  * K7 -- fitness-sharing distances.  Replaces the distance loop of
