@@ -19,6 +19,8 @@ CEV_OK = 0
 STATUS_NONFINITE = 1
 SEAT = {"adversary_0": 0, "agent_0": 1, "agent_1": 2}
 KIND_ES, KIND_GA, KIND_ENV, KIND_FRAMES, KIND_INIT, KIND_XOVER, KIND_ES_MIRROR, KIND_HOF = 0, 1, 2, 3, 4, 5, 6, 7
+KIND_ES_SUBSPACE = 8
+SUBSPACE_MAX_DIM = 32
 ES_SGD, ES_ADAM = 0, 1
 INIT_STATE_DIM = 11
 ROLLOUT_OUT_DIM = 4
@@ -106,6 +108,11 @@ _SIGNATURES = {
     "cev_es_apply_diag_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, POINTER(c_int),
                                       c_float, POINTER(c_double), c_float, c_float, c_void_p]),
     "cev_es_hof_opponents_i64": (c_int, [c_void_p, c_uint64, c_uint32, c_int, c_int64, c_int64, c_void_p, c_void_p]),
+    "cev_es_perturb_subspace_f32": (c_int, [c_void_p, c_void_p, c_int, c_float, c_void_p, c_void_p, c_int64, c_int,
+                                            c_void_p, c_double, c_int, c_uint64, c_int, c_uint32, c_int64, c_int64,
+                                            c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "cev_es_subspace_basis_f32": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, POINTER(c_int), c_void_p,
+                                          c_void_p, c_void_p]),
     "cev_diversity_dist_f32": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_int,
                                        c_void_p, c_void_p]),
     "cev_deepqn_forward": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_void_p, c_int, c_int,

@@ -207,6 +207,41 @@ def es_hof(args, algorithm=None):
     return opts
 
 
+#: Co-ES guided search in the subspace of the last k update estimates and its defaults: 0 = off (the isotropic
+#: search); es_subspace_alpha None = the default share 0.5 of the variance outside the subspace when k > 0
+ES_SUBSPACE_DEFAULTS = {"es_subspace_dim": 0, "es_subspace_alpha": None}
+SUBSPACE_DEFAULT_ALPHA = 0.5
+
+
+def es_subspace(args, algorithm=None):
+    """The Co-ES guided-search settings of ``args`` (an absent attribute is its default), validated: ``ValueError``
+    for any non-default setting with the GA, for a subspace dimension k outside [0, 32], for an alpha outside (0, 1]
+    or given while k = 0, and for k > 0 together with ``separable`` search or ``--regenerate_noise`` (the regenerated
+    update would need the subspace term too).  With k > 0 an alpha left unset becomes 0.5."""
+    opts = {k: getattr(args, k, d) for k, d in ES_SUBSPACE_DEFAULTS.items()}
+    if opts != ES_SUBSPACE_DEFAULTS and (algorithm or getattr(args, "algorithm", "ES")) == "GA":
+        changed = sorted(k for k in opts if opts[k] != ES_SUBSPACE_DEFAULTS[k])
+        raise ValueError(f"{', '.join(changed)}: Co-ES options, not available with --algorithm GA")
+    k = int(opts["es_subspace_dim"])
+    if not 0 <= k <= _lib.SUBSPACE_MAX_DIM:
+        raise ValueError(f"es_subspace_dim must be in [0, {_lib.SUBSPACE_MAX_DIM}], not {k}")
+    alpha = opts["es_subspace_alpha"]
+    if alpha is not None:
+        alpha = float(alpha)
+        if k == 0:
+            raise ValueError("es_subspace_alpha needs es_subspace_dim > 0")
+        if not 0.0 < alpha <= 1.0:
+            raise ValueError(f"es_subspace_alpha must be in (0, 1], not {alpha}")
+    if k:
+        if getattr(args, "es_distribution", "isotropic") != "isotropic":
+            raise ValueError("es_subspace_dim: guided search is not available with es_distribution 'separable'")
+        if not getattr(args, "update_from_members", True):
+            raise ValueError("es_subspace_dim: guided search needs the update from the members, not available with "
+                             "--regenerate_noise")
+        alpha = SUBSPACE_DEFAULT_ALPHA if alpha is None else alpha
+    return {"es_subspace_dim": k, "es_subspace_alpha": alpha}
+
+
 def default_sigma_learning_rate(d):
     """SNES's sigma learning rate for d parameters, (3 + ln d) / (5 sqrt d) (Schaul et al. 2011), in fp64."""
     return (3.0 + np.log(float(d))) / (5.0 * np.sqrt(float(d)))
@@ -505,6 +540,7 @@ class GAEngine(_EngineBase):
         es_options(args, "GA")                           # refuses the Co-ES options
         es_distribution(args, "GA")
         es_hof(args, "GA")
+        es_subspace(args, "GA")
         self.shard = Shard(self.P, self.comm.rank, self.comm.world)
         self.pop = {r: pop_rows[r].to(self.device).contiguous() for r in ROLES}       # [n_local, pitch]
         self.hof = {r: hof_rows[r].to(self.device).contiguous() for r in ROLES}       # [hof, pitch]
@@ -702,7 +738,13 @@ class ESEngine(_EngineBase):
     Opt-in Hall of Fame (``es_hof``): an archive ring ``hof_ring`` fp32 [H, len(theta_cat)] of ``theta_cat``
     snapshots (the founders, then one after every apply), replicated like theta.  Every member then plays K
     opponent sets of E games each: set 0 is the current base agents, sets 1..K-1 are snapshots drawn on the device
-    (``cev_es_hof_opponents_i64``, keyed by (seed, generation)), and its reward is the mean over the K x E games."""
+    (``cev_es_hof_opponents_i64``, keyed by (seed, generation)), and its reward is the mean over the K x E games.
+
+    Opt-in guided search (``es_subspace``): a ring ``subspace_ring`` fp32 [k, len(theta_cat)] of the last k all-reduced
+    update estimates (``delta_cat``), replicated like theta, and its orthonormal basis ``subspace_U`` (k_eff <= k rows
+    per role, ``cev_es_subspace_basis_f32``, recomputed after every apply).  Members are theta + sigma (A z + B U^T c):
+    a share alpha of the variance stays isotropic, the rest lies in the subspace, with the total variance of the
+    isotropic search.  The update is the default members-form K6, which reads sigma eps back as member - theta."""
 
     kind = "ES"
     #: Philox stream of the initial states of ``hof_matrix``
@@ -749,6 +791,19 @@ class ESEngine(_EngineBase):
             self._hof_eval_slot_gen = None
         self.distribution = es_distribution(args, "ES")
         self.separable = self.distribution["es_distribution"] == "separable"
+        self.subspace_opts = es_subspace(args, "ES")
+        #: guided-search subspace dimension k (0: off) and the share alpha of the variance outside it
+        self.subspace_k = self.subspace_opts["es_subspace_dim"]
+        self.subspace_alpha = self.subspace_opts["es_subspace_alpha"]
+        self.subspace_ring = self.subspace_U = self.subspace_keff = None
+        if self.subspace_k:
+            n = self.theta_cat.numel()
+            self.subspace_ring = torch.zeros((self.subspace_k, n), dtype=torch.float32, device=self.device)
+            self.subspace_U = torch.zeros((self.subspace_k, n), dtype=torch.float32, device=self.device)
+            #: k_eff per role on the device (K5 reads it there): 0 until the first estimate
+            self.subspace_keff = torch.zeros(len(ROLES), dtype=torch.int32, device=self.device)
+            #: ring bookkeeping on the host (no sync needed): next slot to write, filled slots [0, filled)
+            self.subspace_head, self.subspace_filled = 0, 0
         self.sigma_cat = self.grad_cat = None
         self.sigma_rows, self.sigma_grad, self.sigma_lr = {}, {}, {}
         if self.separable:
@@ -844,6 +899,13 @@ class ESEngine(_EngineBase):
                 self.k.es_perturb_diag(self.theta[role], self.sigma_rows[role], in_dim, self.seed, role, self.gen,
                                        self.shard.row0, self.shard.n_local, mirrored=self.mirrored,
                                        out=self.members[role])
+            elif self.subspace_k:
+                o, p = self.cols[role]
+                i = ROLES.index(role)
+                self.k.es_perturb_subspace(self.theta[role], in_dim, self.sigma_dev(role), self.subspace_U[:, o:o + p],
+                                           self.subspace_keff[i:i + 1], self.subspace_alpha, self.seed, role, self.gen,
+                                           self.shard.row0, self.shard.n_local, mirrored=self.mirrored,
+                                           out=self.members[role])
             else:
                 perturb = self.k.es_perturb_mirrored if self.mirrored else self.k.es_perturb
                 perturb(self.theta[role], in_dim, self.sigma_dev(role), self.seed, role, self.gen,
@@ -938,6 +1000,21 @@ class ESEngine(_EngineBase):
             self.k.axpy(1.0, self.delta_cat, self.theta_cat)
         if self.hof_size:
             self._hof_append()
+        if self.subspace_k:
+            self._subspace_append()
+
+    def _subspace_append(self):
+        """Append this generation's all-reduced estimate to the ring (a stream-ordered device copy; the bookkeeping
+        stays on the host) and recompute the basis on the device."""
+        self.subspace_ring[self.subspace_head].copy_(self.delta_cat)
+        self.subspace_head = (self.subspace_head + 1) % self.subspace_k
+        self.subspace_filled = min(self.subspace_filled + 1, self.subspace_k)
+        self._subspace_basis()
+
+    def _subspace_basis(self):
+        newest = (self.subspace_head - 1) % self.subspace_k
+        self.k.es_subspace_basis(self.subspace_ring, newest, self.subspace_filled, [layout.OBS_DIM[r] for r in ROLES],
+                                 out=self.subspace_U, k_eff=self.subspace_keff)
 
     def step(self, init_by_role=None, sync=True):
         """One generation.  ``sync=True`` returns the evaluation triple (one host read);
@@ -962,7 +1039,9 @@ class ESEngine(_EngineBase):
                                     if self.shaping else None) for r in ROLES},
                 sigma={r: float(hs["sigma_history"][r][self.gen]) for r in ROLES},
                 sigma_stats={r: self._sigma_stats(r) for r in ROLES},
-                hof_ids=self._hof_ids_record()))
+                hof_ids=self._hof_ids_record(),
+                subspace_rank=({r: int(x) for r, x in zip(ROLES, self.subspace_keff.cpu().tolist())}
+                               if self.subspace_k else None)))
         self.gen += 1
         return self.last_eval() if sync else None
 
@@ -1011,11 +1090,16 @@ class ESEngine(_EngineBase):
 
     def state_dict(self):
         """Base rows, the update options and search distribution settings, for Adam its moments (its step count is
-        the generation count), for separable NES the per-parameter sigmas and for the Hall of Fame its settings, the
-        archive ring and its bookkeeping."""
+        the generation count), for separable NES the per-parameter sigmas, for the Hall of Fame its settings, the
+        archive ring and its bookkeeping, and for guided search its settings, the estimate ring and its bookkeeping
+        (the basis is recomputed from them on load)."""
         sd = self._base_state()
         sd.update(theta={r: self.theta[r].cpu().clone() for r in ROLES}, es_options=dict(self.options),
-                  es_distribution=dict(self.distribution), es_hof=dict(self.hof_opts))
+                  es_distribution=dict(self.distribution), es_hof=dict(self.hof_opts),
+                  es_subspace=dict(self.subspace_opts))
+        if self.subspace_k:
+            sd.update(subspace_ring=self.subspace_ring.cpu().clone(), subspace_head=self.subspace_head,
+                      subspace_filled=self.subspace_filled)
         if self.adam_m is not None:
             sd.update(adam_m=self.adam_m.cpu().clone(), adam_v=self.adam_v.cpu().clone())
         if self.separable:
@@ -1026,8 +1110,8 @@ class ESEngine(_EngineBase):
         return sd
 
     def load_state_dict(self, sd):
-        """Refuses a checkpoint written with other update options, search distribution or Hall-of-Fame settings
-        (one without them was written with the defaults)."""
+        """Refuses a checkpoint written with other update options, search distribution, Hall-of-Fame or guided-search
+        settings (one without them was written with the defaults)."""
         saved = sd.get("es_options", ES_OPTION_DEFAULTS)
         if saved != self.options:
             raise ValueError(f"checkpoint was written with ES options {saved}, this run uses {self.options}")
@@ -1038,6 +1122,10 @@ class ESEngine(_EngineBase):
         saved = sd.get("es_hof", ES_HOF_DEFAULTS)
         if saved != self.hof_opts:
             raise ValueError(f"checkpoint was written with the ES Hall of Fame {saved}, this run uses {self.hof_opts}")
+        saved = sd.get("es_subspace", ES_SUBSPACE_DEFAULTS)
+        if saved != self.subspace_opts:
+            raise ValueError(f"checkpoint was written with the ES guided search {saved}, this run uses "
+                             f"{self.subspace_opts}")
         self._load_base_state(sd)
         for r in ROLES:
             self.theta[r].copy_(sd["theta"][r])
@@ -1047,6 +1135,14 @@ class ESEngine(_EngineBase):
             self.hof_ring.copy_(sd["hof_ring"])
             self.hof_head, self.hof_filled = int(sd["hof_head"]), int(sd["hof_filled"])
             self.hof_slot_gen = [int(g) for g in sd["hof_slot_gen"]]
+        if self.subspace_k:
+            self.subspace_ring.copy_(sd["subspace_ring"])
+            self.subspace_head, self.subspace_filled = int(sd["subspace_head"]), int(sd["subspace_filled"])
+            if self.subspace_filled:
+                self._subspace_basis()
+            else:
+                self.subspace_U.zero_()
+                self.subspace_keff.zero_()
         if self.adam_m is not None:
             self.adam_m.copy_(sd["adam_m"])
             self.adam_v.copy_(sd["adam_v"])

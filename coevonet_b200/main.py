@@ -98,6 +98,17 @@ def parse_arguments(argv=None):
                         "base agents, sets 1..K-1 are snapshots drawn uniformly with replacement (the same on every "
                         "rank); each set plays --envs_per_member games, and the reward is the mean over the K x E "
                         "games")
+    p.add_argument("--es_subspace_dim", type=int, default=0,
+                   help="ES: guided search (Maheswaranathan et al. 2019): put part of the search variance in the "
+                        "subspace spanned by the last k update estimates (an orthonormal basis recomputed every "
+                        "generation on the device), 0 <= k <= 32; the total variance stays that of the isotropic "
+                        "search, so --initial_mutation_power_*, --adaptive and the clamps keep their meaning.  0 = off "
+                        "(the isotropic search of the reference).  Not with --es_distribution separable or "
+                        "--regenerate_noise")
+    p.add_argument("--es_subspace_alpha", type=float, default=None,
+                   help="ES, with --es_subspace_dim k: share alpha in (0, 1] of the variance kept isotropic; members "
+                        "are theta + sigma (sqrt(alpha) z + sqrt((1 - alpha) d / k_eff) U^T c), d the role's number of "
+                        "Linear parameters, k_eff <= k the rank of the basis (default 0.5; 1 = the isotropic search)")
     p.add_argument("--play_discarded_hof_games", action="store_true",
                    help="GA, reference_compat: also simulate the hof_size-1 games per member whose reward the "
                         "reference overwrites (they never reach the fitness; skipped by default)")
@@ -183,10 +194,13 @@ class Args:
         self.sigma_learning_rate = a.sigma_learning_rate
         self.es_hof_size = a.es_hof_size
         self.es_hof_opponents = a.es_hof_opponents
-        from .engine import es_distribution, es_hof, es_options
+        self.es_subspace_dim = a.es_subspace_dim
+        self.es_subspace_alpha = a.es_subspace_alpha
+        from .engine import es_distribution, es_hof, es_options, es_subspace
         es_options(self)                  # ValueError: odd population with mirrored sampling, an ES option with GA
         es_distribution(self)
         es_hof(self)
+        es_subspace(self)
 
     def print_attributes(self, args=None):
         for k, v in vars(self).items():

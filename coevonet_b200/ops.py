@@ -17,7 +17,7 @@ MAX_CYCLES = 25
 
 #: kernels launched per C-ABI call (bench.py reports the total as ``gpu_launches``)
 _KERNELS_PER_CALL = {"cev_es_update_f32": 2, "cev_es_update_members_f32": 2, "cev_es_update_mirrored_f32": 2,
-                     "cev_es_update_diag_f32": 2, "cev_fp32_peak": 4}
+                     "cev_es_update_diag_f32": 2, "cev_es_subspace_basis_f32": 6, "cev_fp32_peak": 4}
 launch_count = 0
 
 
@@ -570,6 +570,58 @@ def es_hof_opponents(seed, gen, K, filled, newest, device, *, out=None):
     check(_call("cev_es_hof_opponents_i64", _h(dev), int(seed), int(gen), int(K), int(filled), int(newest), _ptr(out),
                 _stream(dev)), "cev_es_hof_opponents_i64")
     return out
+
+
+def es_perturb_subspace(theta, in_dim, sigma, U, k_eff, alpha, seed, role, gen, row0, n_rows, *, mirrored=False,
+                        out=None, noise_out=None, coef_out=None):
+    """K5 of guided search: member rows theta + sigma * eps with eps = A z + B U^T c on the Linear entries,
+    A = fp32(sqrt(alpha)), B = fp32(sqrt((1 - alpha) d / k_eff)) (see ``cev_es_perturb_subspace_f32``).  ``U``: fp32
+    [k, pitch] rows of the basis (contiguous rows, any row stride, e.g. the role's columns of a wider buffer);
+    ``k_eff``: one-element int32 DEVICE tensor, the number of basis rows in use.  z is the stream of
+    :func:`es_perturb` (``mirrored`` False) or :func:`es_perturb_mirrored` (True); ``noise_out`` receives s*z and
+    ``coef_out`` fp32 [n_rows, k] the coefficients s*c, s = -1 for the odd member of a mirrored pair."""
+    dev = _need_cuda(theta, k_eff, out, noise_out, coef_out)
+    _need_rows(dev, U)
+    pitch = layout.fc_pitch(in_dim)
+    k = U.shape[0]
+    _need_f32("es_perturb_subspace: theta", theta, pitch)
+    if U.dtype != torch.float32 or U.shape[1] != pitch:
+        raise _lib.CevError(f"es_perturb_subspace: U must be float32 [k, {pitch}]")
+    if k_eff.dtype != torch.int32 or k_eff.numel() != 1:
+        raise _lib.CevError("es_perturb_subspace: k_eff must be a one-element int32 tensor")
+    for name, t, cols in (("out", out, pitch), ("noise_out", noise_out, pitch), ("coef_out", coef_out, k)):
+        if t is not None and (t.dtype != torch.float32 or tuple(t.shape) != (int(n_rows), cols)):
+            raise _lib.CevError(f"es_perturb_subspace: {name} must be float32 [{n_rows}, {cols}]")
+    if out is None:
+        out = torch.empty((n_rows, pitch), dtype=torch.float32, device=dev)
+    role_id = layout.ROLE_ID[role] if isinstance(role, str) else int(role)
+    sig, sig_dev = _sigma_args(sigma)
+    check(_call("cev_es_perturb_subspace_f32", _h(dev), _ptr(theta), int(in_dim), sig, sig_dev, _ptr(U), U.stride(0),
+                int(k), _ptr(k_eff), float(alpha), int(bool(mirrored)), int(seed), role_id, int(gen), int(row0),
+                int(n_rows), pitch, _ptr(out), _ptr(noise_out), _ptr(coef_out), _stream(dev)),
+          "cev_es_perturb_subspace_f32")
+    return out
+
+
+def es_subspace_basis(ring, newest, filled, in_dims, *, out=None, k_eff=None):
+    """Orthonormal basis of the guided-search subspace of each FCNetwork row of ``in_dims`` concatenated in ``ring``
+    (fp32 [k, n]; slots [0, filled) filled, ``newest`` the newest estimate): CholeskyQR2 in fp64 over the estimates
+    newest first, dropping an estimate whose residual norm is <= 1e-4 of its own norm.  Returns (U fp32 [k, n],
+    k_eff int32 [len(in_dims)]) on the device (see ``cev_es_subspace_basis_f32``)."""
+    dev = _need_cuda(ring, out, k_eff)
+    k, n = ring.shape
+    if ring.dtype != torch.float32 or n != sum(layout.fc_pitch(d) for d in in_dims):
+        raise _lib.CevError("es_subspace_basis: ring must be float32 [k, summed pitch of in_dims]")
+    out = torch.empty_like(ring) if out is None else out
+    k_eff = torch.empty(len(in_dims), dtype=torch.int32, device=dev) if k_eff is None else k_eff
+    if out.dtype != torch.float32 or out.shape != ring.shape:
+        raise _lib.CevError(f"es_subspace_basis: out must be float32 [{k}, {n}]")
+    if k_eff.dtype != torch.int32 or k_eff.numel() != len(in_dims):
+        raise _lib.CevError(f"es_subspace_basis: k_eff must be int32 [{len(in_dims)}]")
+    dims = (ctypes.c_int * len(in_dims))(*[int(d) for d in in_dims])
+    check(_call("cev_es_subspace_basis_f32", _h(dev), _ptr(ring), int(k), int(newest), int(filled), len(in_dims),
+                dims, _ptr(out), _ptr(k_eff), _stream(dev)), "cev_es_subspace_basis_f32")
+    return out, k_eff
 
 
 def axpy(a, x, y):

@@ -56,6 +56,7 @@ typedef void* cev_stream;               /* cudaStream_t */
 #define CEV_KIND_XOVER 5
 #define CEV_KIND_ES_MIRROR 6            /* ES pair noise under mirrored sampling: member = pair id */
 #define CEV_KIND_HOF 7                  /* Co-ES Hall-of-Fame opponent draws: member 0, role 0 */
+#define CEV_KIND_ES_SUBSPACE 8          /* Co-ES guided-search coefficients: member = member id, or pair id */
 
 int cev_version(void);
 const char* cev_last_error(void);
@@ -403,6 +404,50 @@ int cev_es_apply_diag_f32(cev_handle* h, float* theta, float* sigma, const float
  */
 int cev_es_hof_opponents_i64(cev_handle* h, uint64_t seed, uint32_t gen, int K, int64_t filled, int64_t newest,
                              int64_t* out, cev_stream stream);
+
+/*
+ * Co-ES guided search in the subspace of the last k update estimates (Guided ES, Maheswaranathan et al. 2019;
+ * the subspace built from the ES's own past updates as in ASEBO, Choromanski et al. 2019).  U is an orthonormal
+ * basis fp32 [k][ldu] of k_eff <= k directions laid out like theta (zero on LayerNorm entries and padding).
+ *
+ * K5: on the Linear entries, with d = the number of Linear entries of the row (cev_fc_dim(in_dim) minus the
+ * LayerNorm entries), A = fp32(sqrt(alpha)) and B = fp32(sqrt((1 - alpha) * d / k_eff)) (fp64, then rounded):
+ *   s_j   = sum_{m < k_eff} fl(U[m][j] * c_m)      (fp32, one rounding per operation, m = 0, 1, ... in order,
+ *                                                   starting from +0)
+ *   eps_j = fl(fl(A * z_j) + fl(B * s_j)),   member = theta + fl(sigma * eps_j)
+ * and the odd member of a mirrored pair is theta + (-fl(sigma * eps_j)).  LayerNorm entries are copied, padding is 0.
+ * z is the stream of cev_es_perturb_f32 (mirrored = 0) or cev_es_perturb_mirrored_f32 (mirrored = 1), with their
+ * shard and pair-cut rules.  c holds k normals per unit u (the member id, or the pair id c >> 1 when mirrored):
+ *   c_{4 m4 + t} = normal t of the Box-Muller pairs of Philox(seed; ctr = (m4, u, gen, role | CEV_KIND_ES_SUBSPACE << 8)),
+ * the transform of the K5 stream, so c does not depend on k_eff (member i uses the first k_eff of its normals).
+ * E||eps||^2 = d, the total variance of the isotropic search.  k_eff is read from the DEVICE int k_eff[0]
+ * (clamped to [0, k]); when k_eff = 0 or alpha = 1 (B = 0) eps = z and the rows are those of the isotropic K5 bit
+ * for bit.  noise_out (optional, [n_rows][pitch]) receives s*z and coef_out (optional, [n_rows][k]) s*c, s = -1 for
+ * the odd member of a mirrored pair and +1 otherwise.  1 <= k <= CEV_SUBSPACE_MAX_DIM, 0 < alpha <= 1,
+ * ldu >= pitch a multiple of 4.
+ */
+#define CEV_SUBSPACE_MAX_DIM 32
+int cev_es_perturb_subspace_f32(cev_handle* h, const float* theta, int in_dim, float sigma, const double* sigma_dev,
+                                const float* U, int64_t ldu, int k, const int* k_eff, double alpha, int mirrored,
+                                uint64_t seed, int role, uint32_t gen, int64_t row0, int64_t n_rows, int64_t pitch,
+                                float* out, float* noise_out, float* coef_out, cev_stream stream);
+
+/*
+ * The orthonormal basis of the guided-search subspace, for n_segments (<= 3) FCNetwork rows concatenated like
+ * cev_es_apply_f32 (in_dims: HOST array; n = the summed pitches).  ring: DEVICE fp32 [k][n], slots [0, filled)
+ * filled, slot `newest` the newest estimate.  Per segment, over its Linear entries, with the columns
+ * D_a = ring[(newest - a) mod k] for a < filled (newest first):
+ *   CholeskyQR2 in fp64: G = D^T D (fp64 products of the fp32 values, summed per column chunk in column order, the
+ *   chunks in order); a right-looking Cholesky of G over a = 0, 1, ... that DROPS column a when its squared
+ *   residual is <= 1e-8 of G[a][a] (its residual norm is <= 1e-4 of its own norm; a zero or non-finite column is
+ *   always dropped); U = fp32(D R^-1) on the kept columns, in their order; then the same once more on U.
+ * U (out): DEVICE fp32 [k][n], rows [0, k_eff) orthonormal, the other rows and every LayerNorm / padding entry 0;
+ * a dropped estimate never enters U, even when it holds an inf or a NaN.
+ * k_eff (out): DEVICE int32 [n_segments].  Deterministic; workspace (n_segments * (ceil(max pitch / 4096) + 1) * k^2
+ * doubles).  ring and U must not overlap.
+ */
+int cev_es_subspace_basis_f32(cev_handle* h, const float* ring, int k, int newest, int filled, int n_segments,
+                              const int* in_dims, float* U, int* k_eff, cev_stream stream);
 
 /*
  * K7 -- fitness-sharing distances.  Replaces the distance loop of
