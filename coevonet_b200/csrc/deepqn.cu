@@ -102,11 +102,12 @@ __device__ __forceinline__ void bn_relu_store(float* __restrict__ out_s, const f
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     for (int c = warp; c < COUT; c += DQ_T / 32) {
         float* row = out_s + c * NPOS;
+        const float x0 = row[0];      // sums of deviations from it: a constant channel normalises to exactly beta
         float s = 0.f;
-        for (int p = lane; p < NPOS; p += 32) s += row[p];
+        for (int p = lane; p < NPOS; p += 32) s += row[p] - x0;
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-        const float mean = s * (1.0f / NPOS);
+        const float mean = x0 + s * (1.0f / NPOS);
         float q = 0.f;
         for (int p = lane; p < NPOS; p += 32) {
             const float d = row[p] - mean;

@@ -194,13 +194,16 @@ deepqn_conv_tc_kernel(const __grid_constant__ CUtensorMap map_w, const ConvParam
                 }
                 asm volatile("bar.sync 1, 256;\n" ::: "memory");
                 // one warp per channel, two-pass statistics; the channels of a warp are independent chains,
-                // unrolled so their shared-memory and shuffle latencies overlap
-                float mean[CPW], rstd[CPW];
+                // unrolled so their shared-memory and shuffle latencies overlap.  The sums are of deviations from
+                // the channel's first value: a constant channel then has exactly zero deviation and variance and
+                // normalises to exactly beta (a rounded mean would leave ulps that rstd = 1/sqrt(eps) scales by 316)
+                float mean[CPW], rstd[CPW], x0[CPW];
 #pragma unroll
                 for (int i = 0; i < CPW; ++i) {
                     const float* row = in_s + (c + 8 * i) * G::LD;
+                    x0[i] = row[0];
                     float s1 = 0.f;
-                    for (int q = lane; q < NPIN; q += 32) s1 += row[q];
+                    for (int q = lane; q < NPIN; q += 32) s1 += row[q] - x0[i];
                     mean[i] = s1;
                 }
 #pragma unroll
@@ -210,7 +213,7 @@ deepqn_conv_tc_kernel(const __grid_constant__ CUtensorMap map_w, const ConvParam
 #pragma unroll
                 for (int i = 0; i < CPW; ++i) {
                     const float* row = in_s + (c + 8 * i) * G::LD;
-                    mean[i] *= (1.0f / NPIN);
+                    mean[i] = x0[i] + mean[i] * (1.0f / NPIN);
                     float qv = 0.f;
                     for (int q = lane; q < NPIN; q += 32) {
                         const float d = row[q] - mean[i];
@@ -368,11 +371,10 @@ __global__ void __launch_bounds__(64) deepqn_bn3_flatten_kernel(const float* __r
         float v[49];
         float s = 0.f;
 #pragma unroll
-        for (int i = 0; i < 49; ++i) {
-            v[i] = src[i * 64];
-            s += v[i];
-        }
-        const float mean = s * (1.0f / 49);
+        for (int i = 0; i < 49; ++i) v[i] = src[i * 64];
+#pragma unroll
+        for (int i = 0; i < 49; ++i) s += v[i] - v[0];          // deviations: exact zero for a constant channel
+        const float mean = v[0] + s * (1.0f / 49);
         float q = 0.f;
 #pragma unroll
         for (int i = 0; i < 49; ++i) {

@@ -351,10 +351,10 @@ int launch_deepqn_fc_tc(cev_handle* h, const float* members, int64_t pitch, int 
     p.ob_off = ob_off;
     p.logits = logits;
     p.actions = actions;
-    static bool configured = false;
-    if (!configured) {
+    static bool configured[16] = {};          // a function attribute is per device
+    if (h->device < 16 && !configured[h->device]) {
         CEV_CUDA(cudaFuncSetAttribute(deepqn_fc_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)F3_SMEM));
-        configured = true;
+        configured[h->device] = true;
     }
     const int grid = P < h->n_sm ? P : h->n_sm;
     deepqn_fc_tc_kernel<<<grid, F3_THREADS, F3_SMEM, stream>>>(map_x, map_w, p);

@@ -653,13 +653,19 @@ def diversity_from_dist(dist):
 
 
 def deepqn_forward(members, frames, c_in, n_actions):
-    """K2: logits fp32[P,B,A] and first-max actions int32[P,B]."""
-    dev = _need_cuda(members, frames)
+    """K2: logits fp32[P,B,A] and first-max actions int32[P,B].  ``members`` fp32[P, >= dqn_dim] with
+    contiguous rows; the row pitch is ``stride(0)`` (rows of a wider buffer qualify)."""
+    dev = _need_cuda(frames)
+    _need_rows(dev, members)
     P, B = frames.shape[0], frames.shape[1]
     if frames.dtype != torch.uint8 or tuple(frames.shape[2:]) != (c_in, 84, 84):
         raise _lib.CevError("deepqn_forward: frames must be uint8 [P,B,C,84,84]")
+    if members.dtype != torch.float32 or members.shape[0] != P or members.shape[1] < layout.dqn_dim(c_in, n_actions):
+        raise _lib.CevError("deepqn_forward: members must be fp32 [P, >= dqn_dim(c_in, n_actions)]")
     logits = torch.empty((P, B, n_actions), dtype=torch.float32, device=dev)
     actions = torch.empty((P, B), dtype=torch.int32, device=dev)
+    if P == 0:
+        return logits, actions
     check(_call("cev_deepqn_forward", _h(dev), _ptr(members), P, members.stride(0),
                                     _ptr(frames), B, int(c_in), int(n_actions), _ptr(logits),
                                     _ptr(actions), _stream(dev)), "cev_deepqn_forward")
