@@ -21,6 +21,9 @@ SEAT = {"adversary_0": 0, "agent_0": 1, "agent_1": 2}
 KIND_ES, KIND_GA, KIND_ENV, KIND_FRAMES, KIND_INIT, KIND_XOVER, KIND_ES_MIRROR, KIND_HOF = 0, 1, 2, 3, 4, 5, 6, 7
 KIND_ES_SUBSPACE = 8
 SUBSPACE_MAX_DIM = 32
+#: Co-ES novelty search (CEV_NOVELTY_* in include/coevonet_b200.h): probe observations per behaviour
+#: characterisation, its length (probes x actions), and the limits of k and of the archive
+NOVELTY_PROBES, NOVELTY_BC_DIM, NOVELTY_MAX_K, NOVELTY_MAX_ARCHIVE = 32, 160, 32, 32768
 ES_SGD, ES_ADAM = 0, 1
 INIT_STATE_DIM = 11
 ROLLOUT_OUT_DIM = 4
@@ -113,6 +116,10 @@ _SIGNATURES = {
                                             c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "cev_es_subspace_basis_f32": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, POINTER(c_int), c_void_p,
                                           c_void_p, c_void_p]),
+    "cev_novelty_probe_obs_f32": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
+    "cev_novelty_bc_f32": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
+                                   c_void_p]),
+    "cev_novelty_knn_f64": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "cev_diversity_dist_f32": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_int,
                                        c_void_p, c_void_p]),
     "cev_deepqn_forward": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_void_p, c_int, c_int,

@@ -242,6 +242,45 @@ def es_subspace(args, algorithm=None):
     return {"es_subspace_dim": k, "es_subspace_alpha": alpha}
 
 
+#: Co-ES novelty search (NS-ES / NSR-ES, Conti et al. 2018) and its defaults: weight 0 = off (the fitness is the
+#: reward); es_novelty_k / es_novelty_archive None = NOVELTY_DEFAULT_K / NOVELTY_DEFAULT_ARCHIVE when the weight is > 0
+ES_NOVELTY_DEFAULTS = {"es_novelty_weight": 0.0, "es_novelty_k": None, "es_novelty_archive": None}
+NOVELTY_DEFAULT_K, NOVELTY_DEFAULT_ARCHIVE = 10, 1024
+#: Philox stream of the novelty search's probe world states (cev_init_states_f64): apart from the training states
+#: (role + 4 * gen), the evaluation games (0x40000000 + gen) and the Hall-of-Fame matrix (0x50000000)
+NOVELTY_PROBE_TAG = 0x60000000
+
+
+def es_novelty(args, algorithm=None):
+    """The Co-ES novelty-search settings of ``args`` (an absent attribute is its default), validated: ``ValueError``
+    for any non-default setting with the GA, for a weight w outside [0, 1], for k or the archive size given while
+    w = 0, for k outside [1, 32], for an archive size outside [1, 32768] and for w > 0 without centered-rank fitness
+    shaping (the reward and the novelty are combined as ranks).  With w > 0 an unset k becomes 10 and an unset
+    archive size 1024."""
+    opts = {k: getattr(args, k, d) for k, d in ES_NOVELTY_DEFAULTS.items()}
+    if opts != ES_NOVELTY_DEFAULTS and (algorithm or getattr(args, "algorithm", "ES")) == "GA":
+        changed = sorted(k for k in opts if opts[k] != ES_NOVELTY_DEFAULTS[k])
+        raise ValueError(f"{', '.join(changed)}: Co-ES options, not available with --algorithm GA")
+    w = float(opts["es_novelty_weight"])
+    if not 0.0 <= w <= 1.0:
+        raise ValueError(f"es_novelty_weight must be in [0, 1], not {w}")
+    if w == 0.0:
+        given = [k for k in ("es_novelty_k", "es_novelty_archive") if opts[k] is not None]
+        if given:
+            raise ValueError(f"{', '.join(given)} needs es_novelty_weight > 0")
+        return dict(ES_NOVELTY_DEFAULTS)
+    k = NOVELTY_DEFAULT_K if opts["es_novelty_k"] is None else int(opts["es_novelty_k"])
+    if not 1 <= k <= _lib.NOVELTY_MAX_K:
+        raise ValueError(f"es_novelty_k must be in [1, {_lib.NOVELTY_MAX_K}], not {k}")
+    A = NOVELTY_DEFAULT_ARCHIVE if opts["es_novelty_archive"] is None else int(opts["es_novelty_archive"])
+    if not 1 <= A <= _lib.NOVELTY_MAX_ARCHIVE:
+        raise ValueError(f"es_novelty_archive must be in [1, {_lib.NOVELTY_MAX_ARCHIVE}], not {A}")
+    if getattr(args, "fitness_shaping", "none") != "centered_rank":
+        raise ValueError("es_novelty_weight combines the ranks of the reward and of the novelty: it needs "
+                         "fitness_shaping 'centered_rank'")
+    return {"es_novelty_weight": w, "es_novelty_k": k, "es_novelty_archive": A}
+
+
 def default_sigma_learning_rate(d):
     """SNES's sigma learning rate for d parameters, (3 + ln d) / (5 sqrt d) (Schaul et al. 2011), in fp64."""
     return (3.0 + np.log(float(d))) / (5.0 * np.sqrt(float(d)))
@@ -541,6 +580,7 @@ class GAEngine(_EngineBase):
         es_distribution(args, "GA")
         es_hof(args, "GA")
         es_subspace(args, "GA")
+        es_novelty(args, "GA")
         self.shard = Shard(self.P, self.comm.rank, self.comm.world)
         self.pop = {r: pop_rows[r].to(self.device).contiguous() for r in ROLES}       # [n_local, pitch]
         self.hof = {r: hof_rows[r].to(self.device).contiguous() for r in ROLES}       # [hof, pitch]
@@ -744,7 +784,13 @@ class ESEngine(_EngineBase):
     update estimates (``delta_cat``), replicated like theta, and its orthonormal basis ``subspace_U`` (k_eff <= k rows
     per role, ``cev_es_subspace_basis_f32``, recomputed after every apply).  Members are theta + sigma (A z + B U^T c):
     a share alpha of the variance stays isotropic, the rest lies in the subspace, with the total variance of the
-    isotropic search.  The update is the default members-form K6, which reads sigma eps back as member - theta."""
+    isotropic search.  The update is the default members-form K6, which reads sigma eps back as member - theta.
+
+    Opt-in novelty search (``es_novelty``, NS-ES / NSR-ES): a member's behaviour characterisation is its softmax action
+    distributions on 32 probe observations (``novelty_probe_obs``, drawn once from the seed), fp32 [160].  Per role a
+    ring ``novelty_ring`` fp32 [A, 160] holds those of past base agents (the founders, then one after every apply),
+    replicated like theta; a member's novelty is the mean distance to its k nearest entries, and the update is
+    weighted by F = (1 - w) cr(reward) + w cr(novelty) (cr: centered ranks of the global vectors)."""
 
     kind = "ES"
     #: Philox stream of the initial states of ``hof_matrix``
@@ -804,6 +850,25 @@ class ESEngine(_EngineBase):
             self.subspace_keff = torch.zeros(len(ROLES), dtype=torch.int32, device=self.device)
             #: ring bookkeeping on the host (no sync needed): next slot to write, filled slots [0, filled)
             self.subspace_head, self.subspace_filled = 0, 0
+        self.novelty_opts = es_novelty(args, "ES")
+        #: novelty weight w (0: off), nearest neighbours k and archive capacity A
+        self.novelty_w = self.novelty_opts["es_novelty_weight"]
+        self.novelty_k = self.novelty_opts["es_novelty_k"]
+        self.novelty_A = self.novelty_opts["es_novelty_archive"]
+        self.novelty_ring = self.novelty_probe_obs = None
+        #: the global novelty of this generation's members (fp64 [P] per role) and this rank's rows of it
+        self.novelty = {r: None for r in ROLES}
+        self._novelty_local = {r: None for r in ROLES}
+        if self.novelty_w:
+            states = self.k.init_states(self.seed, NOVELTY_PROBE_TAG, _lib.NOVELTY_PROBES, self.device)
+            self.novelty_probe_obs = {r: self.k.novelty_probe_obs(states, r) for r in ROLES}
+            self.novelty_ring = torch.zeros((len(ROLES), self.novelty_A, _lib.NOVELTY_BC_DIM), dtype=torch.float32,
+                                            device=self.device)
+            #: ring bookkeeping on the host (no sync needed): next slot to write, filled slots [0, filled), and the
+            #: filled count this generation's novelty was measured against
+            self.novelty_head, self.novelty_filled = 0, 0
+            self._novelty_eval_filled = None
+            self._novelty_append()
         self.sigma_cat = self.grad_cat = None
         self.sigma_rows, self.sigma_grad, self.sigma_lr = {}, {}, {}
         if self.separable:
@@ -925,6 +990,26 @@ class ESEngine(_EngineBase):
         for role in ROLES:
             slot = self._role_slot(outs[role], role, limit)           # [n_local, K, E]
             self.rewards[role] = slot.mean(dim=(1, 2)).contiguous()   # the mean over all K x E games
+        if self.novelty_w:
+            self._member_novelty()
+
+    def _member_novelty(self):
+        """Behaviour characterisations of this rank's members and their k-NN novelty against the role's archive."""
+        for i, role in enumerate(ROLES):
+            bc = self.k.novelty_bc(self.members[role], layout.OBS_DIM[role], self.novelty_probe_obs[role],
+                                   status=self.status)
+            self._novelty_local[role] = self.k.novelty_knn(bc, self.novelty_ring[i], self.novelty_filled, self.novelty_k)
+        self._novelty_eval_filled = self.novelty_filled
+
+    def _novelty_append(self):
+        """Characterise the current base agents straight into slot ``head`` of each role's ring (bookkeeping on the
+        host)."""
+        h = self.novelty_head
+        for i, role in enumerate(ROLES):
+            self.k.novelty_bc(self.theta[role].reshape(1, -1), layout.OBS_DIM[role], self.novelty_probe_obs[role],
+                              out=self.novelty_ring[i, h:h + 1], status=self.status)
+        self.novelty_head = (h + 1) % self.novelty_A
+        self.novelty_filled = min(self.novelty_filled + 1, self.novelty_A)
 
     def update(self):
         """compute_weight_update + apply (evolutionary_strategy.py:120-148,255-265) for the three
@@ -936,7 +1021,10 @@ class ESEngine(_EngineBase):
         if a.fitness_sharing:
             cols += [self.k.diversity_dist(self.members[r], self.theta[r], layout.OBS_DIM[r]).to(torch.float64)
                      for r in ROLES]
-        packed = torch.stack(cols, dim=1).contiguous()                             # [n_local, 3 or 6]
+        nov0 = len(cols)                  # the novelty columns, when on
+        if self.novelty_w:
+            cols += [self._novelty_local[r] for r in ROLES]
+        packed = torch.stack(cols, dim=1).contiguous()                             # [n_local, 3, 6 or 9]
         start = getattr(self.comm, "all_gather_rows_start", None)                  # injected comms may only gather
         if start is not None:
             gathered = start(packed, self.shard)                                   # -> [P, 3 or 6]
@@ -954,6 +1042,8 @@ class ESEngine(_EngineBase):
                     self.fitness[role] = (allp[:, i].to(torch.float32) / (1 + div)).to(torch.float64)
                 else:
                     self.fitness[role] = allp[:, i].contiguous()
+                if self.novelty_w:
+                    self.novelty[role] = allp[:, nov0 + i].contiguous()
 
         need_global = a.fitness_sharing or self.shaping
         if need_global:
@@ -966,6 +1056,11 @@ class ESEngine(_EngineBase):
             if self.shaping:
                 # ranks over the global fitness (after sharing: its division by one positive scalar keeps the order)
                 fit = self.k.centered_ranks(self.fitness[role], self.shard.row0, self.shard.n_local)
+                if self.novelty_w:
+                    # NSR-ES (NS-ES at w = 1): the ranks of the reward and of the novelty, combined in fp64
+                    w = self.novelty_w
+                    fit = (1.0 - w) * fit + w * self.k.centered_ranks(self.novelty[role], self.shard.row0,
+                                                                      self.shard.n_local)
                 self.shaped_fitness[role] = fit
             if self.separable:
                 # always from regenerated noise: z = (member - theta) / sigma would not be exact
@@ -1002,6 +1097,8 @@ class ESEngine(_EngineBase):
             self._hof_append()
         if self.subspace_k:
             self._subspace_append()
+        if self.novelty_w:
+            self._novelty_append()
 
     def _subspace_append(self):
         """Append this generation's all-reduced estimate to the ring (a stream-ordered device copy; the bookkeeping
@@ -1041,7 +1138,9 @@ class ESEngine(_EngineBase):
                 sigma_stats={r: self._sigma_stats(r) for r in ROLES},
                 hof_ids=self._hof_ids_record(),
                 subspace_rank=({r: int(x) for r, x in zip(ROLES, self.subspace_keff.cpu().tolist())}
-                               if self.subspace_k else None)))
+                               if self.subspace_k else None),
+                novelty=({r: self.novelty[r].cpu().numpy().copy() for r in ROLES} if self.novelty_w else None),
+                novelty_filled=self._novelty_eval_filled if self.novelty_w else None))
         self.gen += 1
         return self.last_eval() if sync else None
 
@@ -1091,15 +1190,19 @@ class ESEngine(_EngineBase):
     def state_dict(self):
         """Base rows, the update options and search distribution settings, for Adam its moments (its step count is
         the generation count), for separable NES the per-parameter sigmas, for the Hall of Fame its settings, the
-        archive ring and its bookkeeping, and for guided search its settings, the estimate ring and its bookkeeping
-        (the basis is recomputed from them on load)."""
+        archive ring and its bookkeeping, for guided search its settings, the estimate ring and its bookkeeping
+        (the basis is recomputed from them on load), and for novelty search its settings, the characterisation rings
+        and their bookkeeping (the probe observations are a function of the seed)."""
         sd = self._base_state()
         sd.update(theta={r: self.theta[r].cpu().clone() for r in ROLES}, es_options=dict(self.options),
                   es_distribution=dict(self.distribution), es_hof=dict(self.hof_opts),
-                  es_subspace=dict(self.subspace_opts))
+                  es_subspace=dict(self.subspace_opts), es_novelty=dict(self.novelty_opts))
         if self.subspace_k:
             sd.update(subspace_ring=self.subspace_ring.cpu().clone(), subspace_head=self.subspace_head,
                       subspace_filled=self.subspace_filled)
+        if self.novelty_w:
+            sd.update(novelty_ring=self.novelty_ring.cpu().clone(), novelty_head=self.novelty_head,
+                      novelty_filled=self.novelty_filled)
         if self.adam_m is not None:
             sd.update(adam_m=self.adam_m.cpu().clone(), adam_v=self.adam_v.cpu().clone())
         if self.separable:
@@ -1110,8 +1213,8 @@ class ESEngine(_EngineBase):
         return sd
 
     def load_state_dict(self, sd):
-        """Refuses a checkpoint written with other update options, search distribution, Hall-of-Fame or guided-search
-        settings (one without them was written with the defaults)."""
+        """Refuses a checkpoint written with other update options, search distribution, Hall-of-Fame, guided-search or
+        novelty-search settings (one without them was written with the defaults)."""
         saved = sd.get("es_options", ES_OPTION_DEFAULTS)
         if saved != self.options:
             raise ValueError(f"checkpoint was written with ES options {saved}, this run uses {self.options}")
@@ -1126,9 +1229,16 @@ class ESEngine(_EngineBase):
         if saved != self.subspace_opts:
             raise ValueError(f"checkpoint was written with the ES guided search {saved}, this run uses "
                              f"{self.subspace_opts}")
+        saved = sd.get("es_novelty", ES_NOVELTY_DEFAULTS)
+        if saved != self.novelty_opts:
+            raise ValueError(f"checkpoint was written with the ES novelty search {saved}, this run uses "
+                             f"{self.novelty_opts}")
         self._load_base_state(sd)
         for r in ROLES:
             self.theta[r].copy_(sd["theta"][r])
+        if self.novelty_w:
+            self.novelty_ring.copy_(sd["novelty_ring"])
+            self.novelty_head, self.novelty_filled = int(sd["novelty_head"]), int(sd["novelty_filled"])
         if self.separable:
             self.sigma_cat.copy_(sd["sigma"])
         if self.hof_size:

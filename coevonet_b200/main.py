@@ -109,6 +109,18 @@ def parse_arguments(argv=None):
                    help="ES, with --es_subspace_dim k: share alpha in (0, 1] of the variance kept isotropic; members "
                         "are theta + sigma (sqrt(alpha) z + sqrt((1 - alpha) d / k_eff) U^T c), d the role's number of "
                         "Linear parameters, k_eff <= k the rank of the basis (default 0.5; 1 = the isotropic search)")
+    p.add_argument("--es_novelty_weight", type=float, default=0.0,
+                   help="ES: novelty search (Conti et al. 2018) on a policy behaviour characterisation, the member's "
+                        "action distributions on 32 fixed probe observations: the update is weighted by (1 - w) * "
+                        "rank(reward) + w * rank(novelty), the novelty being the mean distance to the k nearest "
+                        "characterisations of past base agents.  1 = NS-ES, 0.5 = NSR-ES, 0 = off (the reference).  "
+                        "Needs --fitness_shaping centered_rank")
+    p.add_argument("--es_novelty_k", type=int, default=None,
+                   help="ES, with --es_novelty_weight > 0: nearest neighbours k of the novelty, 1 <= k <= 32 "
+                        "(default 10)")
+    p.add_argument("--es_novelty_archive", type=int, default=None,
+                   help="ES, with --es_novelty_weight > 0: archive capacity A per role, 1 <= A <= 32768; the oldest "
+                        "characterisation is overwritten once it is full (default 1024)")
     p.add_argument("--play_discarded_hof_games", action="store_true",
                    help="GA, reference_compat: also simulate the hof_size-1 games per member whose reward the "
                         "reference overwrites (they never reach the fitness; skipped by default)")
@@ -196,11 +208,15 @@ class Args:
         self.es_hof_opponents = a.es_hof_opponents
         self.es_subspace_dim = a.es_subspace_dim
         self.es_subspace_alpha = a.es_subspace_alpha
-        from .engine import es_distribution, es_hof, es_options, es_subspace
+        self.es_novelty_weight = a.es_novelty_weight
+        self.es_novelty_k = a.es_novelty_k
+        self.es_novelty_archive = a.es_novelty_archive
+        from .engine import es_distribution, es_hof, es_novelty, es_options, es_subspace
         es_options(self)                  # ValueError: odd population with mirrored sampling, an ES option with GA
         es_distribution(self)
         es_hof(self)
         es_subspace(self)
+        es_novelty(self)
 
     def print_attributes(self, args=None):
         for k, v in vars(self).items():

@@ -624,6 +624,72 @@ def es_subspace_basis(ring, newest, filled, in_dims, *, out=None, k_eff=None):
     return out, k_eff
 
 
+def novelty_probe_obs(init, role, *, out=None):
+    """Probe observations of the novelty search: fp32 [n, in_dim] = what ``role`` observes in the world state of each
+    initial-state record of ``init`` fp64 [n, 11] (zero velocities), bit for bit the rollout's observation."""
+    dev = _need_cuda(init, out)
+    if init.dtype != torch.float64 or init.dim() != 2 or init.shape[1] != _lib.INIT_STATE_DIM:
+        raise _lib.CevError(f"novelty_probe_obs: init must be float64 [n, {_lib.INIT_STATE_DIM}]")
+    in_dim, n = layout.OBS_DIM[role], init.shape[0]
+    if out is None:
+        out = torch.empty((n, in_dim), dtype=torch.float32, device=dev)
+    if out.dtype != torch.float32 or tuple(out.shape) != (n, in_dim):
+        raise _lib.CevError(f"novelty_probe_obs: out must be float32 [{n}, {in_dim}]")
+    check(_call("cev_novelty_probe_obs_f32", _h(dev), _ptr(init), n, layout.SEAT_OF[role], _ptr(out), _stream(dev)),
+          "cev_novelty_probe_obs_f32")
+    return out
+
+
+def novelty_bc(rows, in_dim, probe_obs, *, out=None, status=None):
+    """Behaviour characterisation of the novelty search: fp32 [P, 160], row m = the softmax action distributions of
+    network row m on the 32 probe observations ``probe_obs`` fp32 [32, in_dim], probe after probe.  ``rows``: fp32
+    [P, >= fc_dim] with contiguous rows (any row stride that is a multiple of 4, e.g. a view of a wider buffer);
+    ``out``: fp32 [P, 160] with contiguous rows (e.g. a slot of the archive ring).  A non-finite logit sets ``status``."""
+    dev = _need_cuda(probe_obs, status)
+    _need_rows(dev, rows)
+    P = rows.shape[0]
+    if rows.dtype != torch.float32 or rows.shape[1] < layout.fc_dim(in_dim) or (P and rows.stride(0) % 4):
+        raise _lib.CevError(f"novelty_bc: rows must be float32 [P, >= {layout.fc_dim(in_dim)}], row stride a "
+                            "multiple of 4")
+    if probe_obs.dtype != torch.float32 or tuple(probe_obs.shape) != (_lib.NOVELTY_PROBES, in_dim):
+        raise _lib.CevError(f"novelty_bc: probe_obs must be float32 [{_lib.NOVELTY_PROBES}, {in_dim}]")
+    if out is None:
+        out = torch.empty((P, _lib.NOVELTY_BC_DIM), dtype=torch.float32, device=dev)
+    _need_rows(dev, out)
+    if out.dtype != torch.float32 or tuple(out.shape) != (P, _lib.NOVELTY_BC_DIM):
+        raise _lib.CevError(f"novelty_bc: out must be float32 [{P}, {_lib.NOVELTY_BC_DIM}]")
+    if P == 0:
+        return out
+    check(_call("cev_novelty_bc_f32", _h(dev), _ptr(rows), rows.stride(0), int(in_dim), P, _ptr(probe_obs), _ptr(out),
+                out.stride(0), _ptr(status), _stream(dev)), "cev_novelty_bc_f32")
+    return out
+
+
+def novelty_knn(bc, ring, filled, k, *, out=None):
+    """k-NN novelty: fp64 [n], entry i = the mean of the min(k, filled) smallest Euclidean distances (fp64) from
+    ``bc[i]`` fp32 [n, 160] to the archive entries ``ring[:filled]`` fp32 [A, 160]."""
+    dev = _need_cuda(bc, ring, out)
+    D = _lib.NOVELTY_BC_DIM
+    if bc.dtype != torch.float32 or bc.dim() != 2 or bc.shape[1] != D:
+        raise _lib.CevError(f"novelty_knn: bc must be float32 [n, {D}]")
+    if ring.dtype != torch.float32 or ring.dim() != 2 or ring.shape[1] != D:
+        raise _lib.CevError(f"novelty_knn: ring must be float32 [A, {D}]")
+    if not 1 <= int(filled) <= ring.shape[0]:
+        raise _lib.CevError(f"novelty_knn: filled must be in [1, {ring.shape[0]}], not {filled}")
+    if not 1 <= int(k) <= _lib.NOVELTY_MAX_K:
+        raise _lib.CevError(f"novelty_knn: k must be in [1, {_lib.NOVELTY_MAX_K}], not {k}")
+    n = bc.shape[0]
+    if out is None:
+        out = torch.empty(n, dtype=torch.float64, device=dev)
+    if out.dtype != torch.float64 or tuple(out.shape) != (n,):
+        raise _lib.CevError(f"novelty_knn: out must be float64 [{n}]")
+    if n == 0:
+        return out
+    check(_call("cev_novelty_knn_f64", _h(dev), _ptr(bc), n, _ptr(ring), int(filled), int(k), _ptr(out), _stream(dev)),
+          "cev_novelty_knn_f64")
+    return out
+
+
 def axpy(a, x, y):
     dev = _need_cuda(x, y)
     check(_call("cev_axpy_f32", _h(dev), float(a), _ptr(x), _ptr(y), min(x.numel(), y.numel()),

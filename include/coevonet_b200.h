@@ -450,6 +450,48 @@ int cev_es_subspace_basis_f32(cev_handle* h, const float* ring, int k, int newes
                               const int* in_dims, float* U, int* k_eff, cev_stream stream);
 
 /*
+ * Co-ES novelty search (NS-ES / NSR-ES, Conti et al. 2018) on a policy-space behaviour characterisation (the
+ * "behavioural embedding" of Parker-Holder et al. 2020): a member is characterised by its action distributions on
+ * CEV_NOVELTY_PROBES fixed probe observations, so the characterisation does not depend on the opponents it played.
+ *
+ * Probe observations: obs fp32 [n][in_dim(seat)] = what seat `seat` (0 adversary_0, 1 agent_0, 2 agent_1) observes
+ * in the world state of init record i (fp64 [n][CEV_INIT_STATE_DIM], zero velocities): the rollout's observation,
+ * fp64 differences rounded to fp32.
+ */
+#define CEV_NOVELTY_PROBES 32
+#define CEV_NOVELTY_BC_DIM 160          /* CEV_NOVELTY_PROBES * 5 actions */
+#define CEV_NOVELTY_MAX_K 32
+#define CEV_NOVELTY_MAX_ARCHIVE 32768
+int cev_novelty_probe_obs_f32(cev_handle* h, const double* init, int64_t n, int seat, float* obs, cev_stream stream);
+
+/*
+ * Behaviour characterisation of P FCNetwork rows (pitch: any multiple of 4 floats >= cev_fc_dim(in_dim); the floats
+ * past the network are never read) on the probe observations probe_obs fp32 [CEV_NOVELTY_PROBES][in_dim]:
+ *   bc[m][5 p + a] = softmax(logits of row m on probe p)[a] = exp(l_a - max l) / sum_b exp(l_b - max l)
+ * fp32 (FFMA forward; the logits within a few ulps of a float32 forward, not bit for bit), row m of bc at
+ * m * bc_pitch (bc_pitch >= CEV_NOVELTY_BC_DIM, so a row can be a slot of an archive ring).  A non-finite logit
+ * sets CEV_STATUS_NONFINITE in *status (optional).  Each row is read from global memory once; deterministic, and a
+ * row's result does not depend on P or on the other rows.
+ */
+int cev_novelty_bc_f32(cev_handle* h, const float* rows, int64_t pitch, int in_dim, int64_t P, const float* probe_obs,
+                       float* bc, int64_t bc_pitch, int32_t* status, cev_stream stream);
+
+/*
+ * k-NN novelty of n characterisations bc fp32 [n][CEV_NOVELTY_BC_DIM] against the archive ring fp32
+ * [>= filled][CEV_NOVELTY_BC_DIM], slots [0, filled) filled (1 <= filled <= CEV_NOVELTY_MAX_ARCHIVE,
+ * 1 <= k <= CEV_NOVELTY_MAX_K):
+ *   dist_e = sqrt(sum_t (x_t - y_et)^2)   fp64, t = 0 .. 159 in order, one rounding per operation (no FMA)
+ *   novelty[i] = (sum of the k_eff smallest dist_e, in ascending order of (dist_e, e)) / k_eff,
+ *                k_eff = min(k, filled), summed from +0 one rounded add at a time
+ * novelty: DEVICE fp64 [n].  Exact given finite inputs (the value does not depend on how ties are broken).  A NaN
+ * distance (a NaN in bc or in the ring) is never among the k smallest; with fewer than k_eff other entries the sum
+ * takes +inf for the missing ones, so such a member's novelty is +inf, where the restatement of the formula gives
+ * NaN.  cev_novelty_bc_f32 has set the status word for a NaN characterisation by then.
+ */
+int cev_novelty_knn_f64(cev_handle* h, const float* bc, int64_t n, const float* ring, int64_t filled, int k,
+                        double* novelty, cev_stream stream);
+
+/*
  * K7 -- fitness-sharing distances.  Replaces the distance loop of
  * diversity_penalty (utils/game_logic_functions.py:12-37):
  * d[i] = || pop[i] - ref ||_2 over the perturbable (Linear) parameters.
