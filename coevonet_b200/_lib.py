@@ -20,6 +20,7 @@ STATUS_NONFINITE = 1
 SEAT = {"adversary_0": 0, "agent_0": 1, "agent_1": 2}
 KIND_ES, KIND_GA, KIND_ENV, KIND_FRAMES, KIND_INIT, KIND_XOVER, KIND_ES_MIRROR, KIND_HOF = 0, 1, 2, 3, 4, 5, 6, 7
 KIND_ES_SUBSPACE = 8
+KIND_GA_NOVELTY = 9
 SUBSPACE_MAX_DIM = 32
 #: Co-ES novelty search (CEV_NOVELTY_* in include/coevonet_b200.h): probe observations per behaviour
 #: characterisation, its length (probes x actions), and the limits of k and of the archive
@@ -120,6 +121,9 @@ _SIGNATURES = {
     "cev_novelty_bc_f32": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
                                    c_void_p]),
     "cev_novelty_knn_f64": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
+    "cev_ga_novelty_knn_f64": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int64, c_int64,
+                                       c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p]),
+    "cev_ga_novelty_draw_i64": (c_int, [c_void_p, c_uint64, c_uint32, c_int, c_int, c_int64, c_void_p, c_void_p]),
     "cev_diversity_dist_f32": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_int,
                                        c_void_p, c_void_p]),
     "cev_deepqn_forward": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_void_p, c_int, c_int,

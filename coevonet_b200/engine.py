@@ -281,6 +281,42 @@ def es_novelty(args, algorithm=None):
     return {"es_novelty_weight": w, "es_novelty_k": k, "es_novelty_archive": A}
 
 
+#: Co-GA novelty search (Lehman & Stanley 2011) and its defaults: weight 0 = off (selection on the fitness); the
+#: others None = GA_NOVELTY_DEFAULT_K / _ARCHIVE / _ADD when the weight is > 0
+GA_NOVELTY_DEFAULTS = {"ga_novelty_weight": 0.0, "ga_novelty_k": None, "ga_novelty_archive": None,
+                       "ga_novelty_archive_add": None}
+GA_NOVELTY_DEFAULT_K, GA_NOVELTY_DEFAULT_ARCHIVE, GA_NOVELTY_DEFAULT_ADD = 10, 1024, 1
+
+
+def ga_novelty(args, algorithm=None):
+    """The Co-GA novelty-search settings of ``args`` (an absent attribute is its default), validated: ``ValueError``
+    for any non-default setting with the ES, for a weight w outside [0, 1] (NaN included), for k, the archive size A
+    or the archive additions m given while w = 0, for k outside [1, 32], for A outside [1, 32768] and for m outside
+    [1, A].  With w > 0 an unset k becomes 10, A 1024 and m 1."""
+    opts = {k: getattr(args, k, d) for k, d in GA_NOVELTY_DEFAULTS.items()}
+    if opts != GA_NOVELTY_DEFAULTS and (algorithm or getattr(args, "algorithm", "ES")) != "GA":
+        changed = sorted(k for k in opts if opts[k] != GA_NOVELTY_DEFAULTS[k])
+        raise ValueError(f"{', '.join(changed)}: Co-GA options, not available with --algorithm ES")
+    w = float(opts["ga_novelty_weight"])
+    if not 0.0 <= w <= 1.0:
+        raise ValueError(f"ga_novelty_weight must be in [0, 1], not {w}")
+    if w == 0.0:
+        given = [k for k in ("ga_novelty_k", "ga_novelty_archive", "ga_novelty_archive_add") if opts[k] is not None]
+        if given:
+            raise ValueError(f"{', '.join(given)} needs ga_novelty_weight > 0")
+        return dict(GA_NOVELTY_DEFAULTS)
+    k = GA_NOVELTY_DEFAULT_K if opts["ga_novelty_k"] is None else int(opts["ga_novelty_k"])
+    if not 1 <= k <= _lib.NOVELTY_MAX_K:
+        raise ValueError(f"ga_novelty_k must be in [1, {_lib.NOVELTY_MAX_K}], not {k}")
+    A = GA_NOVELTY_DEFAULT_ARCHIVE if opts["ga_novelty_archive"] is None else int(opts["ga_novelty_archive"])
+    if not 1 <= A <= _lib.NOVELTY_MAX_ARCHIVE:
+        raise ValueError(f"ga_novelty_archive must be in [1, {_lib.NOVELTY_MAX_ARCHIVE}], not {A}")
+    m = GA_NOVELTY_DEFAULT_ADD if opts["ga_novelty_archive_add"] is None else int(opts["ga_novelty_archive_add"])
+    if not 1 <= m <= A:
+        raise ValueError(f"ga_novelty_archive_add must be in [1, ga_novelty_archive = {A}], not {m}")
+    return {"ga_novelty_weight": w, "ga_novelty_k": k, "ga_novelty_archive": A, "ga_novelty_archive_add": m}
+
+
 def default_sigma_learning_rate(d):
     """SNES's sigma learning rate for d parameters, (3 + ln d) / (5 sqrt d) (Schaul et al. 2011), in fp64."""
     return (3.0 + np.log(float(d))) / (5.0 * np.sqrt(float(d)))
@@ -569,7 +605,15 @@ class _EngineBase:
 class GAEngine(_EngineBase):
     """State: per role the sharded population, the replicated HoF ring
     (oldest first, like the reference's list) and the frozen founder row the
-    reference measures diversity against (Appendix C #3)."""
+    reference measures diversity against (Appendix C #3).
+
+    Opt-in novelty search (``ga_novelty``): a member's behaviour characterisation is the ES novelty search's (its
+    softmax action distributions on 32 probe observations drawn once from the seed), fp32 [160].  Per role a ring
+    ``novelty_ring`` fp32 [A, 160], replicated, starts with the founder's and receives m drawn members'
+    characterisations after every selection.  A member's novelty is the mean distance to its k nearest among the
+    other members and the archive (``cev_ga_novelty_knn_f64``); parents are selected on F = (1 - w) cr(fitness) +
+    w cr(novelty) (cr: centered ranks of the global vectors), while the Hall of Fame and the evaluation games take
+    the fitness-best member."""
 
     kind = "GA"
 
@@ -581,6 +625,12 @@ class GAEngine(_EngineBase):
         es_hof(args, "GA")
         es_subspace(args, "GA")
         es_novelty(args, "GA")
+        self.novelty_opts = ga_novelty(args, "GA")
+        #: novelty weight w (0: off), nearest neighbours k, archive capacity A and additions per generation m
+        self.novelty_w = self.novelty_opts["ga_novelty_weight"]
+        self.novelty_k = self.novelty_opts["ga_novelty_k"]
+        self.novelty_A = self.novelty_opts["ga_novelty_archive"]
+        self.novelty_m = self.novelty_opts["ga_novelty_archive_add"]
         self.shard = Shard(self.P, self.comm.rank, self.comm.world)
         self.pop = {r: pop_rows[r].to(self.device).contiguous() for r in ROLES}       # [n_local, pitch]
         self.hof = {r: hof_rows[r].to(self.device).contiguous() for r in ROLES}       # [hof, pitch]
@@ -591,8 +641,30 @@ class GAEngine(_EngineBase):
             self.comm.broadcast0(self.founder[r])
         self.elites = {r: None for r in ROLES}
         self.elite_ids = {r: None for r in ROLES}
+        #: the row the Hall of Fame and the evaluation games take: elites[0], or with novelty the fitness-best member
+        self.best_rows = {r: None for r in ROLES}
         self.fitness = {r: None for r in ROLES}
         self.diversity = {r: None for r in ROLES}       # 0-dim device tensors
+        self.novelty_ring = self.novelty_probe_obs = None
+        #: the global novelty (fp64 [P]) and selection fitness F of this generation, this rank's rows of the novelty,
+        #: the gathered characterisations [P, 3, 160] and the ids archived after the selection
+        self.novelty = {r: None for r in ROLES}
+        self.shaped_fitness = {r: None for r in ROLES}
+        self._novelty_local = {r: None for r in ROLES}
+        self._novelty_bc_all = None
+        self.novelty_ids = {r: None for r in ROLES}
+        if self.novelty_w:
+            states = self.k.init_states(self.seed, NOVELTY_PROBE_TAG, _lib.NOVELTY_PROBES, self.device)
+            self.novelty_probe_obs = {r: self.k.novelty_probe_obs(states, r) for r in ROLES}
+            self.novelty_ring = torch.zeros((len(ROLES), self.novelty_A, _lib.NOVELTY_BC_DIM), dtype=torch.float32,
+                                            device=self.device)
+            for i, r in enumerate(ROLES):          # slot 0: the founder the reference measures diversity against
+                self.k.novelty_bc(self.founder[r].reshape(1, -1), layout.OBS_DIM[r], self.novelty_probe_obs[r],
+                                  out=self.novelty_ring[i, 0:1], status=self.status)
+            #: ring bookkeeping on the host (no sync needed): next slot to write, filled slots [0, filled), and the
+            #: filled count this generation's novelty was measured against
+            self.novelty_head, self.novelty_filled = 1 % self.novelty_A, 1
+            self._novelty_eval_filled = None
         for r in ROLES:
             assert self.pop[r].shape[0] == self.shard.n_local, "population shard has the wrong row count"
         if int(args.elites_number) > self.P or int(args.elites_number) < 1:
@@ -661,9 +733,12 @@ class GAEngine(_EngineBase):
         outs = self._rollouts(specs, a.max_timesteps_per_episode)
         for r in ROLES:
             self._finish_role(r, outs[r])
-        packed = torch.stack([torch.stack([self._local[r][0].to(torch.float64),
-                                           self._local[r][1].to(torch.float64)], dim=1) for r in ROLES], dim=1)
-        allp = self.comm.all_gather_rows(packed.contiguous(), self.shard)          # [P, 3, 2]
+        if self.novelty_w:
+            self._member_novelty()
+        packed = torch.stack([torch.stack([self._local[r][0].to(torch.float64), self._local[r][1].to(torch.float64)]
+                                          + ([self._novelty_local[r]] if self.novelty_w else []), dim=1)
+                              for r in ROLES], dim=1)
+        allp = self.comm.all_gather_rows(packed.contiguous(), self.shard)          # [P, 3, 2 or 3]
         for i, role in enumerate(ROLES):
             reward = allp[:, i, 0]
             div = self.k.diversity_from_dist(allp[:, i, 1].to(torch.float32))
@@ -672,6 +747,37 @@ class GAEngine(_EngineBase):
             if self.compat or a.fitness_sharing:
                 reward = reward / (1.0 + div.to(reward.dtype))
             self.fitness[role] = reward.contiguous()
+            if self.novelty_w:
+                self.novelty[role] = allp[:, i, 2].contiguous()
+
+    def _member_novelty(self):
+        """Characterise this rank's members, gather the three roles' characterisations [P, 3, 160] in one
+        all-gather, and measure each member's k-NN novelty against the other members and the role's archive."""
+        bc = torch.empty((self.shard.n_local, len(ROLES), _lib.NOVELTY_BC_DIM), dtype=torch.float32,
+                         device=self.device)
+        for i, role in enumerate(ROLES):
+            self.k.novelty_bc(self.pop[role], layout.OBS_DIM[role], self.novelty_probe_obs[role], out=bc[:, i],
+                              status=self.status)
+        self._novelty_bc_all = bc_all = self.comm.all_gather_rows(bc, self.shard)
+        for i, role in enumerate(ROLES):
+            self._novelty_local[role] = self.k.ga_novelty_knn(bc[:, i], self.shard.row0, bc_all[:, i],
+                                                              self.novelty_ring[i], self.novelty_filled,
+                                                              self.novelty_k)
+        self._novelty_eval_filled = self.novelty_filled
+
+    def _novelty_append(self):
+        """Archive the characterisations of m members drawn on the device (the same ids on every rank, from the
+        gathered characterisations: no collective), at ``head`` in draw order; the bookkeeping stays on the host."""
+        h, m, A = self.novelty_head, self.novelty_m, self.novelty_A
+        n1 = min(m, A - h)
+        for i, role in enumerate(ROLES):
+            ids = self.k.ga_novelty_draw(self.seed, self.gen, role, m, self.P, self.device)
+            self.novelty_ids[role] = ids
+            rows = self._novelty_bc_all[:, i].index_select(0, ids)                 # [m, 160]
+            self.novelty_ring[i, h:h + n1] = rows[:n1]
+            self.novelty_ring[i, :m - n1] = rows[n1:]
+        self.novelty_head = (h + m) % A
+        self.novelty_filled = min(self.novelty_filled + m, A)
 
     def evaluate_role(self, role):
         """Evaluation loop of one role alone (tests / tools) -> global fitness fp64[P]."""
@@ -694,29 +800,50 @@ class GAEngine(_EngineBase):
         device and the three roles' elite rows travel in ONE all-reduce."""
         a = self.args
         E = int(a.elites_number)
+        # with novelty search one more row per role: the fitness-best member, for the HoF and the evaluation games
+        rows = E + 1 if self.novelty_w else E
         pitches = [layout.fc_pitch(layout.OBS_DIM[r]) for r in ROLES]
-        cat = torch.empty(E * sum(pitches), dtype=torch.float32, device=self.device)
+        cat = torch.empty(rows * sum(pitches), dtype=torch.float32, device=self.device)
         views, off = {}, 0
         for r, pitch in zip(ROLES, pitches):
-            views[r] = cat[off:off + E * pitch].view(E, pitch)
-            off += E * pitch
-        for role in ROLES:
-            ids = self.k.select_topk(self.fitness[role], E, order=self.order)        # replicated, bit-exact
-            self.elite_ids[role] = ids
+            views[r] = cat[off:off + rows * pitch].view(rows, pitch)
+            off += rows * pitch
+        if self.novelty_w:
+            # each rank ranks its own rows; F is combined in fp64 and gathered for the three roles at once
+            w = self.novelty_w
+            F_local = torch.stack([(1.0 - w) * self.k.centered_ranks(self.fitness[r], self.shard.row0,
+                                                                     self.shard.n_local)
+                                   + w * self.k.centered_ranks(self.novelty[r], self.shard.row0, self.shard.n_local)
+                                   for r in ROLES], dim=1)
+            F_all = self.comm.all_gather_rows(F_local.contiguous(), self.shard)      # [P, 3]
+        for i, role in enumerate(ROLES):
+            if self.novelty_w:
+                self.shaped_fitness[role] = F_all[:, i].contiguous()
+                ids = self.k.select_topk(self.shaped_fitness[role], E, order=self.order)
+                best = self.k.select_topk(self.fitness[role], 1, order=self.order)
+                self.elite_ids[role] = ids
+                ids = torch.cat([ids, best])
+            else:
+                ids = self.k.select_topk(self.fitness[role], E, order=self.order)    # replicated, bit-exact
+                self.elite_ids[role] = ids
             # owner rows, zeros elsewhere; summed over ranks = the elite / HoF broadcast
             self.k.gather_rows(self.pop[role], ids, row0=self.shard.row0, n_local=self.shard.n_local,
                                out=views[role])
         self.comm.all_reduce_sum(cat)
         for role in ROLES:
             in_dim = layout.OBS_DIM[role]
-            elites = views[role]
+            elites = views[role][:E] if self.novelty_w else views[role]
             self.elites[role] = elites
+            best = views[role][E:E + 1] if self.novelty_w else elites[0:1]
+            self.best_rows[role] = best[0]
             # HoF: append the best, drop the oldest (genetic_algorithm.py:270-275)
-            self.hof[role] = torch.cat([self.hof[role][1:], elites[0:1]], dim=0).contiguous()
+            self.hof[role] = torch.cat([self.hof[role][1:], best], dim=0).contiguous()
             # next population: row 0 = best unmutated, rows c>=1 = elites[(c-1)%E] + sigma*N(0,1)
             self.k.ga_repopulate(elites, layout.fc_dim(in_dim), self.sigma_dev(role), self.seed, role, self.gen,
                                  self.shard.row0, self.shard.n_local, out=self.pop[role],
                                  crossover_rate=float(getattr(a, "crossover_rate", 0.0)))
+        if self.novelty_w:
+            self._novelty_append()
 
     def step(self, sync=True):
         """One generation.  ``sync=True`` returns the evaluation triple (one host read);
@@ -726,28 +853,45 @@ class GAEngine(_EngineBase):
             self._join_eval()             # this generation's sigma is the previous generation's output
         self.evaluate()
         self.select_and_repopulate()
-        best = {r: self.elites[r][0] for r in ROLES}
+        best = self.best_rows
         self._finish_generation(best["agent_0"], best["agent_1"], best["adversary_0"])
         if self.history is not None:
             hs = self.host_state()
             self.check_status()
+            nov = self.novelty_w
+
+            def host(t):
+                return {r: t[r].cpu().numpy().copy() for r in ROLES} if nov else None
             self.history.append(dict(
                 fitness={r: self.fitness[r].cpu().numpy().copy() for r in ROLES},
                 elite_ids={r: self.elite_ids[r].cpu().numpy().copy() for r in ROLES},
                 diversity={r: float(self.diversity[r]) for r in ROLES}, evals=self.last_eval(),
-                sigma={r: float(hs["sigma_history"][r][self.gen]) for r in ROLES}))
+                sigma={r: float(hs["sigma_history"][r][self.gen]) for r in ROLES},
+                novelty=host(self.novelty), novelty_filled=self._novelty_eval_filled if nov else None,
+                shaped_fitness=host(self.shaped_fitness), novelty_archive_ids=host(self.novelty_ids)))
         self.gen += 1
         return self.last_eval() if sync else None
 
     def state_dict(self):
         """Everything a run needs to continue bit for bit: this rank's population shard, the HoF
-        ring, founders, generation state (sigmas, histories, counters), the host init-state stream."""
+        ring, founders, generation state (sigmas, histories, counters), the host init-state stream, and the
+        novelty-search settings, with novelty search its characterisation rings and their bookkeeping (the probe
+        observations are a function of the seed)."""
         sd = self._base_state()
         sd.update(pop={r: self.pop[r].cpu() for r in ROLES}, hof={r: self.hof[r].cpu() for r in ROLES},
-                  founder={r: self.founder[r].cpu() for r in ROLES})
+                  founder={r: self.founder[r].cpu() for r in ROLES}, ga_novelty=dict(self.novelty_opts))
+        if self.novelty_w:
+            sd.update(novelty_ring=self.novelty_ring.cpu().clone(), novelty_head=self.novelty_head,
+                      novelty_filled=self.novelty_filled)
         return sd
 
     def load_state_dict(self, sd):
+        """Refuses a checkpoint written with other novelty-search settings (one without them was written with
+        novelty search off)."""
+        saved = sd.get("ga_novelty", GA_NOVELTY_DEFAULTS)
+        if saved != self.novelty_opts:
+            raise ValueError(f"checkpoint was written with the GA novelty search {saved}, this run uses "
+                             f"{self.novelty_opts}")
         self._load_base_state(sd)
         if int(sd["row0"]) != self.shard.row0 or int(sd["n_local"]) != self.shard.n_local:
             raise ValueError("checkpoint shard does not match this rank's row block (same world size needed)")
@@ -755,6 +899,9 @@ class GAEngine(_EngineBase):
             self.pop[r].copy_(sd["pop"][r])
             self.hof[r] = sd["hof"][r].to(self.device).contiguous()
             self.founder[r].copy_(sd["founder"][r])
+        if self.novelty_w:
+            self.novelty_ring.copy_(sd["novelty_ring"])
+            self.novelty_head, self.novelty_filled = int(sd["novelty_head"]), int(sd["novelty_filled"])
 
 
 # ---------------------------------------------------------------------------
@@ -800,6 +947,7 @@ class ESEngine(_EngineBase):
         super().__init__(args, device, env, kernels, comm)
         self.P = int(args.population)
         self.options = es_options(args, "ES")
+        ga_novelty(args, "ES")                           # refuses the Co-GA options
         self.mirrored = self.options["mirrored_sampling"]
         self.shaping = self.options["fitness_shaping"] == "centered_rank"
         #: the fused apply kernel instead of K6 at lr + axpy (the default path)

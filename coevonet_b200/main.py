@@ -121,6 +121,21 @@ def parse_arguments(argv=None):
     p.add_argument("--es_novelty_archive", type=int, default=None,
                    help="ES, with --es_novelty_weight > 0: archive capacity A per role, 1 <= A <= 32768; the oldest "
                         "characterisation is overwritten once it is full (default 1024)")
+    p.add_argument("--ga_novelty_weight", type=float, default=0.0,
+                   help="GA: novelty search (Lehman & Stanley 2011) on the policy behaviour characterisation of "
+                        "--es_novelty_weight: parents are selected on (1 - w) * rank(fitness) + w * rank(novelty), the "
+                        "novelty being the mean distance to the k nearest characterisations among the other members "
+                        "and an archive.  1 = novelty alone, 0.5 = equal weight, 0 = off (the reference)")
+    p.add_argument("--ga_novelty_k", type=int, default=None,
+                   help="GA, with --ga_novelty_weight > 0: nearest neighbours k of the novelty, 1 <= k <= 32 "
+                        "(default 10)")
+    p.add_argument("--ga_novelty_archive", type=int, default=None,
+                   help="GA, with --ga_novelty_weight > 0: archive capacity A per role, 1 <= A <= 32768; slot 0 "
+                        "starts with the founder's characterisation, the oldest entry is overwritten once it is full "
+                        "(default 1024)")
+    p.add_argument("--ga_novelty_archive_add", type=int, default=None,
+                   help="GA, with --ga_novelty_weight > 0: members drawn at random each generation whose "
+                        "characterisations enter the archive, 1 <= m <= A (default 1)")
     p.add_argument("--play_discarded_hof_games", action="store_true",
                    help="GA, reference_compat: also simulate the hof_size-1 games per member whose reward the "
                         "reference overwrites (they never reach the fitness; skipped by default)")
@@ -211,12 +226,17 @@ class Args:
         self.es_novelty_weight = a.es_novelty_weight
         self.es_novelty_k = a.es_novelty_k
         self.es_novelty_archive = a.es_novelty_archive
-        from .engine import es_distribution, es_hof, es_novelty, es_options, es_subspace
+        self.ga_novelty_weight = a.ga_novelty_weight
+        self.ga_novelty_k = a.ga_novelty_k
+        self.ga_novelty_archive = a.ga_novelty_archive
+        self.ga_novelty_archive_add = a.ga_novelty_archive_add
+        from .engine import es_distribution, es_hof, es_novelty, es_options, es_subspace, ga_novelty
         es_options(self)                  # ValueError: odd population with mirrored sampling, an ES option with GA
         es_distribution(self)
         es_hof(self)
         es_subspace(self)
         es_novelty(self)
+        ga_novelty(self)
 
     def print_attributes(self, args=None):
         for k, v in vars(self).items():

@@ -17,7 +17,8 @@ MAX_CYCLES = 25
 
 #: kernels launched per C-ABI call (bench.py reports the total as ``gpu_launches``)
 _KERNELS_PER_CALL = {"cev_es_update_f32": 2, "cev_es_update_members_f32": 2, "cev_es_update_mirrored_f32": 2,
-                     "cev_es_update_diag_f32": 2, "cev_es_subspace_basis_f32": 6, "cev_fp32_peak": 4}
+                     "cev_es_update_diag_f32": 2, "cev_es_subspace_basis_f32": 6, "cev_fp32_peak": 4,
+                     "cev_ga_novelty_knn_f64": 2}
 launch_count = 0
 
 
@@ -687,6 +688,77 @@ def novelty_knn(bc, ring, filled, k, *, out=None):
         return out
     check(_call("cev_novelty_knn_f64", _h(dev), _ptr(bc), n, _ptr(ring), int(filled), int(k), _ptr(out), _stream(dev)),
           "cev_novelty_knn_f64")
+    return out
+
+
+def _need_bc_rows(name, what, t, dev):
+    """Characterisation rows handed to a kernel with their ``stride(0)`` as the row pitch."""
+    D = _lib.NOVELTY_BC_DIM
+    if not t.is_cuda or t.device != dev:
+        raise _lib.CevError(f"{name}: {what} must be a CUDA tensor on the device of the other operands")
+    if t.dtype != torch.float32 or t.dim() != 2 or t.shape[1] != D or t.stride(1) != 1 or \
+            (t.shape[0] and (t.stride(0) % 4 or t.data_ptr() % 16)):
+        raise _lib.CevError(f"{name}: {what} must be float32 [rows, {D}] with contiguous rows, a row stride that is a "
+                            "multiple of 4 and 16-byte alignment")
+
+
+def ga_novelty_knn(x, row0, pop, ring, filled, k, *, splits=0, out=None):
+    """Co-GA k-NN novelty: fp64 [n], entry i = the mean of the k_eff = min(k, P - 1 + filled) smallest fp32
+    Euclidean distances from ``x[i]`` (the characterisation of global row ``row0 + i``) to the other population
+    rows ``pop`` fp32 [P, 160] and the archive slots ``ring[:filled]`` fp32 [A, 160], summed in fp64 in ascending
+    order of (distance, index) (``cev_ga_novelty_knn_f64``).  ``x`` / ``pop``: contiguous rows, any row stride
+    that is a multiple of 4 (e.g. one role's column of a gathered [P, 3, 160] block).  ``splits``: candidate
+    ranges searched by separate CTAs (0 = chosen from the shape); the result does not depend on it."""
+    dev = _need_cuda(ring, out)
+    if dev is None:
+        raise _lib.CevError("ga_novelty_knn: needs CUDA tensors (no CPU fallback)")
+    _need_bc_rows("ga_novelty_knn", "x", x, dev)
+    _need_bc_rows("ga_novelty_knn", "pop", pop, dev)
+    D = _lib.NOVELTY_BC_DIM
+    if ring.dtype != torch.float32 or ring.dim() != 2 or ring.shape[1] != D:
+        raise _lib.CevError(f"ga_novelty_knn: ring must be float32 [A, {D}]")
+    n, P = x.shape[0], pop.shape[0]
+    if P < 1:
+        raise _lib.CevError("ga_novelty_knn: the population needs at least one row")
+    if not 0 <= int(filled) <= min(ring.shape[0], _lib.NOVELTY_MAX_ARCHIVE):
+        raise _lib.CevError(f"ga_novelty_knn: filled must be in [0, {min(ring.shape[0], _lib.NOVELTY_MAX_ARCHIVE)}], "
+                            f"not {filled}")
+    if P - 1 + int(filled) < 1:
+        raise _lib.CevError("ga_novelty_knn: a member needs at least one other candidate (P = 1 needs filled >= 1)")
+    if not 1 <= int(k) <= _lib.NOVELTY_MAX_K:
+        raise _lib.CevError(f"ga_novelty_knn: k must be in [1, {_lib.NOVELTY_MAX_K}], not {k}")
+    if not 0 <= int(row0) <= P - n:
+        raise _lib.CevError(f"ga_novelty_knn: rows [row0, row0 + {n}) must lie in [0, {P}), row0 = {row0}")
+    if int(splits) < 0:
+        raise _lib.CevError(f"ga_novelty_knn: splits must be >= 0, not {splits}")
+    if out is None:
+        out = torch.empty(n, dtype=torch.float64, device=dev)
+    if out.dtype != torch.float64 or tuple(out.shape) != (n,):
+        raise _lib.CevError(f"ga_novelty_knn: out must be float64 [{n}]")
+    if n == 0:
+        return out
+    check(_call("cev_ga_novelty_knn_f64", _h(dev), _ptr(x), x.stride(0), n, int(row0), _ptr(pop), pop.stride(0), P,
+                _ptr(ring), int(filled), int(k), int(splits), _ptr(out), _stream(dev)),
+          "cev_ga_novelty_knn_f64")
+    return out
+
+
+def ga_novelty_draw(seed, gen, role, m, P, device, *, out=None):
+    """Co-GA novelty archive: int64 [m] population ids in [0, P) whose characterisations enter ``role``'s archive
+    after generation ``gen``'s selection, in draw order, from the Philox stream of kind ``KIND_GA_NOVELTY`` keyed
+    by (seed, gen, role), the same on every rank."""
+    if out is None:
+        out = torch.empty(int(m), dtype=torch.int64, device=device)
+    dev = _need_cuda(out)
+    if dev is None:
+        raise _lib.CevError("ga_novelty_draw: needs a CUDA device (no CPU fallback)")
+    if out.dtype != torch.int64 or tuple(out.shape) != (int(m),):
+        raise _lib.CevError(f"ga_novelty_draw: out must be int64 [{m}]")
+    if not 1 <= int(P) <= 1 << 32:
+        raise _lib.CevError(f"ga_novelty_draw: P must be in [1, 2^32], not {P}")
+    role_id = layout.ROLE_ID[role] if isinstance(role, str) else int(role)
+    check(_call("cev_ga_novelty_draw_i64", _h(dev), int(seed), int(gen), role_id, int(m), int(P), _ptr(out),
+                _stream(dev)), "cev_ga_novelty_draw_i64")
     return out
 
 

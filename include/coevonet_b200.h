@@ -492,6 +492,36 @@ int cev_novelty_knn_f64(cev_handle* h, const float* bc, int64_t n, const float* 
                         double* novelty, cev_stream stream);
 
 /*
+ * Co-GA novelty search (Lehman & Stanley 2011, with a GA on deep networks as in Such et al. 2017): the novelty of
+ * a member is measured against the whole current population plus an archive of earlier members' characterisations.
+ *
+ * k-NN novelty of the n members x fp32 [n][x_pitch] (characterisations of the global rows row0 .. row0 + n - 1)
+ * against the candidates: the P population rows pop fp32 [P][pop_pitch] (candidate index c in [0, P); e.g. one
+ * role's column of a gathered [P][3][160] block, pop_pitch = 480) and the archive slots ring fp32 [filled][160]
+ * (index P + s).  A member is never its own candidate (excluded by id, not by value).  Per (member, candidate):
+ *   e_t = fl(q_t - x_t), s = fmaf(e_t, e_t, s)   fp32 from +0, t = 0 .. 159 in order;  dist = sqrt(s) fp32 (rounded)
+ * The candidates are ordered by (dist, index), a NaN dist after every number; with k_eff = min(k, P - 1 + filled)
+ *   novelty[i] = (sum of the k_eff smallest dist, in that order, fp64 from +0, one rounding per add) / k_eff
+ * (a NaN among them makes the novelty NaN).  1 <= k <= CEV_NOVELTY_MAX_K, 0 <= filled <= CEV_NOVELTY_MAX_ARCHIVE,
+ * P - 1 + filled >= 1, row0 + n <= P; pitches are multiples of 4 floats >= 160 and the rows 16-byte aligned.
+ * `splits` candidate ranges are searched by separate CTAs (0 = chosen from the shape, clamped to the candidate
+ * tiles) and merged; the result does not depend on it, on the tiling or on row0's block, so a sharded population
+ * gives the values of an unsharded one.  Deterministic.  novelty: DEVICE fp64 [n].  Uses the handle's workspace.
+ */
+#define CEV_KIND_GA_NOVELTY 9           /* Co-GA novelty archive draws: member 0, role = the role */
+int cev_ga_novelty_knn_f64(cev_handle* h, const float* x, int64_t x_pitch, int64_t n, int64_t row0, const float* pop,
+                           int64_t pop_pitch, int64_t P, const float* ring, int64_t filled, int k, int splits,
+                           double* novelty, cev_stream stream);
+
+/*
+ * The m population ids whose characterisations enter the archive of `role` after generation gen's selection, in
+ * draw order: id_j = (uint64(w_j) * P) >> 32 with w_j word (j & 3) of the Philox block (j >> 2, 0, gen,
+ * role | CEV_KIND_GA_NOVELTY << 8) keyed by seed.  out: DEVICE int64 [m].  1 <= P <= 2^32.
+ */
+int cev_ga_novelty_draw_i64(cev_handle* h, uint64_t seed, uint32_t gen, int role, int m, int64_t P, int64_t* out,
+                            cev_stream stream);
+
+/*
  * K7 -- fitness-sharing distances.  Replaces the distance loop of
  * diversity_penalty (utils/game_logic_functions.py:12-37):
  * d[i] = || pop[i] - ref ||_2 over the perturbable (Linear) parameters.
