@@ -124,6 +124,11 @@ _SIGNATURES = {
     "cev_ga_novelty_knn_f64": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int64, c_int64,
                                        c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p]),
     "cev_ga_novelty_draw_i64": (c_int, [c_void_p, c_uint64, c_uint32, c_int, c_int, c_int64, c_void_p, c_void_p]),
+    "cev_ga_safe_scale_f32": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int, c_void_p, c_float, c_void_p, c_int64,
+                                      c_void_p, c_void_p]),
+    "cev_ga_repopulate_safe_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_float, c_void_p,
+                                           c_float, c_uint64, c_int, c_uint32, c_int64, c_int64, c_void_p, c_void_p,
+                                           c_void_p]),
     "cev_diversity_dist_f32": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_int,
                                        c_void_p, c_void_p]),
     "cev_deepqn_forward": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_void_p, c_int, c_int,

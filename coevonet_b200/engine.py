@@ -317,6 +317,34 @@ def ga_novelty(args, algorithm=None):
     return {"ga_novelty_weight": w, "ga_novelty_k": k, "ga_novelty_archive": A, "ga_novelty_archive_add": m}
 
 
+#: Co-GA safe mutations through output gradients (SM-G-SUM, Lehman et al. 2018) and their defaults: off; with the
+#: option on, an unset floor becomes GA_SAFE_MUTATION_DEFAULT_FLOOR (no mutation is amplified more than 100x)
+GA_SAFE_MUTATION_DEFAULTS = {"ga_safe_mutation": False, "ga_safe_mutation_floor": None}
+GA_SAFE_MUTATION_DEFAULT_FLOOR = 0.01
+
+
+def ga_safe_mutation(args, algorithm=None):
+    """The Co-GA safe-mutation settings of ``args`` (an absent attribute is its default), validated: ``ValueError``
+    for either setting with the ES, for a floor given without ``ga_safe_mutation`` and for a floor that is not finite
+    and > 0 (as a float32, the kernel's type).  With the option on an unset floor becomes 0.01."""
+    opts = {k: getattr(args, k, d) for k, d in GA_SAFE_MUTATION_DEFAULTS.items()}
+    opts["ga_safe_mutation"] = bool(opts["ga_safe_mutation"])
+    if opts != GA_SAFE_MUTATION_DEFAULTS and (algorithm or getattr(args, "algorithm", "ES")) != "GA":
+        changed = sorted(k for k in opts if opts[k] != GA_SAFE_MUTATION_DEFAULTS[k])
+        raise ValueError(f"{', '.join(changed)}: Co-GA options, not available with --algorithm ES")
+    if not opts["ga_safe_mutation"]:
+        if opts["ga_safe_mutation_floor"] is not None:
+            raise ValueError("ga_safe_mutation_floor needs ga_safe_mutation")
+        return dict(GA_SAFE_MUTATION_DEFAULTS)
+    floor = GA_SAFE_MUTATION_DEFAULT_FLOOR if opts["ga_safe_mutation_floor"] is None \
+        else float(opts["ga_safe_mutation_floor"])
+    with np.errstate(over="ignore"):
+        f32 = np.float32(floor)
+    if not (np.isfinite(f32) and f32 > 0):
+        raise ValueError(f"ga_safe_mutation_floor must be finite and > 0, not {floor}")
+    return {"ga_safe_mutation": True, "ga_safe_mutation_floor": floor}
+
+
 def default_sigma_learning_rate(d):
     """SNES's sigma learning rate for d parameters, (3 + ln d) / (5 sqrt d) (Schaul et al. 2011), in fp64."""
     return (3.0 + np.log(float(d))) / (5.0 * np.sqrt(float(d)))
@@ -613,7 +641,11 @@ class GAEngine(_EngineBase):
     characterisations after every selection.  A member's novelty is the mean distance to its k nearest among the
     other members and the archive (``cev_ga_novelty_knn_f64``); parents are selected on F = (1 - w) cr(fitness) +
     w cr(novelty) (cr: centered ranks of the global vectors), while the Hall of Fame and the evaluation games take
-    the fitness-best member."""
+    the fitness-best member.
+
+    Opt-in safe mutations (``ga_safe_mutation``, SM-G-SUM): after the elite all-reduce every rank computes the scale
+    rows of the E elites on the same probe observations (``cev_ga_safe_scale_f32``; deterministic, so replicated
+    without a collective), and K3 multiplies each parameter's fl(sigma z) by the scale of the elite it came from."""
 
     kind = "GA"
 
@@ -626,6 +658,12 @@ class GAEngine(_EngineBase):
         es_subspace(args, "GA")
         es_novelty(args, "GA")
         self.novelty_opts = ga_novelty(args, "GA")
+        self.safe_opts = ga_safe_mutation(args, "GA")
+        #: safe mutations (SM-G-SUM): on / off, and the floor of the sensitivity
+        self.safe = self.safe_opts["ga_safe_mutation"]
+        self.safe_floor = self.safe_opts["ga_safe_mutation_floor"]
+        #: this generation's scale rows per role, fp32 [E, pitch] (``ga_safe_scale`` of the elites)
+        self.safe_scale = {r: None for r in ROLES}
         #: novelty weight w (0: off), nearest neighbours k, archive capacity A and additions per generation m
         self.novelty_w = self.novelty_opts["ga_novelty_weight"]
         self.novelty_k = self.novelty_opts["ga_novelty_k"]
@@ -653,9 +691,11 @@ class GAEngine(_EngineBase):
         self._novelty_local = {r: None for r in ROLES}
         self._novelty_bc_all = None
         self.novelty_ids = {r: None for r in ROLES}
-        if self.novelty_w:
+        if self.novelty_w or self.safe:
+            # one tensor per role, shared by the novelty search and the safe mutations
             states = self.k.init_states(self.seed, NOVELTY_PROBE_TAG, _lib.NOVELTY_PROBES, self.device)
             self.novelty_probe_obs = {r: self.k.novelty_probe_obs(states, r) for r in ROLES}
+        if self.novelty_w:
             self.novelty_ring = torch.zeros((len(ROLES), self.novelty_A, _lib.NOVELTY_BC_DIM), dtype=torch.float32,
                                             device=self.device)
             for i, r in enumerate(ROLES):          # slot 0: the founder the reference measures diversity against
@@ -839,9 +879,14 @@ class GAEngine(_EngineBase):
             # HoF: append the best, drop the oldest (genetic_algorithm.py:270-275)
             self.hof[role] = torch.cat([self.hof[role][1:], best], dim=0).contiguous()
             # next population: row 0 = best unmutated, rows c>=1 = elites[(c-1)%E] + sigma*N(0,1)
+            # (with safe mutations: + fl(sigma*N(0,1)) * c, c the scale row of the elite)
+            extra = {}
+            if self.safe:
+                self.safe_scale[role] = extra["scale"] = self.k.ga_safe_scale(
+                    elites, in_dim, self.novelty_probe_obs[role], self.safe_floor, status=self.status)
             self.k.ga_repopulate(elites, layout.fc_dim(in_dim), self.sigma_dev(role), self.seed, role, self.gen,
                                  self.shard.row0, self.shard.n_local, out=self.pop[role],
-                                 crossover_rate=float(getattr(a, "crossover_rate", 0.0)))
+                                 crossover_rate=float(getattr(a, "crossover_rate", 0.0)), **extra)
         if self.novelty_w:
             self._novelty_append()
 
@@ -868,9 +913,23 @@ class GAEngine(_EngineBase):
                 diversity={r: float(self.diversity[r]) for r in ROLES}, evals=self.last_eval(),
                 sigma={r: float(hs["sigma_history"][r][self.gen]) for r in ROLES},
                 novelty=host(self.novelty), novelty_filled=self._novelty_eval_filled if nov else None,
-                shaped_fitness=host(self.shaped_fitness), novelty_archive_ids=host(self.novelty_ids)))
+                shaped_fitness=host(self.shaped_fitness), novelty_archive_ids=host(self.novelty_ids),
+                safe_mutation_scale=self._safe_scale_stats() if self.safe else None))
         self.gen += 1
         return self.last_eval() if sync else None
+
+    def _safe_scale_stats(self):
+        """Per role the mean, min and max of this generation's scales c over the E x D entries of the elites, and the
+        count of entries at 1 / floor (reduced on the device, one host read)."""
+        at_floor = np.float32(1.0) / np.float32(self.safe_floor)
+        stats = []
+        for r in ROLES:
+            c = self.safe_scale[r][:, :layout.fc_dim(layout.OBS_DIM[r])]
+            stats.append(torch.stack([c.mean(dtype=torch.float64), c.min().double(), c.max().double(),
+                                      (c == float(at_floor)).sum().double()]))
+        host = torch.stack(stats).cpu().numpy()
+        return {r: dict(mean=float(v[0]), min=float(v[1]), max=float(v[2]), n_floor=int(v[3]))
+                for r, v in zip(ROLES, host)}
 
     def state_dict(self):
         """Everything a run needs to continue bit for bit: this rank's population shard, the HoF
@@ -879,19 +938,24 @@ class GAEngine(_EngineBase):
         observations are a function of the seed)."""
         sd = self._base_state()
         sd.update(pop={r: self.pop[r].cpu() for r in ROLES}, hof={r: self.hof[r].cpu() for r in ROLES},
-                  founder={r: self.founder[r].cpu() for r in ROLES}, ga_novelty=dict(self.novelty_opts))
+                  founder={r: self.founder[r].cpu() for r in ROLES}, ga_novelty=dict(self.novelty_opts),
+                  ga_safe_mutation=dict(self.safe_opts))
         if self.novelty_w:
             sd.update(novelty_ring=self.novelty_ring.cpu().clone(), novelty_head=self.novelty_head,
                       novelty_filled=self.novelty_filled)
         return sd
 
     def load_state_dict(self, sd):
-        """Refuses a checkpoint written with other novelty-search settings (one without them was written with
-        novelty search off)."""
+        """Refuses a checkpoint written with other novelty-search or safe-mutation settings (one without them was
+        written with the option off)."""
         saved = sd.get("ga_novelty", GA_NOVELTY_DEFAULTS)
         if saved != self.novelty_opts:
             raise ValueError(f"checkpoint was written with the GA novelty search {saved}, this run uses "
                              f"{self.novelty_opts}")
+        saved = sd.get("ga_safe_mutation", GA_SAFE_MUTATION_DEFAULTS)
+        if saved != self.safe_opts:
+            raise ValueError(f"checkpoint was written with the GA safe mutations {saved}, this run uses "
+                             f"{self.safe_opts}")
         self._load_base_state(sd)
         if int(sd["row0"]) != self.shard.row0 or int(sd["n_local"]) != self.shard.n_local:
             raise ValueError("checkpoint shard does not match this rank's row block (same world size needed)")
@@ -948,6 +1012,7 @@ class ESEngine(_EngineBase):
         self.P = int(args.population)
         self.options = es_options(args, "ES")
         ga_novelty(args, "ES")                           # refuses the Co-GA options
+        ga_safe_mutation(args, "ES")
         self.mirrored = self.options["mirrored_sampling"]
         self.shaping = self.options["fitness_shaping"] == "centered_rank"
         #: the fused apply kernel instead of K6 at lr + axpy (the default path)

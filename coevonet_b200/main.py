@@ -136,6 +136,16 @@ def parse_arguments(argv=None):
     p.add_argument("--ga_novelty_archive_add", type=int, default=None,
                    help="GA, with --ga_novelty_weight > 0: members drawn at random each generation whose "
                         "characterisations enter the archive, 1 <= m <= A (default 1)")
+    p.add_argument("--ga_safe_mutation", action="store_true",
+                   help="GA: safe mutations through output gradients (SM-G-SUM, Lehman et al. 2018): each parameter's "
+                        "mutation sigma * N(0, 1) is divided by s, the size of the response of the network's 5 logits "
+                        "to that parameter summed over the 32 probe observations of the novelty search (clamped below "
+                        "by --ga_safe_mutation_floor; a parameter no logit responds to keeps the plain mutation).  "
+                        "sigma is then the step BEFORE the per-parameter division, so a run typically needs a larger "
+                        "--initial_mutation_power_*.  Off = the reference's mutation")
+    p.add_argument("--ga_safe_mutation_floor", type=float, default=None,
+                   help="GA, with --ga_safe_mutation: the floor of s, finite and > 0; no parameter's mutation is "
+                        "multiplied by more than 1 / floor (default 0.01, i.e. 100x)")
     p.add_argument("--play_discarded_hof_games", action="store_true",
                    help="GA, reference_compat: also simulate the hof_size-1 games per member whose reward the "
                         "reference overwrites (they never reach the fitness; skipped by default)")
@@ -230,13 +240,16 @@ class Args:
         self.ga_novelty_k = a.ga_novelty_k
         self.ga_novelty_archive = a.ga_novelty_archive
         self.ga_novelty_archive_add = a.ga_novelty_archive_add
-        from .engine import es_distribution, es_hof, es_novelty, es_options, es_subspace, ga_novelty
+        self.ga_safe_mutation = a.ga_safe_mutation
+        self.ga_safe_mutation_floor = a.ga_safe_mutation_floor
+        from .engine import es_distribution, es_hof, es_novelty, es_options, es_subspace, ga_novelty, ga_safe_mutation
         es_options(self)                  # ValueError: odd population with mirrored sampling, an ES option with GA
         es_distribution(self)
         es_hof(self)
         es_subspace(self)
         es_novelty(self)
         ga_novelty(self)
+        ga_safe_mutation(self)
 
     def print_attributes(self, args=None):
         for k, v in vars(self).items():

@@ -7,6 +7,7 @@ There is no CPU path: non-CUDA tensors raise.
 from __future__ import annotations
 
 import ctypes
+import math
 
 import torch
 
@@ -18,7 +19,7 @@ MAX_CYCLES = 25
 #: kernels launched per C-ABI call (bench.py reports the total as ``gpu_launches``)
 _KERNELS_PER_CALL = {"cev_es_update_f32": 2, "cev_es_update_members_f32": 2, "cev_es_update_mirrored_f32": 2,
                      "cev_es_update_diag_f32": 2, "cev_es_subspace_basis_f32": 6, "cev_fp32_peak": 4,
-                     "cev_ga_novelty_knn_f64": 2}
+                     "cev_ga_novelty_knn_f64": 2, "cev_ga_safe_scale_f32": 5}
 launch_count = 0
 
 
@@ -287,19 +288,28 @@ def _sigma_args(sigma):
 
 
 def ga_repopulate(elites, dim, sigma, seed, role, gen, row0, n_rows, *, out=None, noise_out=None,
-                  crossover_rate=0.0):
+                  crossover_rate=0.0, scale=None):
     """K3: rows [row0, row0+n_rows) of the next GA population.  ``crossover_rate`` > 0 adds uniform
-    crossover between two elites before the mutation (an extension; 0 = the reference)."""
-    dev = _need_cuda(elites, out, noise_out)
+    crossover between two elites before the mutation (an extension; 0 = the reference).  ``scale`` fp32 [E, pitch]
+    (``ga_safe_scale`` of the elites) turns the mutation of parameter j into fl(fl(sigma * z_j) * c_j), c_j from the
+    elite the parameter was copied from (``cev_ga_repopulate_safe_f32``); None = the plain K3."""
+    dev = _need_cuda(elites, out, noise_out, scale)
     sig, sig_dev = _sigma_args(sigma)
     pitch = elites.stride(0)
     if out is None:
         out = torch.empty((n_rows, pitch), dtype=torch.float32, device=dev)
     role_id = layout.ROLE_ID[role] if isinstance(role, str) else int(role)
-    check(_call("cev_ga_repopulate_f32", 
-        _h(dev), _ptr(elites), elites.shape[0], int(dim), pitch, sig, sig_dev, float(crossover_rate),
-        int(seed), role_id, int(gen), int(row0), int(n_rows), _ptr(out), _ptr(noise_out),
-        _stream(dev)), "cev_ga_repopulate_f32")
+    if scale is None:
+        check(_call("cev_ga_repopulate_f32", 
+            _h(dev), _ptr(elites), elites.shape[0], int(dim), pitch, sig, sig_dev, float(crossover_rate),
+            int(seed), role_id, int(gen), int(row0), int(n_rows), _ptr(out), _ptr(noise_out),
+            _stream(dev)), "cev_ga_repopulate_f32")
+        return out
+    if scale.dtype != torch.float32 or tuple(scale.shape) != tuple(elites.shape) or scale.stride(0) != pitch:
+        raise _lib.CevError(f"ga_repopulate: scale must be float32 {tuple(elites.shape)}, laid out like the elites")
+    check(_call("cev_ga_repopulate_safe_f32", _h(dev), _ptr(elites), _ptr(scale), elites.shape[0], int(dim), pitch,
+                sig, sig_dev, float(crossover_rate), int(seed), role_id, int(gen), int(row0), int(n_rows), _ptr(out),
+                _ptr(noise_out), _stream(dev)), "cev_ga_repopulate_safe_f32")
     return out
 
 
@@ -759,6 +769,39 @@ def ga_novelty_draw(seed, gen, role, m, P, device, *, out=None):
     role_id = layout.ROLE_ID[role] if isinstance(role, str) else int(role)
     check(_call("cev_ga_novelty_draw_i64", _h(dev), int(seed), int(gen), role_id, int(m), int(P), _ptr(out),
                 _stream(dev)), "cev_ga_novelty_draw_i64")
+    return out
+
+
+def ga_safe_scale(elites, in_dim, probe_obs, floor, *, out=None, status=None):
+    """Safe-mutation scales (SM-G-SUM): fp32 [E, pitch], entry j of row e = 1 / max(s_j, floor), or 1 where s_j = 0,
+    with s_j = sqrt(sum_k (sum_t dy_k(x_t) / dW_j)^2) the response of the 5 logits of network row ``elites[e]`` to
+    parameter j on the 32 probe observations ``probe_obs`` fp32 [32, in_dim]; padding entries are 0
+    (``cev_ga_safe_scale_f32``).  ``elites``: fp32 [E, pitch >= fc_dim] with contiguous rows, 16-byte aligned.
+    A non-finite logit or gradient sets ``status``."""
+    dev = _need_cuda(probe_obs, status)
+    _need_rows(dev, elites)
+    E, D = elites.shape[0], layout.fc_dim(in_dim)
+    if in_dim not in (8, 10):
+        raise _lib.CevError(f"ga_safe_scale: in_dim must be 8 or 10, not {in_dim}")
+    if elites.dtype != torch.float32 or elites.shape[1] < D or (E and (elites.stride(0) % 4 or elites.data_ptr() % 16)):
+        raise _lib.CevError(f"ga_safe_scale: elites must be float32 [E, >= {D}], row stride a multiple of 4, "
+                            "16-byte aligned")
+    if probe_obs.dtype != torch.float32 or tuple(probe_obs.shape) != (_lib.NOVELTY_PROBES, in_dim):
+        raise _lib.CevError(f"ga_safe_scale: probe_obs must be float32 [{_lib.NOVELTY_PROBES}, {in_dim}]")
+    f = float(floor)
+    if not (math.isfinite(f) and f > 0.0):
+        raise _lib.CevError(f"ga_safe_scale: floor must be finite and > 0, not {floor}")
+    if out is None:
+        out = torch.empty((E, elites.shape[1]), dtype=torch.float32, device=dev)
+    _need_rows(dev, out)
+    if out.dtype != torch.float32 or out.shape[0] != E or out.shape[1] < D or (E and out.stride(0) % 4):
+        raise _lib.CevError(f"ga_safe_scale: out must be float32 [{E}, >= {D}], row stride a multiple of 4")
+    if status is not None and (status.dtype != torch.int32 or status.numel() != 1):
+        raise _lib.CevError("ga_safe_scale: status must be a one-element int32 tensor")
+    if E == 0:
+        return out
+    check(_call("cev_ga_safe_scale_f32", _h(dev), _ptr(elites), elites.stride(0), int(in_dim), E, _ptr(probe_obs),
+                f, _ptr(out), out.stride(0), _ptr(status), _stream(dev)), "cev_ga_safe_scale_f32")
     return out
 
 

@@ -522,6 +522,35 @@ int cev_ga_novelty_draw_i64(cev_handle* h, uint64_t seed, uint32_t gen, int role
                             cev_stream stream);
 
 /*
+ * Co-GA safe mutations through output gradients (SM-G-SUM, Lehman, Chen, Clune & Stanley, GECCO 2018): each
+ * parameter's mutation is divided by how strongly the network's logits respond to it on the probe observations.
+ *
+ * Scale rows of E parent rows fp32 [E][pitch] of in_dim 8 or 10 (e.g. the gathered elites) on the 32 probe
+ * observations probe_obs fp32 [32][in_dim] (cev_novelty_probe_obs_f32).  With y_k(x_t), k = 0..4, the logits of
+ * the FCNetwork on probe t (ReLU' = [input > 0]; LayerNorm biased-variance, eps 1e-5), for every entry j < D =
+ * cev_fc_dim(in_dim), LayerNorm gains and biases included:
+ *   G_kj = sum_t dy_k(x_t) / dW_j,  s_j = sqrt(sum_k G_kj^2),
+ *   c_j  = 1 if s_j == 0 (no logit responds to the entry), else fl32(1 / max(s_j, floor))
+ * written to scale fp32 [E][scale_pitch]; entries [D, scale_pitch) are 0.  FP32 with every sum in a fixed order:
+ * deterministic, and row e does not depend on E.  A non-finite logit or gradient sets CEV_STATUS_NONFINITE in
+ * *status (may be NULL).  floor: finite and > 0.  Pitches are multiples of 4 floats >= D, rows 16-byte aligned.
+ * Five kernel launches; uses the handle's workspace (about 640 KB per parent).
+ */
+int cev_ga_safe_scale_f32(cev_handle* h, const float* rows, int64_t pitch, int in_dim, int E, const float* probe_obs,
+                          float floor, float* scale, int64_t scale_pitch, int32_t* status, cev_stream stream);
+
+/*
+ * K3 with safe mutations: cev_ga_repopulate_f32 (same arguments, same Philox streams and crossover) where the
+ * mutation of parameter j of child c >= 1 is fl(p_j + fl(fl(sigma * z_j) * c_j)), c_j from scale fp32 [E][pitch]
+ * (cev_ga_safe_scale_f32 of the same elites) of the elite p_j was copied from.  A scale row of ones gives
+ * cev_ga_repopulate_f32's rows bit for bit.
+ */
+int cev_ga_repopulate_safe_f32(cev_handle* h, const float* elites, const float* scale, int E, int D, int64_t pitch,
+                               float sigma, const double* sigma_dev, float crossover_rate, uint64_t seed, int role,
+                               uint32_t gen, int64_t row0, int64_t n_rows, float* out, float* noise_out,
+                               cev_stream stream);
+
+/*
  * K7 -- fitness-sharing distances.  Replaces the distance loop of
  * diversity_penalty (utils/game_logic_functions.py:12-37):
  * d[i] = || pop[i] - ref ||_2 over the perturbable (Linear) parameters.
