@@ -22,6 +22,9 @@ KIND_ES, KIND_GA, KIND_ENV, KIND_FRAMES, KIND_INIT, KIND_XOVER, KIND_ES_MIRROR, 
 KIND_ES_SUBSPACE = 8
 KIND_GA_NOVELTY = 9
 SUBSPACE_MAX_DIM = 32
+#: column chunks of the LM-MA-ES projection and apply, and rank splits of its reduction (es_lmma.cu): they fix the
+#: summation order, which oracle/es_lmma.py restates
+LMMA_PROJECT_CHUNK, LMMA_APPLY_CHUNK, LMMA_REDUCE_SPLIT = 2048, 4096, 8
 #: Co-ES novelty search (CEV_NOVELTY_* in include/coevonet_b200.h): probe observations per behaviour
 #: characterisation, its length (probes x actions), and the limits of k and of the archive
 NOVELTY_PROBES, NOVELTY_BC_DIM, NOVELTY_MAX_K, NOVELTY_MAX_ARCHIVE = 32, 160, 32, 32768
@@ -117,7 +120,19 @@ _SIGNATURES = {
                                             c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "cev_es_subspace_basis_f32": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, POINTER(c_int), c_void_p,
                                           c_void_p, c_void_p]),
-    "cev_novelty_probe_obs_f32": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
+    "cev_es_lmma_project_f32": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_int, POINTER(c_double), c_int,
+                                        c_uint64, c_int, c_uint32, c_int64, c_int64, c_void_p, c_void_p, c_void_p,
+                                        c_void_p, c_void_p]),
+    "cev_es_perturb_lmma_f32": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int64, c_int, c_void_p,
+                                        c_float, c_uint64, c_int, c_uint32, c_int64, c_int64, c_int64, c_void_p,
+                                        c_void_p]),
+    "cev_es_lmma_reduce_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_uint64, c_int,
+                                       c_uint32, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "cev_es_lmma_apply_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int,
+                                      POINTER(c_int), POINTER(c_double), POINTER(c_double), POINTER(c_double),
+                                      c_double, POINTER(c_double), c_void_p, c_void_p, c_double, c_double, c_void_p,
+                                      c_void_p, c_void_p, c_void_p]),
+    "cev_novelty_probe_obs_f32":(c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "cev_novelty_bc_f32": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
                                    c_void_p]),
     "cev_novelty_knn_f64": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_int, c_void_p, c_void_p]),

@@ -153,9 +153,17 @@ def es_options(args, algorithm=None):
     return opts
 
 
-#: the Co-ES search distribution and its default: one isotropic Gaussian per role (the reference), or separable NES
-#: (a per-parameter mutation strength, Schaul et al. 2011); sigma_learning_rate None = default_sigma_learning_rate
+#: the Co-ES search distribution and its default: one isotropic Gaussian per role (the reference), separable NES
+#: (a per-parameter mutation strength, Schaul et al. 2011) or LM-MA-ES (limited-memory matrix adaptation, Loshchilov
+#: et al. 2019); sigma_learning_rate None = default_sigma_learning_rate; es_lmma_memory None = LMMA_DEFAULT_MEMORY
+#: with lmma, and only then part of the settings (so the settings of the other distributions keep their two keys)
 ES_DISTRIBUTION_DEFAULTS = {"es_distribution": "isotropic", "sigma_learning_rate": None}
+#: LM-MA-ES direction vectors per role.  Not the paper's 4 + floor(3 ln n) = 39: vector j moves at c_c,j = lam / (4^j n),
+#: so at lam = 1024 and n ~ 138 k vector 5 reaches ~14 % of its stationary norm in 1e4 generations and vector 7 < 1 %;
+#: vectors past ~8 cost a K5 term each and contribute nothing in runs of this size
+LMMA_DEFAULT_MEMORY = 8
+#: the fewest Linear entries of a role's row (the adversary's): LM-MA-ES needs c_sigma = 2 lam / n < 1 for every role
+LMMA_MIN_DIM = min(len(layout.fc_perturbable_index(d)) for d in set(layout.OBS_DIM.values()))
 
 
 def es_distribution(args, algorithm=None):
@@ -164,8 +172,9 @@ def es_distribution(args, algorithm=None):
     Adam, L2 weight decay or ``--adaptive`` (they would fight the per-parameter step) and for a
     ``sigma_learning_rate`` that is not a finite number > 0 or is given without ``separable``."""
     opts = {k: getattr(args, k, d) for k, d in ES_DISTRIBUTION_DEFAULTS.items()}
-    if opts["es_distribution"] not in ("isotropic", "separable"):
-        raise ValueError(f"es_distribution must be 'isotropic' or 'separable', not {opts['es_distribution']!r}")
+    memory = getattr(args, "es_lmma_memory", None)
+    if opts["es_distribution"] not in ("isotropic", "separable", "lmma"):
+        raise ValueError(f"es_distribution must be 'isotropic', 'separable' or 'lmma', not {opts['es_distribution']!r}")
     if opts != ES_DISTRIBUTION_DEFAULTS and (algorithm or getattr(args, "algorithm", "ES")) == "GA":
         changed = sorted(k for k in opts if opts[k] != ES_DISTRIBUTION_DEFAULTS[k])
         raise ValueError(f"{', '.join(changed)}: Co-ES options, not available with --algorithm GA")
@@ -182,7 +191,58 @@ def es_distribution(args, algorithm=None):
                              "'adam' or a nonzero l2_coeff")
         if getattr(args, "adaptive", False):
             raise ValueError("es_distribution 'separable' adapts every sigma itself: not available with --adaptive")
+    if memory is not None and opts["es_distribution"] != "lmma":
+        raise ValueError("es_lmma_memory needs es_distribution 'lmma'")
+    if opts["es_distribution"] == "lmma":
+        opts["es_lmma_memory"] = memory
+        _lmma_refusals(args, opts)
     return opts
+
+
+def _lmma_refusals(args, opts):
+    """The settings LM-MA-ES refuses (``ValueError``), and its memory m resolved into ``opts``."""
+    m = LMMA_DEFAULT_MEMORY if opts["es_lmma_memory"] is None else int(opts["es_lmma_memory"])
+    if not 1 <= m <= _lib.SUBSPACE_MAX_DIM:
+        raise ValueError(f"es_lmma_memory must be in [1, {_lib.SUBSPACE_MAX_DIM}], not {m}")
+    opts["es_lmma_memory"] = m
+    if getattr(args, "es_optimizer", "sgd") != "sgd" or float(getattr(args, "l2_coeff", 0.0)) != 0.0:
+        raise ValueError("es_distribution 'lmma' takes its own step: not available with es_optimizer 'adam' or a "
+                         "nonzero l2_coeff")
+    if getattr(args, "adaptive", False):
+        raise ValueError("es_distribution 'lmma' adapts sigma by cumulative step-size adaptation: not available with "
+                         "--adaptive")
+    if getattr(args, "fitness_shaping", "none") != "none":
+        raise ValueError("es_distribution 'lmma' weights the ranked members with its own log weights: not available "
+                         "with fitness_shaping 'centered_rank'")
+    if getattr(args, "mirrored_sampling", False):
+        raise ValueError("es_distribution 'lmma': mirrored pairs under truncation selection bias the step-size "
+                         "adaptation; not available with mirrored sampling")
+    if int(getattr(args, "es_subspace_dim", 0) or 0):
+        raise ValueError("es_distribution 'lmma' has its own search shape: not available with es_subspace_dim")
+    if float(getattr(args, "es_novelty_weight", 0.0) or 0.0):
+        raise ValueError("es_distribution 'lmma' recombines on the fitness: not available with es_novelty_weight")
+    P = int(getattr(args, "population", 2))
+    if P < 2:
+        raise ValueError(f"es_distribution 'lmma' selects the best half: needs a population >= 2, not {P}")
+    if 2 * P >= LMMA_MIN_DIM:
+        raise ValueError(f"es_distribution 'lmma' needs c_sigma = 2 population / n < 1: population {P} is too large "
+                         f"for n = {LMMA_MIN_DIM}")
+
+
+def lmma_constants(lam, n, m):
+    """LM-MA-ES's constants (Loshchilov, Glasmachers & Beyer 2019, Algorithm 1) for population lam, dimension n and m
+    vectors, fp64: mu = lam // 2, the log weights w_i = (ln(mu + 1/2) - ln(i + 1)) / sum_j (...) for i < mu,
+    mu_w = 1 / sum w_i^2, c_sigma = 2 lam / n, c_d,j = 1 / (1.5^j n), c_c,j = lam / (4^j n) for j < m, and alpha_k =
+    prod_{j < k} (1 - c_d,j) for k <= m (the coefficient of z after k transform steps)."""
+    mu = int(lam) // 2
+    raw = np.array([np.log(mu + 0.5) - np.log(i + 1) for i in range(mu)], dtype=np.float64)
+    w = raw / raw.sum()
+    c_d = [1.0 / (1.5 ** j * n) for j in range(m)]
+    alpha = [1.0]
+    for j in range(m):
+        alpha.append(alpha[-1] * (1.0 - c_d[j]))
+    return {"mu": mu, "w": w, "mu_w": float(1.0 / np.sum(w * w)), "c_sigma": 2.0 * lam / n, "c_d": c_d,
+            "c_c": [lam / (4.0 ** j * n) for j in range(m)], "alpha": alpha}
 
 
 #: the Co-ES Hall of Fame and its defaults: 0 = off (every member plays the other roles' current base agents only)
@@ -234,7 +294,8 @@ def es_subspace(args, algorithm=None):
             raise ValueError(f"es_subspace_alpha must be in (0, 1], not {alpha}")
     if k:
         if getattr(args, "es_distribution", "isotropic") != "isotropic":
-            raise ValueError("es_subspace_dim: guided search is not available with es_distribution 'separable'")
+            raise ValueError("es_subspace_dim: guided search is not available with es_distribution "
+                             f"{getattr(args, 'es_distribution', 'isotropic')!r}")
         if not getattr(args, "update_from_members", True):
             raise ValueError("es_subspace_dim: guided search needs the update from the members, not available with "
                              "--regenerate_noise")
@@ -1001,7 +1062,12 @@ class ESEngine(_EngineBase):
     distributions on 32 probe observations (``novelty_probe_obs``, drawn once from the seed), fp32 [160].  Per role a
     ring ``novelty_ring`` fp32 [A, 160] holds those of past base agents (the founders, then one after every apply),
     replicated like theta; a member's novelty is the mean distance to its k nearest entries, and the update is
-    weighted by F = (1 - w) cr(reward) + w cr(novelty) (cr: centered ranks of the global vectors)."""
+    weighted by F = (1 - w) cr(reward) + w cr(novelty) (cr: centered ranks of the global vectors).
+
+    Opt-in LM-MA-ES (``es_distribution`` 'lmma', Loshchilov et al. 2019): m direction vectors per role ``lmma_M`` fp32
+    [m, len(theta_cat)], the path ``lmma_p`` and the Gram ``lmma_G`` fp64 [3, m, m], replicated like theta.  Members are
+    theta + sigma (alpha z + sum_l beta_l m_l) through the first k = min(g, m) vectors; the mu best are recombined with
+    log weights, and the apply steps theta, the path, the vectors and sigma (cumulative step-size adaptation)."""
 
     kind = "ES"
     #: Philox stream of the initial states of ``hof_matrix``
@@ -1050,6 +1116,8 @@ class ESEngine(_EngineBase):
             self._hof_eval_slot_gen = None
         self.distribution = es_distribution(args, "ES")
         self.separable = self.distribution["es_distribution"] == "separable"
+        #: LM-MA-ES: m direction vectors per role (0: off)
+        self.lmma_m = self.distribution.get("es_lmma_memory", 0)
         self.subspace_opts = es_subspace(args, "ES")
         #: guided-search subspace dimension k (0: off) and the share alpha of the variance outside it
         self.subspace_k = self.subspace_opts["es_subspace_dim"]
@@ -1105,6 +1173,9 @@ class ESEngine(_EngineBase):
                 lr = self.distribution["sigma_learning_rate"]
                 self.sigma_lr[r] = float(lr) if lr is not None else default_sigma_learning_rate(len(pidx))
                 off += pitch
+        self.lmma_M = self.lmma_p = self.lmma_G = None
+        if self.lmma_m:
+            self._lmma_init(pitches)
         self.adam_m = self.adam_v = None
         if self.options["es_optimizer"] == "adam":
             self.adam_m = torch.zeros_like(self.theta_cat)
@@ -1119,6 +1190,82 @@ class ESEngine(_EngineBase):
         self.weight_stats = {r: None for r in ROLES}      # fp32 [n_local, 4] when args.log_member_weight_stats
         self.member_stats = bool(getattr(args, "log_member_weight_stats", False))
         self.variant = self.rollout_variant(self.P, self.K)
+
+    def _lmma_init(self, pitches):
+        """LM-MA-ES state, replicated like theta: the direction vectors M fp32 [m, len(theta_cat)] (zero), the path p
+        fp32 [len(theta_cat)] (zero), the Gram of each role's vectors fp64 [3, m, m] and the update count g; and
+        grad_cat = [zbar of the roles | betabar fp32 [3, m]], so a generation still has one all-reduce."""
+        m, n = self.lmma_m, self.theta_cat.numel()
+        self.lmma_M = torch.zeros((m, n), dtype=torch.float32, device=self.device)
+        self.lmma_p = torch.zeros(n, dtype=torch.float32, device=self.device)
+        self.lmma_G = torch.zeros((len(ROLES), m, m), dtype=torch.float64, device=self.device)
+        self.lmma_stats = torch.zeros((len(ROLES), 2), dtype=torch.float64, device=self.device)
+        self.lmma_gen = 0
+        self.grad_cat = torch.zeros(n + len(ROLES) * m, dtype=torch.float32, device=self.device)
+        self.delta_cat = self.grad_cat[:n]
+        self.lmma_betabar = self.grad_cat[n:].view(len(ROLES), m)
+        off = 0
+        for r, pitch in zip(ROLES, pitches):
+            self.last_delta[r] = self.grad_cat[off:off + pitch]
+            off += pitch
+        #: per role: the constants (n = the role's Linear entries), the weights on the device, this generation's
+        #: transform coefficients beta fp32 [n_local, k] and selected ids
+        self.lmma_const = {r: lmma_constants(self.P, len(layout.fc_perturbable_index(layout.OBS_DIM[r])), m)
+                           for r in ROLES}
+        self.lmma_w = {r: torch.tensor(c["w"], dtype=torch.float32).to(self.device) for r, c in self.lmma_const.items()}
+        self.lmma_beta = {r: None for r in ROLES}
+        self.lmma_ids = {r: None for r in ROLES}
+
+    def _lmma_k(self):
+        """Vectors in use this generation: k = min(g, m)."""
+        return min(self.lmma_gen, self.lmma_m)
+
+    def _lmma_perturb(self, role):
+        """K5 of LM-MA-ES: the isotropic K5 while k = 0, else the projection and the LM-MA K5."""
+        in_dim, k = layout.OBS_DIM[role], self._lmma_k()
+        if k == 0:
+            self.lmma_beta[role] = torch.zeros((self.shard.n_local, 0), dtype=torch.float32, device=self.device)
+            self.k.es_perturb(self.theta[role], in_dim, self.sigma_dev(role), self.seed, role, self.gen,
+                              self.shard.row0, self.shard.n_local, out=self.members[role])
+            return
+        o, p = self.cols[role]
+        c = self.lmma_const[role]
+        M = self.lmma_M[:, o:o + p]
+        beta = self.k.es_lmma_project(M, k, self.lmma_G[ROLES.index(role)], c["c_d"][:k], in_dim, self.seed, role,
+                                      self.gen, self.shard.row0, self.shard.n_local, status=self.status)
+        self.lmma_beta[role] = beta
+        self.k.es_perturb_lmma(self.theta[role], in_dim, self.sigma_dev(role), M, k, beta, c["alpha"][k], self.seed,
+                               role, self.gen, self.shard.row0, self.shard.n_local, out=self.members[role])
+
+    def _lmma_update(self):
+        """Select the mu best of the global fitness (ties to the lower index, NaN last, whatever reference_compat
+        says: the reference has no LM-MA-ES), recombine this rank's selected normals, all-reduce, apply."""
+        a = self.args
+        k = self._lmma_k()
+        for i, role in enumerate(ROLES):
+            c = self.lmma_const[role]
+            ids = self.k.select_topk(self.fitness[role], c["mu"], order=_lib.ORDER_STABLE_DESC)
+            self.lmma_ids[role] = ids
+            self.k.es_lmma_reduce(ids, self.lmma_w[role], self.lmma_beta[role], layout.OBS_DIM[role], self.seed, role,
+                                  self.gen, self.shard.row0, self.shard.n_local, zbar=self.last_delta[role],
+                                  betabar=self.lmma_betabar[i, :k])
+        self.comm.all_reduce_sum(self.grad_cat)
+        self._join_eval()                 # the previous generation's evaluation games read theta and sigma
+        # replicated on every rank from the same all-reduced buffer: the replicas stay identical
+        cs = [self.lmma_const[r] for r in ROLES]
+        self.k.es_lmma_apply(self.theta_cat, self.lmma_M, self.lmma_p, self.delta_cat, self.lmma_betabar,
+                             [layout.OBS_DIM[r] for r in ROLES], k=k, alpha=[c["alpha"][k] for c in cs],
+                             c_sigma=[c["c_sigma"] for c in cs], mu_w=[c["mu_w"] for c in cs], c_m=a.learning_rate,
+                             c_c=[c["c_c"] for c in cs], G=self.lmma_G, gstate=self.gstate,
+                             sigma_min=a.min_mutation_power, sigma_max=a.max_mutation_power, stats=self.lmma_stats,
+                             status=self.status)
+        self.lmma_gen += 1
+
+    def _lmma_record(self, k):
+        """History record of LM-MA-ES: per role the vectors used, |p_sigma|^2 / n and sigma after the update."""
+        st = self.lmma_stats.cpu().numpy()
+        return {r: {"k_eff": k, "p_sigma_norm2_over_n": float(st[i, 0]), "sigma_after": float(st[i, 1])}
+                for i, r in enumerate(ROLES)}
 
     def _base_opponents(self, role):
         """Rows of the two other seats (ascending seat order): the base rows [1, pitch], or with the Hall of Fame the
@@ -1177,6 +1324,8 @@ class ESEngine(_EngineBase):
                 self.k.es_perturb_diag(self.theta[role], self.sigma_rows[role], in_dim, self.seed, role, self.gen,
                                        self.shard.row0, self.shard.n_local, mirrored=self.mirrored,
                                        out=self.members[role])
+            elif self.lmma_m:
+                self._lmma_perturb(role)
             elif self.subspace_k:
                 o, p = self.cols[role]
                 i = ROLES.index(role)
@@ -1258,6 +1407,12 @@ class ESEngine(_EngineBase):
                 if self.novelty_w:
                     self.novelty[role] = allp[:, nov0 + i].contiguous()
 
+        if self.lmma_m:
+            finish_fitness()              # the selection ranks the global fitness
+            self._lmma_update()
+            if self.hof_size:
+                self._hof_append()
+            return
         need_global = a.fitness_sharing or self.shaping
         if need_global:
             finish_fitness()              # the update needs the shared fitness / the ranks of the global fitness
@@ -1332,6 +1487,7 @@ class ESEngine(_EngineBase):
         self._raise_pending_status()
         if self.adaptive:
             self._join_eval()             # this generation's sigma is the previous generation's output
+        lmma_k = self._lmma_k() if self.lmma_m else None
         self.evaluate(init_by_role)
         self.update()
         self._finish_generation(self.theta["agent_0"], self.theta["agent_1"], self.theta["adversary_0"])
@@ -1353,7 +1509,8 @@ class ESEngine(_EngineBase):
                 subspace_rank=({r: int(x) for r, x in zip(ROLES, self.subspace_keff.cpu().tolist())}
                                if self.subspace_k else None),
                 novelty=({r: self.novelty[r].cpu().numpy().copy() for r in ROLES} if self.novelty_w else None),
-                novelty_filled=self._novelty_eval_filled if self.novelty_w else None))
+                novelty_filled=self._novelty_eval_filled if self.novelty_w else None,
+                lmma=self._lmma_record(lmma_k) if self.lmma_m else None))
         self.gen += 1
         return self.last_eval() if sync else None
 
@@ -1420,6 +1577,9 @@ class ESEngine(_EngineBase):
             sd.update(adam_m=self.adam_m.cpu().clone(), adam_v=self.adam_v.cpu().clone())
         if self.separable:
             sd.update(sigma=self.sigma_cat.cpu().clone())
+        if self.lmma_m:
+            sd.update(lmma_M=self.lmma_M.cpu().clone(), lmma_p=self.lmma_p.cpu().clone(),
+                      lmma_G=self.lmma_G.cpu().clone(), lmma_gen=self.lmma_gen)
         if self.hof_size:
             sd.update(hof_ring=self.hof_ring.cpu().clone(), hof_head=self.hof_head, hof_filled=self.hof_filled,
                       hof_slot_gen=list(self.hof_slot_gen))
@@ -1431,7 +1591,10 @@ class ESEngine(_EngineBase):
         saved = sd.get("es_options", ES_OPTION_DEFAULTS)
         if saved != self.options:
             raise ValueError(f"checkpoint was written with ES options {saved}, this run uses {self.options}")
-        saved = sd.get("es_distribution", ES_DISTRIBUTION_DEFAULTS)
+        # a checkpoint written before a setting existed was written with its default
+        saved = {**ES_DISTRIBUTION_DEFAULTS, **sd.get("es_distribution", {})}
+        if saved.get("es_distribution") != "lmma":
+            saved.pop("es_lmma_memory", None)
         if saved != self.distribution:
             raise ValueError(f"checkpoint was written with the ES distribution {saved}, this run uses "
                              f"{self.distribution}")
@@ -1454,6 +1617,11 @@ class ESEngine(_EngineBase):
             self.novelty_head, self.novelty_filled = int(sd["novelty_head"]), int(sd["novelty_filled"])
         if self.separable:
             self.sigma_cat.copy_(sd["sigma"])
+        if self.lmma_m:
+            self.lmma_M.copy_(sd["lmma_M"])
+            self.lmma_p.copy_(sd["lmma_p"])
+            self.lmma_G.copy_(sd["lmma_G"])
+            self.lmma_gen = int(sd["lmma_gen"])
         if self.hof_size:
             self.hof_ring.copy_(sd["hof_ring"])
             self.hof_head, self.hof_filled = int(sd["hof_head"]), int(sd["hof_filled"])

@@ -79,13 +79,22 @@ def parse_arguments(argv=None):
                         "large for Adam (try 0.01)")
     p.add_argument("--l2_coeff", type=float, default=0.0,
                    help="ES: L2 weight decay, the step follows g = ghat - l2_coeff * theta (with sgd or adam)")
-    p.add_argument("--es_distribution", choices=["isotropic", "separable"], default="isotropic",
-                   help="ES: search with one mutation power per role (isotropic, the reference) or with one per "
+    p.add_argument("--es_distribution", choices=["isotropic", "separable", "lmma"], default="isotropic",
+                   help="ES: search with one mutation power per role (isotropic, the reference), with one per "
                         "parameter adapted by separable NES (Schaul et al. 2011): sigma starts at "
                         "--initial_mutation_power_*, moves by exp(sigma_learning_rate/2 * g_sigma) every generation and "
                         "stays in [--min_mutation_power, --max_mutation_power]; --learning_rate is then SNES's "
                         "eta_mu (1.0 is the textbook value; the default stays the reference's 0.1).  Not with "
-                        "--es_optimizer adam, --l2_coeff or --adaptive")
+                        "--es_optimizer adam, --l2_coeff or --adaptive.  Or lmma: LM-MA-ES (Loshchilov et al. 2019), "
+                        "a search shape adapted from the best half of the population through --es_lmma_memory "
+                        "direction vectors per role, with sigma adapted by cumulative step-size adaptation (clamped to "
+                        "[--min_mutation_power, --max_mutation_power]); --learning_rate is then its c_m (the paper's "
+                        "value is 1.0).  Not with --es_optimizer adam, --l2_coeff, --adaptive, --fitness_shaping "
+                        "centered_rank, --mirrored_sampling, --es_subspace_dim or --es_novelty_weight")
+    p.add_argument("--es_lmma_memory", type=int, default=None,
+                   help="ES, lmma: direction vectors m per role, 1 <= m <= 32 (default 8, not the paper's "
+                        "4 + 3 ln n = 39: vector j moves at rate population / (4^j n), so at a population of 1024 and "
+                        "n ~ 138 k vectors past ~8 barely move in 1e4 generations and cost one K5 term each)")
     p.add_argument("--sigma_learning_rate", type=float, default=None,
                    help="ES, separable: learning rate of log sigma for all roles (default: (3 + ln d) / (5 sqrt d) "
                         "per role, d = its number of Linear parameters)")
@@ -103,7 +112,7 @@ def parse_arguments(argv=None):
                         "subspace spanned by the last k update estimates (an orthonormal basis recomputed every "
                         "generation on the device), 0 <= k <= 32; the total variance stays that of the isotropic "
                         "search, so --initial_mutation_power_*, --adaptive and the clamps keep their meaning.  0 = off "
-                        "(the isotropic search of the reference).  Not with --es_distribution separable or "
+                        "(the isotropic search of the reference).  Not with --es_distribution separable / lmma or "
                         "--regenerate_noise")
     p.add_argument("--es_subspace_alpha", type=float, default=None,
                    help="ES, with --es_subspace_dim k: share alpha in (0, 1] of the variance kept isotropic; members "
@@ -229,6 +238,7 @@ class Args:
         self.l2_coeff = a.l2_coeff
         self.es_distribution = a.es_distribution
         self.sigma_learning_rate = a.sigma_learning_rate
+        self.es_lmma_memory = a.es_lmma_memory
         self.es_hof_size = a.es_hof_size
         self.es_hof_opponents = a.es_hof_opponents
         self.es_subspace_dim = a.es_subspace_dim

@@ -635,6 +635,135 @@ def es_subspace_basis(ring, newest, filled, in_dims, *, out=None, k_eff=None):
     return out, k_eff
 
 
+def _need_status(name, status):
+    if status is not None and (status.dtype != torch.int32 or status.numel() != 1):
+        raise _lib.CevError(f"{name}: status must be a one-element int32 tensor")
+
+
+def _need_sigma_dev(name, sigma):
+    if not (isinstance(sigma, torch.Tensor) and sigma.dtype == torch.float64 and sigma.numel() == 1):
+        raise _lib.CevError(f"{name}: sigma must be a one-element float64 device tensor (the generation state slot)")
+
+
+def es_lmma_project(M, k, G, cd, in_dim, seed, role, gen, row0, n_rows, *, beta=None, s_out=None, status=None):
+    """LM-MA-ES projection and transform coefficients (see ``cev_es_lmma_project_f32``): s = M[:k] z_i in fp64 for the
+    members [row0, row0 + n_rows) (z the stream of :func:`es_perturb`), then the compact form of the sequential
+    transform with the Gram ``G`` fp64 [m, m] and ``cd`` (host, the k values c_d,j).  ``M``: fp32 [>= k, pitch] rows
+    (contiguous rows, any row stride).  Returns beta fp32 [n_rows, k]; ``s_out`` (optional) receives s fp64
+    [n_rows, k]; a non-finite s or beta sets ``status``."""
+    dev = _need_cuda(G, beta, s_out, status)
+    _need_rows(dev, M)
+    pitch = layout.fc_pitch(in_dim)
+    k, n_rows = int(k), int(n_rows)
+    if M.dtype != torch.float32 or M.shape[1] != pitch or not 1 <= k <= min(M.shape[0], _lib.SUBSPACE_MAX_DIM):
+        raise _lib.CevError(f"es_lmma_project: M must be float32 [>= k, {pitch}] and 1 <= k <= 32")
+    if G.dtype != torch.float64 or G.dim() != 2 or G.shape[0] != G.shape[1] or G.shape[0] < k:
+        raise _lib.CevError("es_lmma_project: G must be float64 [m, m] with m >= k")
+    if len(cd) != k:
+        raise _lib.CevError(f"es_lmma_project: need k = {k} values of c_d")
+    for name, t, dt in (("beta", beta, torch.float32), ("s_out", s_out, torch.float64)):
+        if t is not None and (t.dtype != dt or tuple(t.shape) != (n_rows, k)):
+            raise _lib.CevError(f"es_lmma_project: {name} must be {dt} [{n_rows}, {k}]")
+    _need_status("es_lmma_project", status)
+    if beta is None:
+        beta = torch.empty((n_rows, k), dtype=torch.float32, device=dev)
+    n_chunks = -(-layout.fc_dim(in_dim) // _lib.LMMA_PROJECT_CHUNK)
+    part = torch.empty(max(n_chunks * n_rows * k, 1), dtype=torch.float64, device=dev)
+    role_id = layout.ROLE_ID[role] if isinstance(role, str) else int(role)
+    cd_arr = (ctypes.c_double * k)(*[float(c) for c in cd])
+    check(_call("cev_es_lmma_project_f32", _h(dev), _ptr(M), M.stride(0), k, _ptr(G), G.shape[0], cd_arr, int(in_dim),
+                int(seed), role_id, int(gen), int(row0), n_rows, _ptr(part), _ptr(beta), _ptr(s_out), _ptr(status),
+                _stream(dev), launches=2), "cev_es_lmma_project_f32")
+    return beta
+
+
+def es_perturb_lmma(theta, in_dim, sigma, M, k, beta, alpha, seed, role, gen, row0, n_rows, *, out=None):
+    """LM-MA K5 (see ``cev_es_perturb_lmma_f32``): member rows theta + fl(sigma eps) with eps = fl(fl(fp32(alpha) z) +
+    sum_{l < k} fl(M[l] beta_l)) on the Linear entries, z the stream of :func:`es_perturb`.  ``sigma``: the
+    one-element fp64 DEVICE slot; ``beta``: fp32 [n_rows, k] from :func:`es_lmma_project`."""
+    dev = _need_cuda(theta, sigma, beta, out)
+    _need_rows(dev, M)
+    _need_sigma_dev("es_perturb_lmma", sigma)
+    pitch = layout.fc_pitch(in_dim)
+    k, n_rows = int(k), int(n_rows)
+    _need_f32("es_perturb_lmma: theta", theta, pitch)
+    if M.dtype != torch.float32 or M.shape[1] != pitch or not 1 <= k <= min(M.shape[0], _lib.SUBSPACE_MAX_DIM):
+        raise _lib.CevError(f"es_perturb_lmma: M must be float32 [>= k, {pitch}] and 1 <= k <= 32")
+    if beta.dtype != torch.float32 or tuple(beta.shape) != (n_rows, k):
+        raise _lib.CevError(f"es_perturb_lmma: beta must be float32 [{n_rows}, {k}]")
+    if out is not None and (out.dtype != torch.float32 or tuple(out.shape) != (n_rows, pitch)):
+        raise _lib.CevError(f"es_perturb_lmma: out must be float32 [{n_rows}, {pitch}]")
+    if out is None:
+        out = torch.empty((n_rows, pitch), dtype=torch.float32, device=dev)
+    role_id = layout.ROLE_ID[role] if isinstance(role, str) else int(role)
+    check(_call("cev_es_perturb_lmma_f32", _h(dev), _ptr(theta), int(in_dim), _ptr(sigma), _ptr(M), M.stride(0), k,
+                _ptr(beta), float(alpha), int(seed), role_id, int(gen), int(row0), n_rows, pitch, _ptr(out),
+                _stream(dev)), "cev_es_perturb_lmma_f32")
+    return out
+
+
+def es_lmma_reduce(ids, w, beta, in_dim, seed, role, gen, row0, n_rows, *, zbar=None, betabar=None):
+    """LM-MA weighted recombination over this rank's rows (see ``cev_es_lmma_reduce_f32``): ``ids`` int64 [mu] the
+    selected members best first, ``w`` fp32 [mu] their weights, ``beta`` fp32 [n_rows, k] (k may be 0).  Returns
+    (zbar fp32 [pitch], betabar fp32 [k]), this rank's share of sum_i w_i z_(i) and sum_i w_i beta_(i)."""
+    dev = _need_cuda(ids, w, beta if beta.numel() else None, zbar, betabar)
+    pitch = layout.fc_pitch(in_dim)
+    mu, k = ids.numel(), beta.shape[1]
+    if ids.dtype != torch.int64 or w.dtype != torch.float32 or w.numel() != mu or mu < 1:
+        raise _lib.CevError("es_lmma_reduce: ids must be int64 [mu >= 1] and w float32 [mu]")
+    if beta.dtype != torch.float32 or beta.dim() != 2 or beta.shape[0] != int(n_rows) or k > _lib.SUBSPACE_MAX_DIM:
+        raise _lib.CevError(f"es_lmma_reduce: beta must be float32 [{n_rows}, k <= 32]")
+    zbar = torch.empty(pitch, dtype=torch.float32, device=dev) if zbar is None else zbar
+    betabar = torch.empty(k, dtype=torch.float32, device=dev) if betabar is None else betabar
+    _need_f32("es_lmma_reduce: zbar", zbar, pitch)
+    _need_f32("es_lmma_reduce: betabar", betabar, k)
+    part = torch.empty(_lib.LMMA_REDUCE_SPLIT * pitch, dtype=torch.float64, device=dev)
+    role_id = layout.ROLE_ID[role] if isinstance(role, str) else int(role)
+    check(_call("cev_es_lmma_reduce_f32", _h(dev), _ptr(ids), _ptr(w), mu, _ptr(beta) if k else ctypes.c_void_p(0), k,
+                int(in_dim), int(seed), role_id, int(gen), int(row0), int(n_rows), _ptr(part), _ptr(zbar),
+                _ptr(betabar) if k else ctypes.c_void_p(0), _stream(dev), launches=2), "cev_es_lmma_reduce_f32")
+    return zbar, betabar
+
+
+def es_lmma_apply(theta, M, p, zbar, betabar, in_dims, *, k, alpha, c_sigma, mu_w, c_m, c_c, G, gstate, sigma_min,
+                  sigma_max, stats=None, status=None):
+    """LM-MA apply over the FCNetwork rows of ``in_dims`` concatenated in ``theta`` / ``p`` / ``zbar`` (fp32 [n]) and
+    the rows of ``M`` (fp32 [m, n]); see ``cev_es_lmma_apply_f32``.  ``betabar`` fp32 [len(in_dims), m] (the first k of
+    each row used); ``alpha``, ``c_sigma``, ``mu_w``: one per row; ``c_c``: [len(in_dims)][m].  Steps theta with the old
+    M, updates p and every vector, writes the new Gram into ``G`` fp64 [len(in_dims), m, m] and the adapted sigma into
+    the generation state ``gstate``.  Returns ``stats`` fp64 [len(in_dims), 2] = (|p|^2 / n, sigma after)."""
+    dev = _need_cuda(theta, M, p, zbar, betabar, G, gstate, stats, status)
+    n = sum(layout.fc_pitch(d) for d in in_dims)
+    ns = len(in_dims)
+    m = M.shape[0]
+    for name, x in (("theta", theta), ("p", p), ("zbar", zbar)):
+        _need_f32(f"es_lmma_apply: {name}", x, n)
+    if M.dtype != torch.float32 or tuple(M.shape) != (m, n) or not 1 <= m <= _lib.SUBSPACE_MAX_DIM:
+        raise _lib.CevError(f"es_lmma_apply: M must be float32 [m <= 32, {n}]")
+    if betabar.dtype != torch.float32 or betabar.numel() != ns * m:
+        raise _lib.CevError(f"es_lmma_apply: betabar must be float32 [{ns}, {m}]")
+    if G.dtype != torch.float64 or tuple(G.shape) != (ns, m, m):
+        raise _lib.CevError(f"es_lmma_apply: G must be float64 [{ns}, {m}, {m}]")
+    if gstate.dtype != torch.float64:
+        raise _lib.CevError("es_lmma_apply: gstate must be float64")
+    if not 0 <= int(k) <= m or any(len(x) != ns for x in (alpha, c_sigma, mu_w, c_c)) or any(len(c) != m for c in c_c):
+        raise _lib.CevError("es_lmma_apply: need 0 <= k <= m and one alpha / c_sigma / mu_w / c_c row per row")
+    _need_status("es_lmma_apply", status)
+    if stats is None:
+        stats = torch.empty((ns, 2), dtype=torch.float64, device=dev)
+    n_chunks = -(-max(layout.fc_pitch(d) for d in in_dims) // _lib.LMMA_APPLY_CHUNK)
+    part = torch.empty(ns * n_chunks * (m * (m + 1) // 2 + 1), dtype=torch.float64, device=dev)
+
+    def arr(vals):
+        return (ctypes.c_double * len(vals))(*[float(v) for v in vals])
+    dims = (ctypes.c_int * ns)(*[int(d) for d in in_dims])
+    check(_call("cev_es_lmma_apply_f32", _h(dev), _ptr(theta), _ptr(M), m, int(k), _ptr(p), _ptr(zbar), _ptr(betabar),
+                ns, dims, arr(alpha), arr(c_sigma), arr(mu_w), float(c_m), arr([c for row in c_c for c in row]), _ptr(G),
+                _ptr(gstate), float(sigma_min), float(sigma_max), _ptr(part), _ptr(stats), _ptr(status), _stream(dev),
+                launches=2), "cev_es_lmma_apply_f32")
+    return stats
+
+
 def novelty_probe_obs(init, role, *, out=None):
     """Probe observations of the novelty search: fp32 [n, in_dim] = what ``role`` observes in the world state of each
     initial-state record of ``init`` fp64 [n, 11] (zero velocities), bit for bit the rollout's observation."""

@@ -450,6 +450,66 @@ int cev_es_subspace_basis_f32(cev_handle* h, const float* ring, int k, int newes
                               const int* in_dims, float* U, int* k_eff, cev_stream stream);
 
 /*
+ * Co-ES limited-memory matrix adaptation (LM-MA-ES, Loshchilov, Glasmachers & Beyer, IEEE TEC 23(2), 2019).  Per
+ * role m direction vectors M fp32 [m][ldm] laid out like theta (zero on LayerNorm entries and padding), their Gram
+ * G fp64 [m][ldg], an evolution path p and sigma in CEV_GS_SIGMA + role.  z_i is member i's normals of the stream of
+ * cev_es_perturb_f32 on the Linear entries; at generation g the first k = min(g, m) vectors are in use.
+ *
+ * Projection and coefficients: s_l = m_l . z_i for l < k, with fp32 x fp32 products accumulated in fp64 one add at a
+ * time, in column order within fixed chunks of 2048 columns from +0, and the chunks summed in order, so s does not
+ * depend on row0, n_rows or the grid.  Then, every operation one fp64 rounding (cd: HOST fp64 [k], c_d,j):
+ *   alpha = 1, beta = 0; for j < k: q = alpha s_j + sum_{l<j} beta_l G[j][l] (l in order);
+ *   beta_l *= (1 - cd[j]) for l < j; beta_j = cd[j] q; alpha *= (1 - cd[j])
+ * beta (out): DEVICE fp32 [n_rows][k]; part: DEVICE workspace fp64 [ceil(fc_dim / 2048)][n_rows][k]; s_out
+ * (optional): fp64 [n_rows][k].  A non-finite s or beta sets CEV_STATUS_NONFINITE in *status (optional).
+ */
+int cev_es_lmma_project_f32(cev_handle* h, const float* M, int64_t ldm, int k, const double* G, int ldg,
+                            const double* cd, int in_dim, uint64_t seed, int role, uint32_t gen, int64_t row0,
+                            int64_t n_rows, double* part, float* beta, double* s_out, int* status, cev_stream stream);
+
+/*
+ * LM-MA K5: on the Linear entries eps_j = fl(fl(alpha * z_j) + S_j), S_j = sum_{l < k} fl(M[l][j] * beta[i][l])
+ * (fp32, l in order, from +0), member = theta + fl(fp32(sigma_dev[0]) * eps_j); LayerNorm entries copied, padding 0.
+ * This is cev_es_perturb_subspace_f32's arithmetic with A = alpha and B = 1.  beta: DEVICE fp32 [n_rows][k] (row r =
+ * member row0 + r).  1 <= k <= CEV_SUBSPACE_MAX_DIM, ldm >= pitch a multiple of 4.
+ */
+int cev_es_perturb_lmma_f32(cev_handle* h, const float* theta, int in_dim, const double* sigma_dev, const float* M,
+                            int64_t ldm, int k, const float* beta, float alpha, uint64_t seed, int role, uint32_t gen,
+                            int64_t row0, int64_t n_rows, int64_t pitch, float* out, cev_stream stream);
+
+/*
+ * LM-MA weighted recombination over this rank's rows [row0, row0 + n_rows): ids DEVICE int64 [mu] (the selected
+ * members, best first) and w DEVICE fp32 [mu] (the weight of each rank).  zbar (out, fp32 [pitch]) = sum over the ranks
+ * a whose member is local, in rank order within 8 fixed splits of [0, mu), of fma(w_a, z_id[j], .) in fp64 (exact
+ * products), the splits summed in order, rounded to fp32 once (0 off the Linear entries); betabar (out, fp32 [k]) =
+ * fp32(sum in rank order of fma(w_a, beta[id - row0][l], .)) in fp64.  Members of other ranks add nothing, so the sum
+ * over ranks of zbar / betabar is the population's.  part: DEVICE workspace fp64 [8][pitch].
+ */
+int cev_es_lmma_reduce_f32(cev_handle* h, const int64_t* ids, const float* w, int mu, const float* beta, int k,
+                           int in_dim, uint64_t seed, int role, uint32_t gen, int64_t row0, int64_t n_rows,
+                           double* part, float* zbar, float* betabar, cev_stream stream);
+
+/*
+ * LM-MA apply over n_segments (<= 3) FCNetwork rows concatenated like cev_es_apply_f32 (in_dims, alpha, c_sigma,
+ * mu_w: HOST arrays [n_segments]; c_c: HOST fp64 [n_segments][m]).  M: DEVICE fp32 [m][n], p, theta, zbar: fp32 [n],
+ * betabar: fp32 [n_segments][m] (the first k of each used).  On the Linear entries, every operation one fp64 rounding
+ * and every store one fp32 rounding:
+ *   dbar = alpha zbar + sum_{l<k} betabar_l M[l] (M before its update); theta += (c_m fp32(sigma)) dbar;
+ *   p = (1 - c_s) p + sqrt(mu_w c_s (2 - c_s)) zbar;  M[l] = (1 - c_c,l) M[l] + sqrt(mu_w c_c,l (2 - c_c,l)) zbar, l < m
+ * then G (out, DEVICE fp64 [n_segments][m][m]) = the Gram of the new M and |p|^2 (fp64 products of the fp32 values,
+ * column order within chunks of 4096 columns, the chunks in order), and
+ *   sigma = clamp(sigma exp(c_s / 2 (|p|^2 / n - 1)), sigma_min, sigma_max)   (n: the row's Linear entries)
+ * into gstate[CEV_GS_SIGMA + s]; stats (out, DEVICE fp64 [n_segments][2]) = (|p|^2 / n, sigma).  A non-finite |p|^2 or
+ * Gram entry sets CEV_STATUS_NONFINITE and leaves sigma.  part: DEVICE workspace fp64
+ * [n_segments][ceil(max pitch / 4096)][m (m + 1) / 2 + 1].
+ */
+int cev_es_lmma_apply_f32(cev_handle* h, float* theta, float* M, int m, int k, float* p, const float* zbar,
+                          const float* betabar, int n_segments, const int* in_dims, const double* alpha,
+                          const double* c_sigma, const double* mu_w, double c_m, const double* c_c, double* G,
+                          double* gstate, double sigma_min, double sigma_max, double* part, double* stats,
+                          int* status, cev_stream stream);
+
+/*
  * Co-ES novelty search (NS-ES / NSR-ES, Conti et al. 2018) on a policy-space behaviour characterisation (the
  * "behavioural embedding" of Parker-Holder et al. 2020): a member is characterised by its action distributions on
  * CEV_NOVELTY_PROBES fixed probe observations, so the characterisation does not depend on the opponents it played.
